@@ -611,6 +611,8 @@ def main():
     ap.add_argument("--c4-pairs", type=int, default=C4_PAIRS, help="BASELINE config 4: distinct pairs of the whole job (0: skip the leg)")
     ap.add_argument("--c5", type=int, default=1, help="BASELINE config 5: the 24 576-pose hard-binned sweep (0: skip)")
     ap.add_argument("--old-gpu", type=int, default=1, help="time the reference's own CUDA code beside ours (0: skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (Htarget, Hjoint, der of every pair slot) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -679,6 +681,11 @@ def main():
     launches = ctx.launch_count() - launches0
     Ht, Hj, der = ctx.fetch_results(n_slots, True)
     assert np.all(np.isfinite(Hj)) and np.all(np.isfinite(der)), "non-finite results in the timed region"
+    if args.dump_outputs:  # fp64, 1 KB per pair slot
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        suffix = f"_rank{rank}" if world > 1 else ""
+        for name, a in (("Htarget", Ht), ("Hjoint", Hj), ("der", der)):
+            np.save(os.path.join(args.dump_outputs, f"{name}{suffix}.npy"), a)
 
     # ---------------- end to end through the host-buffer C-ABI call (`e2e`)
     for k in range(args.warmup):

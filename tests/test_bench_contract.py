@@ -4,6 +4,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -67,6 +69,39 @@ def test_fp64_roofline_and_sweep_helpers():
     d = orc.se3_mul(first, orc.se3_inverse(orc.se3_from_mat16(gt)))
     assert abs(2 * np.arcsin(min(1.0, np.linalg.norm(d[3:6]))) - np.hypot(0.05, 0.05)) < 1e-3  # rotation axes 0 and 1 at -0.05 rad each
     assert len({tuple(np.round(q, 12)) for q in poses[:4096]}) == 4096
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step(tmp_path, orc, synth):
+    """--dump-outputs writes what the timed path returned in its last step: slot s of a step k is pair s mod 6 at
+    make_poses(step k)[s]; checked against the oracle for two slots that share a pair."""
+    import importlib.util
+    import numpy as np
+    warmup, steps, slots = 3, 2, 7
+    out = subprocess.check_output([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", str(warmup),
+                                   "--pairs", str(slots), "--solves", "0", "--c4-pairs", "0", "--c5", "0", "--old-gpu", "0",
+                                   "--cpu-budget", "0", "--dump-outputs", str(tmp_path)], timeout=900).decode().strip().splitlines()
+    d = json.loads(out[-1])
+    assert d["steps"] == steps and d["warmup"] == warmup
+    Ht, Hj, der = (np.load(tmp_path / f"{n}.npy") for n in ("Htarget", "Hjoint", "der"))
+    assert Ht.shape == Hj.shape == (slots, 16) and der.shape == (slots, 16, 6)
+    assert Ht.dtype == Hj.dtype == der.dtype == np.float64
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    pairs = [synth.make_pair(1000 + i, bench.ROWS, bench.COLS) for i in range(bench.DISTINCT_PAIRS)]
+    pose0 = [orc.reference_perturbation(p.T_wc1) for p in pairs]
+    last = warmup + steps - 1
+    M = bench.make_poses(orc, pose0, last % min(warmup + steps, 8), slots)
+    p = pairs[0]
+    P = orc.Problem(p.im0, p.depth0, p.im1, p.T_wc0, p.intr, bench.CELL, bench.BINS, threads=4)
+    P.set_quirks(0, 1)
+    P.prepare(pose0[0])
+    for s in (0, bench.DISTINCT_PAIRS):
+        Hto, Hjo, _, Jo = P.eval(orc.se3_from_mat16(M[s]), True)
+        np.testing.assert_allclose(Ht[s], Hto, rtol=1e-10)
+        np.testing.assert_allclose(Hj[s], Hjo, rtol=1e-10)
+        assert np.max(np.abs(der[s] - Jo) / np.abs(Jo).max(axis=1, keepdims=True)) < 1e-5
 
 
 def test_make_sequence_variants():
