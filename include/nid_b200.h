@@ -183,7 +183,6 @@ int nid_event_elapsed_ms(nid_ctx* ctx, float* ms);
  * "lm_speculate" (0..8, default 4: up to four problems per nid_solve_jobs call run in latency mode, every round
  * evaluates this many trial poses of the LM schedule at once; 0/1: plain state machine);
  * "lm_graph" (1, default: a round of the latency mode is one CUDA-graph launch);
- * "sorted_mode" (1 class tasks, 2 span tasks, 0 automatic);
  * launch shapes, for tests and A/B timing only -- none of them changes a result: "stage_bulk" (-1 by geometry, 0 / 1: pass 2
  * stages the cell's log tables by a bulk copy), "asm_wide" (1 default: the 1024-thread assembly where it pays, 0 never, 2 always) */
 int nid_set_option(nid_ctx* ctx, const char* key, int value);

@@ -66,7 +66,6 @@ EvalParams make_params(nid_ctx* c, int n_jobs) {
   p.part = c->part; p.jpart = sorted ? c->jpart_s : c->jpart; p.hist = c->opt_keep_hist ? c->hist : nullptr;
   p.ht = c->ht; p.hj = c->hj; p.err = c->err; p.der = c->der; p.gn = c->gn;
   p.sd0 = c->sd0; p.sd1 = c->sd1; p.sd2 = c->sd2; p.sid = c->sid;
-  p.sv = c->sv; p.span_mode = c->span_mode ? 1 : 0;
   p.stage_bulk = (c->opt_stage_bulk < 0 ? (long long)c->rb * c->cb < NID_SMALL_CELL_PX : c->opt_stage_bulk) ? 1 : 0;
   p.sl_off = c->sl_off; p.sl_task = c->sl_task; p.sl_desc = c->sl_desc; p.task_cls = c->task_cls; p.sl_cell = c->sl_cell; p.nslices = c->nslices;
   p.sell_cap = c->sell_cap; p.max_slices = c->max_slices; p.Twc0 = c->Twc0;
@@ -81,28 +80,6 @@ EvalParams make_params(nid_ctx* c, int n_jobs) {
 // 640x480, cost+Jacobian: 4x4 cells/16 bins 77k vs 9k evals/s, the reference's default 16x16 cells/10 bins 29k vs 9k
 // (tools/time_config.py). The natural-order kernels remain for bin counts outside [6, 40] and as a second,
 // independently written implementation the parity tests hold to the same bar.
-// Task kind of the sorted path, fixed per geometry: cells of fewer than NID_SPAN_PX pixels take span tasks;
-// caller-supplied world points and more than 20 bins keep class tasks. MEASURED (B200, 640x480, 16x16 cells, 10 bins):
-// span tasks halve the assembly (2.1 -> 1.1 us per evaluation) but their 16 shared-memory read-modify-writes per pixel
-// saturate the shared-memory pipe in pass 1 (5.0 -> 7.8 us) and pass 2 gains nothing (7.5 us either way): 60.9k
-// against 68.5k evaluations/s. The automatic threshold is therefore 0 (class tasks everywhere); span tasks stay
-// available and tested behind nid_set_option("sorted_mode", 2).
-#ifndef NID_SPAN_PX
-#define NID_SPAN_PX 0
-#endif
-static bool want_span(const nid_ctx* c) {
-  if (!use_sorted(c) || c->sell_points || c->bins > 20 || c->opt_sorted_mode == 1) return false;
-  return c->opt_sorted_mode == 2 || (long long)c->rb * c->cb < NID_SPAN_PX;
-}
-static void update_task_kind(nid_ctx* c) {
-  const bool span = want_span(c);
-  if (span != c->span_mode) {
-    c->span_mode = span;
-    std::fill(c->pair_prepared.begin(), c->pair_prepared.end(), 0);  // the pixel store is laid out per task kind
-    std::fill(c->pair_sorted.begin(), c->pair_sorted.end(), 0);
-  }
-}
-
 bool use_sorted(const nid_ctx* c) {
   // the assembly tables must fit in shared memory; the end-block fold needs the two 3x3 blocks disjoint (B >= 6, the
   // reference's smallest knot table, computeH.cu:100)
@@ -124,15 +101,13 @@ int ensure_job_buffers(nid_ctx* c) {
   const size_t hs = (size_t)c->bins * c->bins + c->bins;
   if (c->opt_keep_hist && !c->hist) OKR(dalloc(&c->hist, J * NC * hs, "hist"));
   if (use_sorted(c)) {
-    const size_t rows_per_task = c->span_mode ? 4 : 1;
     const size_t need = (size_t)std::max(c->max_ntasks_prepared, 1);
-    if (c->g_stride < need || c->g_rows < rows_per_task) {
+    if (c->g_stride < need) {
       CU(cudaStreamSynchronize(c->stream), "sync before growing job buffers");
       if (c->G) cudaFree(c->G);
       c->G = nullptr;
-      OKR(dalloc(&c->G, J * std::max(need, c->g_stride) * c->bins * rows_per_task, "G"));
-      c->g_stride = std::max(need, c->g_stride);
-      c->g_rows = rows_per_task;
+      OKR(dalloc(&c->G, J * need * c->bins, "G"));
+      c->g_stride = need;
     }
     if (!c->jpart_s) OKR(dalloc(&c->jpart_s, J * (size_t)c->max_slices * 6, "jpart_s"));  // one partial per slice
     if (!c->wv) {
@@ -381,7 +356,6 @@ int nid_create(nid_ctx** out, int device, int rows, int cols, int cell, int bins
   c->pair_sorted.assign(P, 0);
   OKR(launch_build_lut(c));
   OKR(sorted_init(c));
-  c->span_mode = want_span(c);
   CU(cudaStreamSynchronize(c->stream), "sync after lut");
   *out = c;
   return NID_OK;
@@ -394,7 +368,7 @@ int nid_destroy(nid_ctx* c) {
   void* ptrs[] = {c->pwx, c->pwy, c->pwz, c->im0, c->im1, c->inb0, c->n_c, c->href, c->cam, c->Twc0, c->cnt, c->d_depth,
                   c->d_img64, c->d_flag, c->d_pix, c->d_pix4, c->d_pix4_jobs, c->chunk_cnt, c->d_bsv, c->d_bsi, c->lut_w, c->lut_k, c->poses,
                   c->job_pair, c->aux_pose, c->part, c->jpart, c->hist, c->ht, c->hj, c->err, c->der, c->gn, c->hard,
-                  c->depth, c->sd0, c->sd1, c->sd2, c->sid, c->sv, c->sl_off, c->sl_task, c->sl_desc, c->task_cls, c->sl_cell, c->nslices, c->task_pos,
+                  c->depth, c->sd0, c->sd1, c->sd2, c->sid, c->sl_off, c->sl_task, c->sl_desc, c->task_cls, c->sl_cell, c->nslices, c->task_pos,
                   c->lay_tot, c->lay_base, c->prep_poses, c->depth16, c->depth_factor, c->d_tex2, c->d_pack, c->tasks, c->ntasks, c->cell_task_start, c->cell_slice_start, c->G, c->jpart_s, c->fp1, c->cls_task_start, c->span_start, c->wv};
   for (auto t : c->h_k1tex) if (t) cudaDestroyTextureObject(t);
   for (auto arr : c->k1_arrays) if (arr) cudaFreeArray(arr);
@@ -557,7 +531,6 @@ int nid_set_pair_points(nid_ctx* c, int pair, const double* points_3d, const dou
       CU(cudaStreamSynchronize(c->stream), "sync before switching to the point form");
       c->sell_points = true;
       std::fill(c->pair_prepared.begin(), c->pair_prepared.end(), 0);
-      update_task_kind(c);
     }
   }
   OKR(upload_images_f64(c, pair, im0, im1));
@@ -616,7 +589,6 @@ static int build_sorted_layout(nid_ctx* c, int pair0, int n) {
     OKR(dalloc(&c->sd1, (size_t)c->n_pairs * c->sell_cap, "sd1"));
     OKR(dalloc(&c->sd2, (size_t)c->n_pairs * c->sell_cap, "sd2"));
   }
-  if (c->span_mode && !c->sv) OKR(dalloc(&c->sv, (size_t)c->n_pairs * c->sell_cap, "sv"));
   if (!c->chunk_cnt) {
     const size_t nchunks = ((size_t)c->rb * c->cb + 255) / 256;
     OKR(dalloc(&c->chunk_cnt, (size_t)c->setup_batch * c->ncell * nchunks * NID_NCLS, "chunk_cnt"));
@@ -1263,14 +1235,6 @@ int nid_set_option(nid_ctx* c, const char* key, int value) {
     if (value < 0 || value > 2) { set_error("path must be 0 (auto), 1 (natural) or 2 (sorted)"); return NID_ERR_ARG; }
     if (value == 2 && (c->bins > NID_SORTED_MAX_BINS || c->bins < NID_SORTED_MIN_BINS)) { set_error("the sorted path supports 6 to 40 bins"); return NID_ERR_UNSUPPORTED; }
     c->opt_path = value;
-    update_task_kind(c);
-    return NID_OK;
-  }
-  if (!strcmp(key, "sorted_mode")) {
-    if (value < 0 || value > 2) { set_error("sorted_mode must be 0 (automatic), 1 (class tasks) or 2 (span tasks)"); return NID_ERR_ARG; }
-    if (value == 2 && (c->bins > 20 || c->sell_points || !use_sorted(c))) { set_error("span tasks need the sorted path, depth pairs and at most 20 bins"); return NID_ERR_UNSUPPORTED; }
-    c->opt_sorted_mode = value;
-    update_task_kind(c);
     return NID_OK;
   }
   if (!strcmp(key, "keep_hist")) { c->opt_keep_hist = value; return NID_OK; }

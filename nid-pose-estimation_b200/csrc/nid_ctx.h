@@ -55,8 +55,6 @@ struct EvalParams {
   const double* sd1;    // point form only: world y
   const double* sd2;    // point form only: world z
   const unsigned* sid;  // [n_pairs][sell_cap] (row << 16) | col, 0xFFFFFFFF = padding
-  uint8_t* sv;          // span tasks only: [n_pairs][sell_cap] reference intensity of the pixel in that slot
-  int span_mode;        // tasks are (cell, reference span) runs instead of (cell, reference intensity) runs
   int stage_bulk;       // pass 2 stages the cell's log tables by a bulk copy (small cells: short slices)
   const int* sl_off;    // [n_pairs][max_slices+1] first pixel slot of every slice (multiples of 128)
   const int* sl_task;   // [n_pairs][max_slices*32] task of every lane, -1 = none
@@ -121,9 +119,6 @@ struct nid_ctx {
   double* depth = nullptr;     // [n_pairs][N] reference depth as uploaded (depth form)
   double *sd0 = nullptr, *sd1 = nullptr, *sd2 = nullptr;
   unsigned* sid = nullptr;
-  uint8_t* sv = nullptr;       // span tasks: reference intensity per pixel slot
-  bool span_mode = false;      // small cells: tasks by reference span (nid_sorted.cu, "span tasks"); fixed per geometry
-  int opt_sorted_mode = 0;     // 0 automatic, 1 class tasks, 2 span tasks
   size_t sell_cap = 0;
   int* sl_desc = nullptr;
   unsigned short* task_cls = nullptr;
@@ -158,7 +153,6 @@ struct nid_ctx {
   std::vector<double> h_Twc0, h_cam;  // host copies per pair (geometry tables are built on the host)
   unsigned* d_pack = nullptr;  // [setup_batch][N] scratch for the packed textures
   size_t g_stride = 0;
-  size_t g_rows = 0;           // rows of `bins` doubles per task in G (1: class tasks, 4: span tasks)
   int opt_path = 0;            // 0 auto, 1 natural-order atomics (v1), 2 sorted
   int opt_keep_hist = 0;
   std::vector<char> pair_set, pair_prepared, pair_sorted;

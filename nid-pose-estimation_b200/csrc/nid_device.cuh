@@ -34,17 +34,8 @@ __device__ __forceinline__ void warp_project(const Pose& P, const Cam& cam, doub
   x1 = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(P.m[0], x0), __dmul_rn(P.m[3], y0)), __dmul_rn(P.m[6], z0)), P.m[9]);
   y1 = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(P.m[1], x0), __dmul_rn(P.m[4], y0)), __dmul_rn(P.m[7], z0)), P.m[10]);
   z1 = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(P.m[2], x0), __dmul_rn(P.m[5], y0)), __dmul_rn(P.m[8], z0)), P.m[11]);
-#ifdef NID_ABL_NODIV
-  u = cam.fx * x1 * 0.38 + cam.cx;
-  v = cam.fy * y1 * 0.38 + cam.cy;
-#elif defined(NID_ABL_RCP)
-  const double rz = 1.0 / z1;
-  u = fma(cam.fx * x1, rz, cam.cx);
-  v = fma(cam.fy * y1, rz, cam.cy);
-#else
   u = __dadd_rn(__ddiv_rn(__dmul_rn(cam.fx, x1), z1), cam.cx);
   v = __dadd_rn(__ddiv_rn(__dmul_rn(cam.fy, y1), z1), cam.cy);
-#endif
 }
 
 // The CPU edge projects a second time in linearizeOplus, as fx*(x/z)+cx (types_six_dof_expmap.cpp:407-421);
@@ -159,19 +150,11 @@ __device__ __forceinline__ void bspline4(double ub, int k, int bins, double w[4]
 }
 
 // ---- fast variants used by the sorted kernels -----------------------------------------------------
-// exact small-integer -> double without the (slow) I2F.F64 path: bits(2^52 + v) - 2^52
-#ifndef NID_U2D_MODE
-#define NID_U2D_MODE 0  // 0: magic constant (one move + one DADD); 1: I2F.F64 (one XU-pipe instruction)
-#endif
-#if NID_U2D_MODE == 1
-__device__ __forceinline__ double u2d(unsigned v) { return __uint2double_rn(v); }
-__device__ __forceinline__ double i2d_small(int v) { return __int2double_rn(v); }
-#else
+// exact small-integer -> double without the I2F.F64 path: bits(2^52 + v) - 2^52 (one move + one DADD)
 __device__ __forceinline__ double u2d(unsigned v) { return __hiloint2double(0x43300000, (int)v) - 4503599627370496.0; }
 __device__ __forceinline__ double i2d_small(int v) {  // |v| < 2^20
   return __hiloint2double(0x43300000, v + 1048576) - (4503599627370496.0 + 1048576.0);
 }
-#endif
 
 // Centre sample and central-difference gradient (types_six_dof_expmap.cpp:434-435 via .h:310-328) from
 // 12 taps instead of 5 x 4: for u,v >= 1 the five bilinear samples share their fractional weights.

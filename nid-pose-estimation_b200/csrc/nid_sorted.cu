@@ -38,9 +38,7 @@
 // loads and prefetched into L2 two groups ahead, so that L1 stays with the target-image gathers; CTAs are small
 // (pass 1: one warp, register budget for 18-20 resident warps; pass 2: two warps at 16 resident warps); the
 // shared-memory carve-out is requested per kernel. Also in this file: the device-side construction of the task and
-// slice tables (k_layout_*), the warp-per-cell assembly for small cells, the optional cp.async.bulk ring of the pixel
-// store and the optional span tasks (both measured slower than what ships, kept as build / run-time options), and
-// kernel 1 on its own (k_warp_sample_jobs).
+// slice tables (k_layout_*), the warp-per-cell assembly for small cells, and kernel 1 on its own (k_warp_sample_jobs).
 #include <cuda_fp16.h>
 #include <math.h>
 #include <stdlib.h>
@@ -65,9 +63,6 @@ namespace nid {
 #define NID_BLK_JOB blockIdx.x
 #define NID_BLK_CHUNK blockIdx.y
 #define NID_GRID(jobs, chunks) dim3(jobs, chunks)
-#ifndef NID_CARVEOUT
-#define NID_CARVEOUT 1
-#endif
 #ifndef NID_PREFETCH_L2
 #define NID_PREFETCH_L2 2  // groups beyond the register prefetch that the pixel kernels pull into L2 (0: off)
 #endif
@@ -98,7 +93,6 @@ __device__ __forceinline__ int sell_key(const EvalParams& p, size_t base, int c,
   col = (c % p.cell) * p.cb + t % p.cb;
   const size_t i = base + (size_t)row * p.cols + col;
   if (isnan(p.pwx[i])) return -1;
-  if (p.span_mode) return p.inb0[i] ? __ldg(p.lut_k + p.im0[i]) : p.bins - 3;  // reference span; NS = no reference sample
   return p.inb0[i] ? (int)p.im0[i] : 256;
 }
 
@@ -176,7 +170,6 @@ __global__ void __launch_bounds__(256) k_scatter_sell(EvalParams p, int pair0, i
     if (PTS) { sd0[dst] = p.pwx[i]; sd1[dst] = p.pwy[i]; sd2[dst] = p.pwz[i]; }
     else sd0[dst] = depth[(size_t)row * p.cols + col];
     sid[dst] = ((unsigned)row << 16) | (unsigned)col;
-    if (p.span_mode) p.sv[dst] = p.im0[i];
   }
 }
 
@@ -201,15 +194,12 @@ struct CellLayoutSm {
   int T, F, S, SF, slots;
 };
 
-// span: lut_k (reference span of every intensity) when the tasks are per span, else nullptr; NS = bins - 3
-__device__ __forceinline__ void cell_layout(const unsigned* __restrict__ cnt, int L, CellLayoutSm& s,
-                                            const int* __restrict__ span = nullptr, int NS = 0) {
+__device__ __forceinline__ void cell_layout(const unsigned* __restrict__ cnt, int L, CellLayoutSm& s) {
   const int v = threadIdx.x, lane = v & 31, w = v >> 5;
   constexpr int NW = NID_LAYOUT_THREADS / 32;
-  int c = v < NID_NCLS ? (int)cnt[v] : 0;
-  const int c_px = c;  // pixels of reference intensity v (n_c below counts these whatever the task kind)
+  const int c = v < NID_NCLS ? (int)cnt[v] : 0;  // pixels of reference intensity v
   {  // n_c = pixels with a reference sample; cells under 300 get no tasks (computeH.cu:271)
-    int n = v < 256 ? c_px : 0;
+    int n = v < 256 ? c : 0;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
     if (lane == 0) s.wsum[0][w] = n;
@@ -219,15 +209,6 @@ __device__ __forceinline__ void cell_layout(const unsigned* __restrict__ cnt, in
 #pragma unroll
   for (int i = 0; i < NW; i++) n_c += s.wsum[0][i];
   __syncthreads();
-  if (span) {  // "class" k = reference span k (k < NS), NS = pixels without a reference sample; integer sums: any order
-    if (v < NID_NCLS) s.r[v] = 0;
-    __syncthreads();
-    if (v < 256) { if (c) atomicAdd(&s.r[span[v]], c); }
-    else if (v == 256) s.r[NS] = c;  // (nothing else lands on index NS: span[v] < NS)
-    __syncthreads();
-    c = v < NID_NCLS ? s.r[v] : 0;
-    __syncthreads();
-  }
   const int cc = n_c >= NID_MIN_CELL_POINTS ? c : 0;
   const int nf = cc / L, r = cc - nf * L, nt = nf + (r > 0 ? 1 : 0);
   int a = nt, b = nf;  // inclusive scans over the classes
@@ -272,10 +253,10 @@ __device__ __forceinline__ void cell_layout(const unsigned* __restrict__ cnt, in
 
 // totals per (pair, cell): tasks, slices, pixel slots
 __global__ void __launch_bounds__(NID_LAYOUT_THREADS) k_layout_totals(int pair0, int ncell, int L, const unsigned* __restrict__ cnt,
-                                                                      int* __restrict__ tot, const int* __restrict__ span, int NS) {
+                                                                      int* __restrict__ tot) {
   __shared__ CellLayoutSm s;
   const int c = blockIdx.x, pair = pair0 + blockIdx.y;
-  cell_layout(cnt + ((size_t)pair * ncell + c) * NID_NCLS, L, s, span, NS);
+  cell_layout(cnt + ((size_t)pair * ncell + c) * NID_NCLS, L, s);
   if (threadIdx.x == 0) {
     int* o = tot + ((size_t)blockIdx.y * ncell + c) * 3;
     o[0] = s.T; o[1] = s.S; o[2] = s.slots;
@@ -346,7 +327,7 @@ __global__ void __launch_bounds__(NID_LAYOUT_THREADS) k_layout_write(EvalParams 
                                                                      int* __restrict__ cls_task_start) {
   __shared__ CellLayoutSm s;
   const int c = blockIdx.x, pair = pair0 + blockIdx.y;
-  cell_layout(cnt + ((size_t)pair * p.ncell + c) * NID_NCLS, L, s, p.span_mode ? p.lut_k : nullptr, p.bins - 3);
+  cell_layout(cnt + ((size_t)pair * p.ncell + c) * NID_NCLS, L, s);
   const int* bs = base + ((size_t)blockIdx.y * p.ncell + c) * 3;
   const int tb = bs[0], sb = bs[1], pb = bs[2];
   if (tb + s.T > p.max_tasks || sb + s.S > p.max_slices) return;  // flagged by k_layout_scan
@@ -567,31 +548,10 @@ __device__ __forceinline__ uint4 gather_u32(cudaTextureObject_t tex, int ix, int
 // a rounding-level identity is a bin whose clamped sum is exactly zero in the reference while U-sums cancel only
 // to rounding: that happens iff every contributing pixel sits at u == 0 exactly (N_1(0) = N_2(0) = 0), so pixels
 // with u == 0 are counted apart and enter bin 0 with weight exactly 1.
-// (64-bit literals cost two instructions each time the compiler has to re-materialise one under register pressure;
-// read from the constant bank they are plain operands of the fp64 instructions: NID_KC)
-#ifndef NID_KC
-#define NID_KC 0  // measured: the compiler hoists the constant loads into registers and spills more (136.7k vs 141.5k evals/s)
-#endif
-__constant__ double kc_[8] = {1.0 / 6.0, 0.5, 2.0 / 3.0, 1.0, 1.5, 2.0, 0.0, 0.0};
-#if NID_KC
-#define KC_S6 kc_[0]
-#define KC_H kc_[1]
-#define KC_23 kc_[2]
-#define KC_1 kc_[3]
-#define KC_15 kc_[4]
-#define KC_2 kc_[5]
-#else
-#define KC_S6 (1.0 / 6.0)
-#define KC_H 0.5
-#define KC_23 (2.0 / 3.0)
-#define KC_1 1.0
-#define KC_15 1.5
-#define KC_2 2.0
-#endif
 __device__ __forceinline__ void bspline4_uniform(double f, double w[4]) {
-  const double s6 = KC_S6, h = KC_H;
+  const double s6 = 1.0 / 6.0, h = 0.5;
   w[0] = fma(f, fma(f, fma(f, -s6, h), -h), s6);
-  w[1] = fma(f * f, fma(f, h, -KC_1), KC_23);
+  w[1] = fma(f * f, fma(f, h, -1.0), 2.0 / 3.0);
   w[2] = fma(f, fma(f, fma(f, -h, h), h), s6);
   w[3] = f * f * f * s6;
 }
@@ -617,15 +577,6 @@ __device__ __forceinline__ void fold_table(double* w, int stride, int B) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// The sliced pixel store is read once per evaluation: evict-first loads (ld.global.cs)
-#ifndef NID_STREAM_LOADS
-#define NID_STREAM_LOADS 1
-#endif
-#if NID_STREAM_LOADS
-#define NID_LD_STREAM(p) __ldcs(p)
-#else
-#define NID_LD_STREAM(p) (*(p))
-#endif
 // One group = four consecutive pixels of a lane's task (32 B of depths + 16 B of pixel ids per lane).
 template <bool PTS>
 struct Group {
@@ -633,13 +584,13 @@ struct Group {
   double a0[4], a1[4], a2[4];
   __device__ __forceinline__ void load(const double* q0, const double* q1, const double* q2, const unsigned* qi, size_t o) {
     // read-once stream: evict-first loads keep L1 for the target-image gathers
-    const uint4 i4 = NID_LD_STREAM(reinterpret_cast<const uint4*>(qi + o));
+    const uint4 i4 = __ldcs(reinterpret_cast<const uint4*>(qi + o));
     id[0] = i4.x; id[1] = i4.y; id[2] = i4.z; id[3] = i4.w;
-    const double2 xa = NID_LD_STREAM(reinterpret_cast<const double2*>(q0 + o)), xb = NID_LD_STREAM(reinterpret_cast<const double2*>(q0 + o + 2));
+    const double2 xa = __ldcs(reinterpret_cast<const double2*>(q0 + o)), xb = __ldcs(reinterpret_cast<const double2*>(q0 + o + 2));
     a0[0] = xa.x; a0[1] = xa.y; a0[2] = xb.x; a0[3] = xb.y;
     if (PTS) {
-      const double2 ya = NID_LD_STREAM(reinterpret_cast<const double2*>(q1 + o)), yb = NID_LD_STREAM(reinterpret_cast<const double2*>(q1 + o + 2));
-      const double2 za = NID_LD_STREAM(reinterpret_cast<const double2*>(q2 + o)), zb = NID_LD_STREAM(reinterpret_cast<const double2*>(q2 + o + 2));
+      const double2 ya = __ldcs(reinterpret_cast<const double2*>(q1 + o)), yb = __ldcs(reinterpret_cast<const double2*>(q1 + o + 2));
+      const double2 za = __ldcs(reinterpret_cast<const double2*>(q2 + o)), zb = __ldcs(reinterpret_cast<const double2*>(q2 + o + 2));
       a1[0] = ya.x; a1[1] = ya.y; a1[2] = yb.x; a1[3] = yb.y;
       a2[0] = za.x; a2[1] = za.y; a2[2] = zb.x; a2[3] = zb.y;
     } else {
@@ -649,25 +600,8 @@ struct Group {
   }
 };
 
-// ---- Blackwell/Hopper bulk-copy path of the pixel store (depth form): every warp owns a small ring of stages in shared
-// memory; one elected lane queues the groups of the warp's slice as 1-D bulk copies (cp.async.bulk, executed by the
-// TMA unit: no registers, no LSU instructions, no per-lane address arithmetic) that complete on an mbarrier per stage;
-// the lanes wait on the barrier's phase and read their four pixels with 128-bit shared loads. Compared with the
-// register double-buffer this frees the twelve registers of the prefetched group and all of the prefetch code.
-#ifndef NID_BULK
-#define NID_BULK 0  // measured at C2: 123.9k evals/s with the ring (3 stages), 141.8k with the register double-buffer: the ring
-                    // takes 18 KB of shared memory per CTA out of the L1 that serves the target-image gathers
-#endif
-#ifndef NID_BULK_STAGES
-#define NID_BULK_STAGES 3
-#endif
-#ifndef NID_BULK_FENCE
-#define NID_BULK_FENCE 0
-#endif
-struct __align__(16) BulkStage {
-  double z[128];    // group g of the slice: lane l owns z[4 l .. 4 l + 3]
-  unsigned id[128];
-};
+// mbarrier and bulk-copy (cp.async.bulk) helpers: pass 2 of small cells stages the cell's log tables by one bulk copy
+// (k_jac_sell, BULK)
 __device__ __forceinline__ unsigned smem_u32(const void* ptr) { return (unsigned)__cvta_generic_to_shared(ptr); }
 __device__ __forceinline__ void mbar_init(unsigned long long* bar, int count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
@@ -690,49 +624,6 @@ __device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned pari
       "DONE:\n"
       "}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
 }
-// the warp's ring: stages, barriers; issue() is called by one lane
-struct BulkRing {
-  BulkStage* st;
-  unsigned long long* bar;
-  const double* gz;      // the slice's depths in the pixel store (warp base)
-  const unsigned* gid;   // ... and pixel ids
-  int nst;
-  __device__ __forceinline__ void init(int lane) {
-    if (lane == 0)
-      for (int s = 0; s < nst; s++) mbar_init(bar + s, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncwarp();
-  }
-  __device__ __forceinline__ void issue(int g) const {
-    const int s = g % nst;
-    mbar_expect_tx(bar + s, (unsigned)sizeof(BulkStage));
-    bulk_g2s(st[s].z, gz + (size_t)g * 128, 1024u, bar + s);
-    bulk_g2s(st[s].id, gid + (size_t)g * 128, 512u, bar + s);
-  }
-  // group g into registers (all lanes), then the stage is handed back to the copy engine for group g + nst
-  template <bool PTS>
-  __device__ __forceinline__ void take(int g, int ngroups, int lane, Group<PTS>& G) const {
-    const int s = g % nst;
-    mbar_wait(bar + s, (unsigned)((g / nst) & 1));
-    const double2 xa = *reinterpret_cast<const double2*>(st[s].z + 4 * lane), xb = *reinterpret_cast<const double2*>(st[s].z + 4 * lane + 2);
-    const uint4 i4 = *reinterpret_cast<const uint4*>(st[s].id + 4 * lane);
-    G.a0[0] = xa.x; G.a0[1] = xa.y; G.a0[2] = xb.x; G.a0[3] = xb.y;
-    G.id[0] = i4.x; G.id[1] = i4.y; G.id[2] = i4.z; G.id[3] = i4.w;
-#pragma unroll
-    for (int j = 0; j < 4; j++) { G.a1[j] = 0.0; G.a2[j] = 0.0; }
-    __syncwarp();  // every lane has read the stage
-    if (lane == 0 && g + nst < ngroups) {
-#if NID_BULK_FENCE
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // (compiles to MEMBAR.ALL.CTA + FENCE.VIEW.ASYNC: costly)
-#endif
-      // the stage's reads are complete (their values were consumed before the __syncwarp above could be passed by the
-      // issuing lane's later instructions only in program order; the refill lands hundreds of cycles later)
-      issue(g + nst);
-    }
-  }
-};
-static inline int bulk_stages(int bins) { return bins > 32 ? 2 : NID_BULK_STAGES; }
-static inline size_t bulk_smem(int T, int bins) { return (size_t)(T / 32) * bulk_stages(bins) * (sizeof(BulkStage) + 8); }
 
 // what the rare exact paths need from global memory
 struct ExactSrc {
@@ -761,16 +652,11 @@ __device__ __forceinline__ void make_exact(const ExactSrc& xs, int rows, int col
 // weights, then the accumulations in pixel order into the lane's private row h[b * T] (T = threads per CTA).
 // fp: the pair's footprint-packed target image, fp[y*cols + x] = I(x,y) | I(x+1,y)<<8 | I(x,y+1)<<16 | I(x+1,y+1)<<24.
 // n0 counts the lane's pixels with u == 0 exactly (see bspline4_uniform).
-// MODE 1 (span tasks, small cells): the lane's task holds pixels of one reference SPAN but of any reference intensity;
-// the lane accumulates the four joint-histogram rows of that span, h[(m * B + b) * T] += w_ref,v[m] * w_t[n], with the
-// pixel's reference weights looked up from its intensity byte (vv: the group's four bytes; noref: pixels without a
-// reference sample, weight row (1, 0, 0, 0)); n0m[m]: the reference weights of the pixels with u == 0 exactly.
-template <bool PTS, int W, int T, int MODE = 0>
+template <bool PTS, int W, int T>
 __device__ __forceinline__ void hist_pixels(const double* __restrict__ g, const ExactSrc& xs, int rows, int cols,
                                             const Group<PTS>& G, int j0, const GroupAddr& ga,
                                             const unsigned* __restrict__ fp, double s, int NS, double* __restrict__ h,
-                                            int& n0, const double* __restrict__ lutw = nullptr, unsigned vv = 0u,
-                                            bool noref = false, double* n0m = nullptr) {
+                                            int& n0) {
   Px r[W];
   bool anyexact = false;
 #pragma unroll
@@ -824,37 +710,14 @@ __device__ __forceinline__ void hist_pixels(const double* __restrict__ g, const 
     bspline4_uniform(ub - u2d((unsigned)kt[j]), wt[j]);
     const bool zero = ub == 0.0;
     acc[j] = r[j].ok && !zero;
-    if (MODE == 0) n0 += (r[j].ok && zero) ? 1 : 0;
-    else if (r[j].ok && zero) {
-      const unsigned v = (vv >> (8 * (j0 + j))) & 0xffu;
-#pragma unroll
-      for (int m = 0; m < 4; m++) n0m[m] += noref ? (m == 0 ? 1.0 : 0.0) : __ldg(lutw + 4 * v + m);
-    }
+    n0 += (r[j].ok && zero) ? 1 : 0;
   }
 #pragma unroll
   for (int j = 0; j < W; j++) {
     if (!acc[j]) continue;
-    if (MODE == 0) {
-      double* hk = h + kt[j] * T;
+    double* hk = h + kt[j] * T;
 #pragma unroll
-      for (int n = 0; n < 4; n++) hk[n * T] += wt[j][n];
-    } else {
-      const int B = NS + 3;
-      const unsigned v = (vv >> (8 * (j0 + j))) & 0xffu;
-      if (noref) {
-        double* hk = h + kt[j] * T;
-#pragma unroll
-        for (int n = 0; n < 4; n++) hk[n * T] += wt[j][n];
-      } else {
-#pragma unroll
-        for (int m = 0; m < 4; m++) {
-          const double wr = __ldg(lutw + 4 * v + m);
-          double* hk = h + (m * B + kt[j]) * T;
-#pragma unroll
-          for (int n = 0; n < 4; n++) hk[n * T] = fma(wr, wt[j][n], hk[n * T]);
-        }
-      }
-    }
+    for (int n = 0; n < 4; n++) hk[n * T] += wt[j][n];
   }
 }
 
@@ -914,14 +777,8 @@ __device__ __forceinline__ void store_task_rows(double* hw, int B, int lane, int
 #ifndef NID_HIST_W
 #define NID_HIST_W 4
 #endif
-#ifndef NID_HIST_HALF_LAST
-#define NID_HIST_HALF_LAST 0  // measured: the two-pixel tail step costs pass 1 more than the skipped half step saves (3.69 against 3.60 us at 16x16 cells, 2.45 against 2.31 at 4x4)
-#endif
 #ifndef NID_JAC_W
 #define NID_JAC_W 2
-#endif
-#ifndef NID_JAC_INTTAP
-#define NID_JAC_INTTAP 0
 #endif
 #ifndef NID_HIST_TMAX
 #define NID_HIST_TMAX 32  // largest CTA of pass 1 / pass 2 (pick_block shrinks it when few jobs are in flight); measured best:
@@ -950,16 +807,12 @@ __device__ __forceinline__ void store_task_rows(double* hw, int B, int lane, int
 #define NID_JAC_REGS_SMALL 96
 #endif
 #define NID_JAC_WARPS_SMALL (2048 / NID_JAC_REGS_SMALL)  // resident warps the register file holds at that budget
-#ifndef NID_JAC_NOPF
-#define NID_JAC_NOPF 0
-#endif
 template <bool PTS, int NG, int T>
 __global__ void __launch_bounds__(T, NID_HIST_WARPS * 32 / T)
 k_hist_sell(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTable<NG> gt) {
   extern __shared__ __align__(16) double sm[];
   const int B = p.bins, NS = B - 3;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  // (the job / pair / slice-count entries of the parameter table, which pass 2 uses, cost this kernel 24 bytes of spills)
   // (the job / pair / slice-count entries of the parameter table, which pass 2 uses, cost this kernel 24 bytes of spills:
   // measured slower at 4x4 and at 16x16 cells)
   const int job = job_at(p, NID_BLK_JOB);
@@ -970,10 +823,6 @@ k_hist_sell(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTab
   const int* so = p.sl_off + (size_t)pair * (p.max_slices + 1) + slice;
   const int off0 = so[0], ngroups = (so[1] - off0) >> 7;
   const int task = p.sl_task[((size_t)pair * p.max_slices + slice) * 32 + lane];  // (for the epilogue; requested early)
-#if NID_HIST_HALF_LAST
-  // (see k_jac_sell: the second half of the slice's last group is empty when its longest task ends in the first half)
-  const bool half_last = (((__shfl_sync(0xffffffffu, p.sl_desc[((size_t)pair * p.max_slices + slice) * 32 + lane], 0) & 0x1ff) - 1) & 3) < 2;
-#endif
   double* h = sm + threadIdx.x;  // h[b * T]
   for (int b = 0; b < B; b++) h[b * T] = 0.0;
   const size_t sbase = (size_t)pair * p.sell_cap + off0 + lane * 4;
@@ -986,48 +835,22 @@ k_hist_sell(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTab
   const double s = (double)NS / 255.0;
   int n0 = 0;
   Group<PTS> G;
-  if (NID_BULK && !PTS) {
-    // shared: rows [B][T] | per warp: ring stages | per warp: barriers
-    BulkRing ring;
-    ring.nst = B > 32 ? 2 : NID_BULK_STAGES;
-    ring.st = reinterpret_cast<BulkStage*>(sm + B * T) + warp * ring.nst;
-    ring.bar = reinterpret_cast<unsigned long long*>(reinterpret_cast<BulkStage*>(sm + B * T) + (T >> 5) * ring.nst) + warp * ring.nst;
-    ring.gz = p.sd0 + (size_t)pair * p.sell_cap + off0;
-    ring.gid = p.sid + (size_t)pair * p.sell_cap + off0;
-    ring.init(lane);
-    if (lane == 0)
-      for (int gq = 0; gq < ring.nst && gq < ngroups; gq++) ring.issue(gq);
-    for (int gi = 0; gi < ngroups; gi++) {
-      ring.take<PTS>(gi, ngroups, lane, G);
-      const size_t go = (size_t)gi * 128;
-      const GroupAddr ga{q0 + go, nullptr, nullptr, qi + go};
-#pragma unroll
-      for (int j0 = 0; j0 < 4; j0 += NID_HIST_W) hist_pixels<PTS, NID_HIST_W, T>(g, xs, p.rows, p.cols, G, j0, ga, fp, s, NS, h, n0);
-    }
-  } else {
-    G.load(q0, q1, q2, qi, 0);
-    for (int gi = 0; gi < ngroups; gi++) {
-      Group<PTS> Gn = G;
-      if (gi + 1 < ngroups) Gn.load(q0, q1, q2, qi, (size_t)(gi + 1) * 128);
+  G.load(q0, q1, q2, qi, 0);
+  for (int gi = 0; gi < ngroups; gi++) {
+    Group<PTS> Gn = G;
+    if (gi + 1 < ngroups) Gn.load(q0, q1, q2, qi, (size_t)(gi + 1) * 128);
 #if NID_PREFETCH_L2 > 0
-      if (gi + 1 + NID_PREFETCH_L2 < ngroups) {
-        const size_t po = (size_t)(gi + 1 + NID_PREFETCH_L2) * 128;
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(q0 + po));
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(qi + po));
-      }
-#endif
-      const size_t go = (size_t)gi * 128;
-      const GroupAddr ga{q0 + go, PTS ? q1 + go : nullptr, PTS ? q2 + go : nullptr, qi + go};
-#if NID_HIST_HALF_LAST
-      if (half_last && gi + 1 == ngroups) hist_pixels<PTS, 2, T>(g, xs, p.rows, p.cols, G, 0, ga, fp, s, NS, h, n0);
-      else
-#endif
-      {
-#pragma unroll
-        for (int j0 = 0; j0 < 4; j0 += NID_HIST_W) hist_pixels<PTS, NID_HIST_W, T>(g, xs, p.rows, p.cols, G, j0, ga, fp, s, NS, h, n0);
-      }
-      G = Gn;
+    if (gi + 1 + NID_PREFETCH_L2 < ngroups) {
+      const size_t po = (size_t)(gi + 1 + NID_PREFETCH_L2) * 128;
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(q0 + po));
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(qi + po));
     }
+#endif
+    const size_t go = (size_t)gi * 128;
+    const GroupAddr ga{q0 + go, PTS ? q1 + go : nullptr, PTS ? q2 + go : nullptr, qi + go};
+#pragma unroll
+    for (int j0 = 0; j0 < 4; j0 += NID_HIST_W) hist_pixels<PTS, NID_HIST_W, T>(g, xs, p.rows, p.cols, G, j0, ga, fp, s, NS, h, n0);
+    G = Gn;
   }
   fold_row(h, T, B, (double)n0);  // uniform sums -> sums of the reference's clamped basis
   __syncwarp();
@@ -1047,19 +870,8 @@ k_hist_sell(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTab
 #define NID_ASM_THREADS 256
 #endif
 #define NID_ASM_SMALL 128
-#ifndef NID_ASM_STREAM
-#define NID_ASM_STREAM 1  // task rows are read once: evict-first loads
-#endif
-#if NID_ASM_STREAM
-#define NID_ASM_LD(p) __ldcs(p)
-#else
-#define NID_ASM_LD(p) (*(p))
-#endif
 #ifndef NID_ASM_BATCH
 #define NID_ASM_BATCH 12  // task rows a thread keeps in flight
-#endif
-#ifndef NID_ASM_PAIRS
-#define NID_ASM_PAIRS(B) true
 #endif
 #ifndef NID_ASM_CHUNK
 #define NID_ASM_CHUNK 16  // task rows of a class that are summed in one go (see assemble_body)
@@ -1069,19 +881,9 @@ k_hist_sell(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTab
 #endif
 // NT threads per CTA: 256 in general, 128 for small cells (many cells per job, little work per cell: twice the CTAs
 // resident per SM). Fixed per geometry, so results never depend on how a batch is launched.
-#ifdef NID_ASM_TRACE
-__device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
-#define ASM_T(i) do { __syncthreads(); if (threadIdx.x == 0) tr_[i] = gtimer(); } while (0)
-#else
-#define ASM_T(i)
-#endif
 template <int NT>
 __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac) {
   extern __shared__ __align__(16) double sm[];
-#ifdef NID_ASM_TRACE
-  unsigned long long tr_[12];
-  if (threadIdx.x == 0) tr_[0] = gtimer();
-#endif
   __shared__ double scratch[8];
   __shared__ int s_cts[NID_NCLS + 1];
   __shared__ int s_bnd[NT / 3 + 2];
@@ -1116,10 +918,9 @@ __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac)
     for (int i = threadIdx.x; i <= NS; i += blockDim.x) s_span[i] = p.span_start[i];
     if (NID_FEW_BINS(B)) for (int i = threadIdx.x; i < 1024; i += blockDim.x) wl[i] = p.lut_w[i];
     __syncthreads();
-    ASM_T(1);
     // many bins: a thread owns two adjacent bins of a row (one 16-byte load; rows are 16-byte aligned when B is even),
     // which doubles the number of runs in flight; with few bins there are enough runs already
-    const bool pairs = (B & 1) == 0 && NID_ASM_PAIRS(B);
+    const bool pairs = (B & 1) == 0;
     const int tpr = pairs ? B >> 1 : B;  // threads per row
     const int ng = NT / tpr;
     const int tfirst = s_cts[0], tlast = s_cts[NID_NCLS], ntask = tlast - tfirst;
@@ -1141,7 +942,6 @@ __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac)
       if (s_cts[v + 1] == s_cts[v]) hvs[i] = 0.0;
     }
     __syncthreads();
-    ASM_T(7);
     const int g = threadIdx.x / tpr, tt = (threadIdx.x % tpr) * (pairs ? 2 : 1);
     double* Gjob = p.G + (size_t)job * p.g_stride * B;
     if (g < ng && s_bnd[g] < s_bnd[g + 1]) {
@@ -1197,7 +997,7 @@ __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac)
           const int rem = tend - t;
           double x[NID_ASM_BATCH];
 #pragma unroll
-          for (int i = 0; i < NID_ASM_BATCH; i++) x[i] = (i < rem) ? NID_ASM_LD(gp + i * B) : 0.0;
+          for (int i = 0; i < NID_ASM_BATCH; i++) x[i] = (i < rem) ? __ldcs(gp + i * B) : 0.0;  // (read once: evict-first)
 #pragma unroll
           for (int i = 0; i < NID_ASM_BATCH; i++) {
             if (i < rem) {
@@ -1212,7 +1012,6 @@ __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac)
       close_segment();
     }
     __syncthreads();  // (the chunk sums this CTA parked in G are visible to all of its threads)
-    ASM_T(8);
     if (g < ng) {
       for (int v = g; v < NID_NCLS; v += ng) {
         const int m = s_cts[v + 1] - s_cts[v];
@@ -1241,7 +1040,6 @@ __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac)
     }
   }
   __syncthreads();
-  ASM_T(2);
   // ---- P_j: item (kk, r, t) sums the classes of span r-kk (in class order: the summation order is part of the result)
   {
     const unsigned mdiv = (1048576u + (unsigned)B - 1u) / (unsigned)B;  // idx / B == (idx * mdiv) >> 20 for idx < 2^20 / B
@@ -1281,7 +1079,6 @@ __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac)
     red[threadIdx.x] = a;
   }
   __syncthreads();
-  ASM_T(3);
   for (int idx = threadIdx.x; idx < BB; idx += blockDim.x) {
     const double a = ((part[idx] + part[BB + idx]) + part[2 * BB + idx]) + part[3 * BB + idx];
     const double q = a / (double)nc;
@@ -1301,7 +1098,6 @@ __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac)
     red[tt] = (q < kSigma) ? 0.0 : 1.0 + lg;
   }
   __syncthreads();
-  ASM_T(4);
   // ---- H_j: 128 partial sums (partial j takes the terms j, j + 128, ... in order), an xor tree inside each of the four
   // warps, the four warp sums in order. H_t: the same with one warp's worth of partials.
   {
@@ -1322,7 +1118,6 @@ __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac)
   __syncthreads();
   const double Hj = ((scratch[0] + scratch[1]) + scratch[2]) + scratch[3];
   const double Ht = scratch[4];
-  ASM_T(5);
   const double Href = p.href[pair * p.ncell + c];
   if (threadIdx.x == 0) {
     p.ht[o] = Ht; p.hj[o] = Hj;
@@ -1343,12 +1138,6 @@ __device__ __forceinline__ void assemble_body(const EvalParams& p, int want_jac)
     }
     if ((int)threadIdx.x < B) wv[B * BP + threadIdx.x] = red[threadIdx.x] * coefT;
   }
-#ifdef NID_ASM_TRACE
-  ASM_T(6);
-  if (threadIdx.x == 0)
-    printf("asm cell %d job %d start %llu end %llu: (bnd %llu stream %llu fold %llu) prologue %llu rows %llu pj %llu entropy %llu sums %llu tables %llu ns\n", c, job, tr_[0] % 10000000ull, tr_[6] % 10000000ull, tr_[7] - tr_[1], tr_[8] - tr_[7], tr_[2] - tr_[8], tr_[1] - tr_[0], tr_[2] - tr_[1],
-           tr_[3] - tr_[2], tr_[4] - tr_[3], tr_[5] - tr_[4], tr_[6] - tr_[5]);
-#endif
 }
 
 __global__ void __launch_bounds__(NID_ASM_THREADS, NID_ASM_MINB) k_assemble(EvalParams p, int want_jac) {
@@ -1424,7 +1213,7 @@ __global__ void __launch_bounds__(NID_ASMW_WARPS * 32, BATCH > 8 ? 1 : NID_ASMW_
 #pragma unroll
     for (int i = 0; i < BATCH; i++) {
       const bool in = mine && tb + i * NG + g < t1;
-      x[i] = in ? NID_ASM_LD(gp + i * rstep) : 0.0;
+      x[i] = in ? __ldcs(gp + i * rstep) : 0.0;  // (read once: evict-first)
       cls[i] = in ? (int)__ldg(tcp + i * NG) : 256;
     }
 #pragma unroll
@@ -1531,16 +1320,11 @@ __device__ __forceinline__ double tapd(unsigned v) { return __hiloint2double(0x4
 
 // Pass 2 on W pixels of a group at once; acc[6] are the lane's Jacobian partial sums.
 // wq: the lane's folded class table (fold_table), element t at wq[t * T].
-// MODE 1 (span tasks): wq points at the warp's staged, folded tables W^ (rows padded to BP = B + 1) followed by V^; the
-// lane's task belongs to reference span kr and every pixel brings its own reference weights (looked up from its
-// intensity byte): c_i = sum_n U'_n(f) (V^[k+n] + sum_m w_ref,v[m] W^[kr+m][k+n]).
-template <bool PTS, int W, int T, int MODE = 0>
+template <bool PTS, int W, int T>
 __device__ __forceinline__ void jac_pixels(const double* __restrict__ g, const ExactSrc& xs, int rows, int cols,
                                            const Group<PTS>& G, int j0, cudaTextureObject_t tex2,
                                            const uint8_t* __restrict__ im1, double s, int NS, double hfx, double hfy,
-                                           const double* __restrict__ wq, double acc[6],
-                                           const double* __restrict__ lutw = nullptr, unsigned vv = 0u, bool noref = false,
-                                           int kr = 0) {
+                                           const double* __restrict__ wq, double acc[6]) {
   Px r[W];
 #pragma unroll
   for (int j = 0; j < W; j++) front<PTS, false>(g, rows, cols, G.a0[j0 + j], G.a1[j0 + j], G.a2[j0 + j], G.id[j0 + j], r[j]);
@@ -1550,14 +1334,6 @@ __device__ __forceinline__ void jac_pixels(const double* __restrict__ g, const E
 #pragma unroll
   for (int j = 0; j < W; j++) {
     // texel = I | (Gx+256) << 8 | (Gy+256) << 17; the biases cancel in the differences
-#if NID_JAC_INTTAP
-    const int i00 = t[j].w & 0xffu, i01 = t[j].z & 0xffu, i10 = t[j].x & 0xffu, i11 = t[j].y & 0xffu;
-    const int x00 = (t[j].w >> 8) & 0x1ffu, x01 = (t[j].z >> 8) & 0x1ffu, x10 = (t[j].x >> 8) & 0x1ffu, x11 = (t[j].y >> 8) & 0x1ffu;
-    const int y00 = t[j].w >> 17, y01 = t[j].z >> 17, y10 = t[j].x >> 17, y11 = t[j].y >> 17;
-    double ic = bilinear_fast(r[j].dx, r[j].dy, u2d(i00), i2d_small(i01 - i00), u2d(i10), i2d_small(i11 - i10));
-    double gx2 = bilinear_fast(r[j].dx, r[j].dy, i2d_small(x00 - 256), i2d_small(x01 - x00), i2d_small(x10 - 256), i2d_small(x11 - x10));
-    double gy2 = bilinear_fast(r[j].dx, r[j].dy, i2d_small(y00 - 256), i2d_small(y01 - y00), i2d_small(y10 - 256), i2d_small(y11 - y10));
-#else
     const double two52 = 4503599627370496.0;
     const double i00 = tapd(t[j].w & 0xffu), i01 = tapd(t[j].z & 0xffu), i10 = tapd(t[j].x & 0xffu), i11 = tapd(t[j].y & 0xffu);
     const double x00 = tapd((t[j].w >> 8) & 0x1ffu), x01 = tapd((t[j].z >> 8) & 0x1ffu);
@@ -1566,7 +1342,6 @@ __device__ __forceinline__ void jac_pixels(const double* __restrict__ g, const E
     double ic = bilinear_fast(r[j].dx, r[j].dy, i00 - two52, i01 - i00, i10 - two52, i11 - i10);
     double gx2 = bilinear_fast(r[j].dx, r[j].dy, x00 - (two52 + 256.0), x01 - x00, x10 - (two52 + 256.0), x11 - x10);
     double gy2 = bilinear_fast(r[j].dx, r[j].dy, y00 - (two52 + 256.0), y01 - y00, y10 - (two52 + 256.0), y11 - y10);
-#endif
     // rare: undecided by the fast path, saturated plateau, or first image row / column
     const bool sat = (t[j].w & t[j].z & t[j].x & t[j].y & 0xffu) == 0xffu;
     if (r[j].fix || (r[j].jac && (sat || r[j].ix < 1 || r[j].iy < 1))) {
@@ -1581,30 +1356,12 @@ __device__ __forceinline__ void jac_pixels(const double* __restrict__ g, const E
     const int k = min((int)ub, NS - 1);  // 0 <= ub <= NS (== NS only by rounding)
     const double f = ub - u2d((unsigned)k);
     // c_i = sum_m N'_{k+m}(u_i) Wv[k+m] = sum_m U'_m(f) W^v[k+m]: uniform cubic derivative, folded class table
-    const double dw0 = fma(f, fma(f, -KC_H, KC_1), -KC_H);
-    const double dw1 = f * fma(f, KC_15, -KC_2);
-    const double dw2 = fma(f, fma(f, -KC_15, KC_1), KC_H);
-    const double dw3 = KC_H * f * f;
-    double ci;
-    if (MODE == 0) {
-      const double* q = wq + k * T;
-      ci = fma(dw3, q[3 * T], fma(dw2, q[2 * T], fma(dw1, q[T], dw0 * q[0])));
-    } else {
-      const int B = NS + 3, BP = B + 1;
-      const double* V = wq + B * BP + k;
-      double c0 = V[0], c1 = V[1], c2 = V[2], c3 = V[3];
-      if (!noref) {
-        const unsigned v = (vv >> (8 * (j0 + j))) & 0xffu;
-        const double* Wr = wq + kr * BP + k;
-#pragma unroll
-        for (int m = 0; m < 4; m++) {
-          const double wr = __ldg(lutw + 4 * v + m);
-          c0 = fma(wr, Wr[m * BP], c0); c1 = fma(wr, Wr[m * BP + 1], c1);
-          c2 = fma(wr, Wr[m * BP + 2], c2); c3 = fma(wr, Wr[m * BP + 3], c3);
-        }
-      }
-      ci = fma(dw3, c3, fma(dw2, c2, fma(dw1, c1, dw0 * c0)));
-    }
+    const double dw0 = fma(f, fma(f, -0.5, 1.0), -0.5);
+    const double dw1 = f * fma(f, 1.5, -2.0);
+    const double dw2 = fma(f, fma(f, -1.5, 1.0), 0.5);
+    const double dw3 = 0.5 * f * f;
+    const double* q = wq + k * T;
+    double ci = fma(dw3, q[3 * T], fma(dw2, q[2 * T], fma(dw1, q[T], dw0 * q[0])));
     if (ub == 0.0) ci = 0.0;  // the reference's BsplineDer quirk
     if (!r[j].jac) continue;  // (a padding slot may carry z = 0 and non-finite coordinates)
     // d(u,v)/d(xi), types_six_dof_expmap.cpp:438-450, in normalised coordinates xn = x/z, yn = y/z
@@ -1651,22 +1408,7 @@ k_jac_sell(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTabl
   const double* q2 = PTS ? p.sd2 + sbase : nullptr;
   const unsigned* qi = p.sid + sbase;
   Group<PTS> G;
-  BulkRing ring;
-  if (NID_BULK && !PTS) {
-    // shared: class tables [B][T] | per-warp log tables (few bins) | per warp: ring stages | per warp: barriers
-    ring.nst = B > 32 ? 2 : NID_BULK_STAGES;
-    double* after = sm + B * T + (NID_FEW_BINS(B) ? (T >> 5) * (wv_stride(B) + 1) : 0);
-    after += (B * T + (NID_FEW_BINS(B) ? (T >> 5) * (wv_stride(B) + 1) : 0)) & 1;  // 16-byte alignment of the stages
-    ring.st = reinterpret_cast<BulkStage*>(after) + warp * ring.nst;
-    ring.bar = reinterpret_cast<unsigned long long*>(reinterpret_cast<BulkStage*>(after) + (T >> 5) * ring.nst) + warp * ring.nst;
-    ring.gz = p.sd0 + (size_t)pair * p.sell_cap + off0;
-    ring.gid = p.sid + (size_t)pair * p.sell_cap + off0;
-    ring.init(lane);
-    if (lane == 0)
-      for (int gq = 0; gq < ring.nst && gq < ngroups; gq++) ring.issue(gq);  // (in flight while the class table is built)
-  } else {
-    G.load(q0, q1, q2, qi, 0);
-  }
+  G.load(q0, q1, q2, qi, 0);
   // ---- class table of the lane's task (class v, cell of the slice):
   //   Wv[t] = V[t] + sum_kk w_ref,v[kk] W[k_r(v)+kk][t]     (class 256: V only)
   // from the cell's scaled log tables W|V (k_assemble), staged per warp with rows padded to B+1, then folded onto
@@ -1740,45 +1482,22 @@ k_jac_sell(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTabl
   const double s = (double)NS / 255.0;
   const double hfx = 0.5 * g[16], hfy = 0.5 * g[17];  // the /2 of the central differences folded in
   double acc[6] = {0, 0, 0, 0, 0, 0};
-  if (NID_BULK && !PTS) {
-    for (int gi = 0; gi < ngroups; gi++) {
-      ring.take<PTS>(gi, ngroups, lane, G);
-#pragma unroll
-      for (int j0 = 0; j0 < 4; j0 += NID_JAC_W) jac_pixels<PTS, NID_JAC_W, T>(g, xs, p.rows, p.cols, G, j0, tex2, im1, s, NS, hfx, hfy, wq, acc);
-    }
-  } else {
-#if NID_JAC_NOPF
-    // no register double-buffer: the group is loaded when it is needed (it was pulled into L2 two groups earlier);
-    // twelve registers less per thread
-    for (int gi = 0; gi < ngroups; gi++) {
-      if (gi > 0) G.load(q0, q1, q2, qi, (size_t)gi * 128);
-      if (gi + 2 < ngroups) {
-        const size_t po = (size_t)(gi + 2) * 128;
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(q0 + po));
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(qi + po));
-      }
-#pragma unroll
-      for (int j0 = 0; j0 < 4; j0 += NID_JAC_W) jac_pixels<PTS, NID_JAC_W, T>(g, xs, p.rows, p.cols, G, j0, tex2, im1, s, NS, hfx, hfy, wq, acc);
-    }
-#else
-    for (int gi = 0; gi < ngroups; gi++) {
-      Group<PTS> Gn = G;
-      if (gi + 1 < ngroups) Gn.load(q0, q1, q2, qi, (size_t)(gi + 1) * 128);
+  for (int gi = 0; gi < ngroups; gi++) {
+    Group<PTS> Gn = G;
+    if (gi + 1 < ngroups) Gn.load(q0, q1, q2, qi, (size_t)(gi + 1) * 128);
 #if NID_PREFETCH_L2 > 0
-      if (gi + 1 + NID_PREFETCH_L2 < ngroups) {
-        const size_t po = (size_t)(gi + 1 + NID_PREFETCH_L2) * 128;
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(q0 + po));
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(qi + po));
-      }
-#endif
-#pragma unroll
-      for (int j0 = 0; j0 < 4; j0 += NID_JAC_W) {
-        if (BULK && j0 >= 2 && half_last && gi + 1 == ngroups) break;  // (small cells only: 5.07 -> 4.98 us; at 4x4 cells 3.43 -> 3.48)
-        jac_pixels<PTS, NID_JAC_W, T>(g, xs, p.rows, p.cols, G, j0, tex2, im1, s, NS, hfx, hfy, wq, acc);
-      }
-      G = Gn;
+    if (gi + 1 + NID_PREFETCH_L2 < ngroups) {
+      const size_t po = (size_t)(gi + 1 + NID_PREFETCH_L2) * 128;
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(q0 + po));
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(qi + po));
     }
 #endif
+#pragma unroll
+    for (int j0 = 0; j0 < 4; j0 += NID_JAC_W) {
+      if (BULK && j0 >= 2 && half_last && gi + 1 == ngroups) break;  // (small cells only: 5.07 -> 4.98 us; at 4x4 cells 3.43 -> 3.48)
+      jac_pixels<PTS, NID_JAC_W, T>(g, xs, p.rows, p.cols, G, j0, tex2, im1, s, NS, hfx, hfy, wq, acc);
+    }
+    G = Gn;
   }
   // one partial per slice: fixed-order butterfly over the 32 lanes (lanes without a task hold zeros)
 #pragma unroll
@@ -1793,227 +1512,6 @@ k_jac_sell(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTabl
 #pragma unroll
     for (int k = 1; k < 6; k++) vv = lane == k ? acc[k] : vv;
     p.jpart[((size_t)job * p.max_slices + slice) * 6 + lane] = vv;
-  }
-}
-
-// ================================================================================================ span tasks
-// Small cells (the reference's default 16x16 cells of a 640x480 image hold 1200 pixels: fewer than five per reference
-// intensity) are a poor fit for (cell, class) tasks: a task is a handful of pixels, and the per-task and per-slice work
-// (row set-up, fold, row store, class table) outweighs the pixels. There the valid pixels of a cell are regrouped by
-// reference SPAN k_r instead (B - 3 spans plus one for pixels without a reference sample), tasks are full runs of L
-// pixels again, and what the class factorisation saved is paid per pixel: the lane keeps the four joint-histogram rows
-// of its span, 16 accumulations per pixel instead of 4 (pass 1), and pass 2 forms the pixel's table entry from the
-// four reference weights instead of reading a per-class table. The pixel's reference intensity travels with it (one
-// byte per pixel slot, plane `sv`). Everything else -- front end, exact paths, uniform basis and fold -- is shared.
-template <int NG, int T>
-__global__ void __launch_bounds__(T, NID_HIST_MINB * 256 / T)
-k_hist_span(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTable<NG> gt) {
-  extern __shared__ __align__(16) double sm[];
-  const int B = p.bins, NS = B - 3;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int job = job_at(p, NID_BLK_JOB);
-  const int pair = p.job_pair[job];
-  const double* g = gt.g[NID_BLK_JOB];
-  const int slice = NID_BLK_CHUNK * (T >> 5) + warp;
-  if (slice >= p.nslices[pair]) return;  // (no block-wide barrier below)
-  const int* so = p.sl_off + (size_t)pair * (p.max_slices + 1) + slice;
-  const int off0 = so[0], ngroups = (so[1] - off0) >> 7;
-  const int task = p.sl_task[((size_t)pair * p.max_slices + slice) * 32 + lane];
-  const int span = task >= 0 ? ((p.tasks[(size_t)pair * p.max_tasks + task].y >> 9) & 0x1ff) : NS;
-  const bool noref = span >= NS;
-  double* h = sm + threadIdx.x;  // h[(m * B + b) * T]
-  for (int b = 0; b < 4 * B; b++) h[b * T] = 0.0;
-  const size_t sbase = (size_t)pair * p.sell_cap + off0 + lane * 4;
-  const double* q0 = p.sd0 + sbase;
-  const unsigned* qi = p.sid + sbase;
-  const unsigned* qv = reinterpret_cast<const unsigned*>(p.sv + sbase);  // four intensity bytes per group and lane
-  const unsigned* fp = p.fp1 + (size_t)pair * p.N;
-  const ExactSrc xs{p.poses + 16 * job, p.Twc0 + 16 * pair, p.cam + 4 * pair};
-  const double s = (double)NS / 255.0;
-  int n0 = 0;
-  double n0m[4] = {0.0, 0.0, 0.0, 0.0};
-  Group<false> G;
-  G.load(q0, nullptr, nullptr, qi, 0);
-  unsigned vv = NID_LD_STREAM(qv);
-  for (int gi = 0; gi < ngroups; gi++) {
-    Group<false> Gn = G;
-    unsigned vn = vv;
-    if (gi + 1 < ngroups) { Gn.load(q0, nullptr, nullptr, qi, (size_t)(gi + 1) * 128); vn = NID_LD_STREAM(qv + (size_t)(gi + 1) * 32); }
-    const size_t go = (size_t)gi * 128;
-    const GroupAddr ga{q0 + go, nullptr, nullptr, qi + go};
-#pragma unroll
-    for (int j0 = 0; j0 < 4; j0 += NID_HIST_W)
-      hist_pixels<false, NID_HIST_W, T, 1>(g, xs, p.rows, p.cols, G, j0, ga, fp, s, NS, h, n0, p.lut_w, vv, noref, n0m);
-    G = Gn;
-    vv = vn;
-  }
-  // uniform sums -> sums of the reference's clamped basis, row by row; then the four rows go out
-  double* Gj = p.G + (size_t)job * p.g_stride * (4 * B);
-#pragma unroll 1
-  for (int m = 0; m < 4; m++) {
-    fold_row(h + m * B * T, T, B, n0m[m]);
-    __syncwarp();
-    store_task_rows<T>(sm + (size_t)m * B * T + (threadIdx.x & ~31), B, lane, task, Gj + m * B, (size_t)4 * B);
-  }
-}
-
-// Assembly for span tasks: one warp per (cell, job) as in k_assemble_warp; a task of span k brings four rows,
-// P_j[k+m][t] += row_m[t], and P_t[t] is the sum of all rows (the four reference weights of a pixel add up to 1).
-__global__ void __launch_bounds__(NID_ASMW_WARPS * 32, NID_ASMW_MINB) k_assemble_span(EvalParams p, int want_jac, int n_jobs) {
-  extern __shared__ __align__(16) double sm[];
-  const int B = p.bins, BB = B * B, NS = B - 3;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int unit = blockIdx.x * NID_ASMW_WARPS + warp;
-  if (unit >= n_jobs * p.ncell) return;
-  const int c = unit % p.ncell, job = job_at(p, unit / p.ncell);
-  const int pair = p.job_pair[job];
-  const int nc = p.n_c[pair * p.ncell + c];
-  const size_t o = (size_t)job * p.ncell + c;
-  if (nc < NID_MIN_CELL_POINTS) {
-    if (lane == 0) { p.ht[o] = nan(""); p.hj[o] = nan(""); p.err[o] = nan(""); }
-    return;
-  }
-  const int NGR = 32 / B;
-  const int g = lane / B, t = lane - g * B;
-  const bool mine = g < NGR;
-  const int stride = BB + B;
-  double* cp = sm + (size_t)warp * NGR * stride;
-  for (int i = lane; i < NGR * stride; i += 32) cp[i] = 0.0;
-  __syncwarp();
-  double* Pj = cp + (mine ? g : 0) * stride + t;
-  double pt = 0.0;
-  const int t0 = p.cell_task_start[pair * (p.ncell + 1) + c], t1 = p.cell_task_start[pair * (p.ncell + 1) + c + 1];
-  const int2* tk = p.tasks + (size_t)pair * p.max_tasks;
-  const double* G = p.G + (size_t)job * p.g_stride * (4 * B) + t;
-  for (int tb = t0; tb < t1; tb += 2 * NGR) {  // two tasks (eight rows) in flight per sub-group
-    double x[2][4];
-    int sp[2];
-#pragma unroll
-    for (int i = 0; i < 2; i++) {
-      const int tt = tb + i * NGR + g;
-      const bool in = mine && tt < t1;
-#pragma unroll
-      for (int m = 0; m < 4; m++) x[i][m] = in ? NID_ASM_LD(G + ((size_t)tt * 4 + m) * B) : 0.0;
-      sp[i] = in ? ((tk[tt].y >> 9) & 0x1ff) : NS;
-    }
-#pragma unroll
-    for (int i = 0; i < 2; i++) {
-      pt += (x[i][0] + x[i][1]) + (x[i][2] + x[i][3]);
-      if (sp[i] < NS) {
-        double* q = Pj + sp[i] * B;
-#pragma unroll
-        for (int m = 0; m < 4; m++) q[m * B] += x[i][m];
-      }
-    }
-  }
-  if (mine) cp[g * stride + BB + t] = pt;
-  __syncwarp();
-  for (int i = lane; i < stride; i += 32) {
-    double a = cp[i];
-    for (int k = 1; k < NGR; k++) a += cp[k * stride + i];
-    cp[i] = a;
-  }
-  __syncwarp();
-  double ej = 0.0, et = 0.0;
-  const double dn = (double)nc;
-  double* hist = p.hist ? p.hist + o * (size_t)(BB + B) : nullptr;
-  for (int i = lane; i < stride; i += 32) {
-    const double q = cp[i] / dn;
-    const double lg = (q < kSigma) ? 0.0 : log2(q);
-    if (i < BB) ej -= q * lg; else et -= q * lg;
-    cp[i] = (q < kSigma) ? 0.0 : 1.0 + lg;
-    if (hist) hist[i] = q;
-  }
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) {
-    ej += __shfl_xor_sync(0xffffffffu, ej, off);
-    et += __shfl_xor_sync(0xffffffffu, et, off);
-  }
-  const double Hj = ej, Ht = et;
-  const double Href = p.href[pair * p.ncell + c];
-  if (lane == 0) {
-    p.ht[o] = Ht; p.hj[o] = Hj;
-    p.err[o] = (2 * Hj - Href - Ht) / Hj;
-  }
-  __syncwarp();
-  if (want_jac) {
-    const double s_over = ((double)(B - 3) / 255.0) / ((double)nc * Hj * Hj);
-    const double coefJ = -s_over * (Ht + Href);
-    const double coefT = s_over * Hj;
-    const int BP = wv_row(B);
-    const unsigned mdiv = (1048576u + (unsigned)B - 1u) / (unsigned)B;
-    double* wv = p.wv + o * (size_t)wv_stride(B);
-    for (int i = lane; i < stride; i += 32) {
-      const int r = (int)(((unsigned)i * mdiv) >> 20);  // (i >= BB: r = B, the row of V)
-      wv[r * BP + (i - r * B)] = cp[i] * (i < BB ? coefJ : coefT);
-    }
-  }
-}
-
-// Pass 2 for span tasks: the warp stages the cell's scaled log tables W | V (rows padded to B + 1), folds every row
-// (and V) onto the uniform basis along the target index, and every pixel evaluates its own table entry.
-template <int NG, int T>
-__global__ void __launch_bounds__(T, NID_JAC_MINB * 128 / T)
-k_jac_span(const __grid_constant__ EvalParams p, const __grid_constant__ GeoTable<NG> gt) {
-  extern __shared__ __align__(16) double sm[];
-  const int B = p.bins, NS = B - 3, BP = B + 1;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int job = job_at(p, NID_BLK_JOB);
-  const int pair = p.job_pair[job];
-  const double* g = gt.g[NID_BLK_JOB];
-  const int slice = NID_BLK_CHUNK * (T >> 5) + warp;
-  if (slice >= p.nslices[pair]) return;  // (no block-wide barrier below)
-  const int* so = p.sl_off + (size_t)pair * (p.max_slices + 1) + slice;
-  const int off0 = so[0], ngroups = (so[1] - off0) >> 7;
-  const int task = p.sl_task[((size_t)pair * p.max_slices + slice) * 32 + lane];
-  const size_t sbase = (size_t)pair * p.sell_cap + off0 + lane * 4;
-  const double* q0 = p.sd0 + sbase;
-  const unsigned* qi = p.sid + sbase;
-  const unsigned* qv = reinterpret_cast<const unsigned*>(p.sv + sbase);
-  Group<false> G;
-  G.load(q0, nullptr, nullptr, qi, 0);
-  unsigned vv = NID_LD_STREAM(qv);
-  const int span = task >= 0 ? ((p.tasks[(size_t)pair * p.max_tasks + task].y >> 9) & 0x1ff) : NS;
-  const bool noref = span >= NS;
-  double* Ww = sm + (size_t)warp * (B * BP + B + 4);  // W^ [B][BP] | V^ [B] (+ slack: the last span reads V^[k..k+3] with k <= NS-1)
-  {
-    const int cell = p.sl_cell[(size_t)pair * p.max_slices + slice];
-    const double* wvg = p.wv + ((size_t)job * p.ncell + cell) * (size_t)wv_stride(B);
-    double* Vw = Ww + B * BP;
-    for (int i = lane; i < B * BP + B; i += 32) Ww[i] = wvg[i];  // (the block is stored with rows of B + 1 already)
-    __syncwarp();
-    for (int r = lane; r <= B; r += 32) fold_table(r < B ? Ww + r * BP : Vw, 1, B);  // rows of W^, then V^
-    __syncwarp();
-  }
-  const cudaTextureObject_t tex2 = p.tex2[pair];
-  const uint8_t* im1 = p.im1 + (size_t)pair * p.N;
-  const ExactSrc xs{p.poses + 16 * job, p.Twc0 + 16 * pair, p.cam + 4 * pair};
-  const double s = (double)NS / 255.0;
-  const double hfx = 0.5 * g[16], hfy = 0.5 * g[17];
-  const int kr = noref ? 0 : span;
-  double acc[6] = {0, 0, 0, 0, 0, 0};
-  for (int gi = 0; gi < ngroups; gi++) {
-    Group<false> Gn = G;
-    unsigned vn = vv;
-    if (gi + 1 < ngroups) { Gn.load(q0, nullptr, nullptr, qi, (size_t)(gi + 1) * 128); vn = NID_LD_STREAM(qv + (size_t)(gi + 1) * 32); }
-#pragma unroll
-    for (int j0 = 0; j0 < 4; j0 += NID_JAC_W)
-      jac_pixels<false, NID_JAC_W, T, 1>(g, xs, p.rows, p.cols, G, j0, tex2, im1, s, NS, hfx, hfy, Ww, acc, p.lut_w, vv, noref, kr);
-    G = Gn;
-    vv = vn;
-  }
-#pragma unroll
-  for (int k = 0; k < 6; k++) {
-    double vx = acc[k];
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) vx += __shfl_xor_sync(0xffffffffu, vx, off);
-    acc[k] = vx;
-  }
-  if (lane < 6) {
-    double vx = acc[0];
-#pragma unroll
-    for (int k = 1; k < 6; k++) vx = lane == k ? acc[k] : vx;
-    p.jpart[((size_t)job * p.max_slices + slice) * 6 + lane] = vx;
   }
 }
 
@@ -2168,9 +1666,6 @@ __device__ __noinline__ unsigned warp_sample_literal(const EvalParams& p, int jo
 #ifndef NID_WS_W
 #define NID_WS_W 4
 #endif
-#ifndef NID_WS_ORDER
-#define NID_WS_ORDER 0
-#endif
 // Geometry entries of this kernel (fill_geo_k1): [0..2] A, [3..5] B, [6..8] C with the ray d = A col + B row + C
 // (rows 0 and 1 pre-multiplied by fx, fy), [9..11] translation (same scaling), [12..14] 128 A, [15..17] B - cols A
 // (the step into the next image row), [18] cx, [19] cy.
@@ -2180,11 +1675,7 @@ k_warp_sample_jobs(const __grid_constant__ EvalParams p, const __grid_constant__
                    const double* __restrict__ depth64, const uint16_t* __restrict__ depth16,
                    const double* __restrict__ factor_all, float4* __restrict__ out) {
   constexpr int W = NID_WS_W;
-#if NID_WS_ORDER
-  const int jb = blockIdx.y, cb_ = blockIdx.x;  // chunk index fast: neighbouring CTAs stream one pair
-#else
   const int jb = blockIdx.x, cb_ = blockIdx.y;  // job index fast
-#endif
   const int job = job_at(p, jb);
   const int pair = p.job_pair[job];
   const double* g = gt.g[jb];
@@ -2251,20 +1742,9 @@ k_warp_sample_jobs(const __grid_constant__ EvalParams p, const __grid_constant__
   for (int j = 0; j < W; j++) {
     // one gather per plane: .w (ix,iy) .z (ix+1,iy) .x (ix,iy+1) .y (ix+1,iy+1)
     const float gxc = (float)(jxs[j] + 1), gyc = (float)(jys[j] + 1);
-#ifdef NID_WS_NOGATHER
-    const float4 I = make_float4(gxc, gyc, 3.f, 4.f), X = I, Y = I;
-#else
     const float4 I = tex2Dgather<float4>(tex, gxc, gyc, 0);
-#if defined(NID_WS_G1)
-    const float4 X = make_float4(I.y, I.x, I.w, I.z), Y = make_float4(I.z, I.w, I.x, I.y);
-#elif defined(NID_WS_G2)
-    const float4 X = tex2Dgather<float4>(tex, gxc, gyc + (float)p.rows, 0);
-    const float4 Y = make_float4(I.z + X.x, I.w, I.x, I.y);
-#else
     const float4 X = tex2Dgather<float4>(tex, gxc, gyc + (float)p.rows, 0);
     const float4 Y = tex2Dgather<float4>(tex, gxc, gyc + (float)(2 * p.rows), 0);
-#endif
-#endif
     const float fx_ = dxf[j], fy_ = dyf[j];
     const float w11 = fx_ * fy_, w01 = fx_ - w11, w10 = fy_ - w11, w00 = (1.0f - fx_) - w10;
     float ic = fmaf(w11, I.y, fmaf(w10, I.x, fmaf(w01, I.z, w00 * I.w)));
@@ -2284,9 +1764,6 @@ k_warp_sample_jobs(const __grid_constant__ EvalParams p, const __grid_constant__
     ic = vc ? ic : 0.f;
     gx = vj ? gx : 0.f; gy = vj ? gy : 0.f;
     const float fl = vc ? (vj ? 3.f : 1.f) : 0.f;
-#ifdef NID_WS_NOSTORE
-    if (ic == 123.456f)
-#endif
     if (full || i0 + j * 128 < p.N) __stcs(o + j * 128, make_float4(ic, gx, gy, fl));
   }
 }
@@ -2306,8 +1783,7 @@ int launch_layout_and_scatter(nid_ctx* c, int pair0, int n) {
   EvalParams p = make_params(c, 1);
   const int L = c->task_px;
   const dim3 gcell(c->ncell, n);
-  k_layout_totals<<<gcell, NID_LAYOUT_THREADS, 0, c->stream>>>(pair0, c->ncell, L, c->cnt, c->lay_tot, c->span_mode ? c->lut_k : nullptr,
-                                                              c->bins - 3);
+  k_layout_totals<<<gcell, NID_LAYOUT_THREADS, 0, c->stream>>>(pair0, c->ncell, L, c->cnt, c->lay_tot);
   NID_LAUNCH_CHECK(c, "k_layout_totals");
   k_layout_scan<<<n, 256, 0, c->stream>>>(p, pair0, c->lay_tot, c->lay_base, c->cell_task_start, c->cell_slice_start, c->ntasks,
                                          c->nslices, c->sl_off, c->d_flag + 1);
@@ -2348,14 +1824,11 @@ int launch_pack(nid_ctx* c, int pair0, int n) {
   return NID_OK;
 }
 
-size_t hist_sell_smem(const nid_ctx* c, int T = 256) {
-  return sizeof(double) * ((size_t)c->bins * T) + ((NID_BULK && !c->sell_points) ? bulk_smem(T, c->bins) : 0);
-}
+size_t hist_sell_smem(const nid_ctx* c, int T = 256) { return sizeof(double) * ((size_t)c->bins * T); }
 size_t jac_sell_smem(const nid_ctx* c, int T = 128) {
   const size_t B = c->bins;
   // class tables [B][T] | per warp: the staged block W | V | per warp: its mbarrier (few bins)
-  return sizeof(double) * (B * T + (NID_FEW_BINS(c->bins) ? (size_t)(T / 32) * (wv_stride(c->bins) + 1) : 0)) +
-         ((NID_BULK && !c->sell_points) ? 8 + bulk_smem(T, c->bins) : 0);
+  return sizeof(double) * (B * T + (NID_FEW_BINS(c->bins) ? (size_t)(T / 32) * (wv_stride(c->bins) + 1) : 0));
 }
 
 // Threads per CTA of the pixel kernels: the largest of 32..tmax that still gives every SM about two CTAs; a
@@ -2365,15 +1838,12 @@ static int pick_block(const nid_ctx* c, int ns, int n_jobs, int tmax) {
     if ((long long)n_jobs * ((ns + T / 32 - 1) / (T / 32)) >= 2LL * c->sm_count) return T;
   return 32;
 }
-// cells of fewer than 4096 pixels take the 128-thread assembly
+// cells of fewer than NID_ASM_SMALL_PX pixels take the warp assembly (at most 32 bins) or the 128-thread one
 #ifndef NID_ASM_SMALL_PX
 #define NID_ASM_SMALL_PX 8192
 #endif
 static bool assemble_small(const nid_ctx* c) { return (long long)c->rb * c->cb < NID_ASM_SMALL_PX; }
-#ifndef NID_ASM_WARP
-#define NID_ASM_WARP 1
-#endif
-static bool assemble_warp(const nid_ctx* c) { return NID_ASM_WARP && assemble_small(c) && c->bins <= 32; }
+static bool assemble_warp(const nid_ctx* c) { return assemble_small(c) && c->bins <= 32; }
 static size_t assemble_warp_smem(const nid_ctx* c) {
   return sizeof(double) * (size_t)NID_ASMW_WARPS * (32 / c->bins) * ((size_t)c->bins * c->bins + c->bins);
 }
@@ -2461,55 +1931,10 @@ static void launch_jac_chunks(nid_ctx* c, const EvalParams& p, int ns, int job0,
     c->launches++;
   }
 }
-size_t hist_span_smem(const nid_ctx* c, int T) { return sizeof(double) * ((size_t)4 * c->bins * T); }
-size_t jac_span_smem(const nid_ctx* c, int T) {
-  const size_t B = c->bins;
-  return sizeof(double) * (size_t)(T / 32) * (B * (B + 1) + B + 4);
-}
-template <int NG>
-static void launch_hist_span_chunks(nid_ctx* c, const EvalParams& p, int ns, int job0, int n_jobs, const int* h_list) {
-  const int T = pick_block(c, ns, n_jobs, NID_HIST_TMAX);
-  const size_t sm = hist_span_smem(c, T);
-  for (int s0 = 0; s0 < n_jobs; s0 += NG) {
-    const int n = std::min(NG, n_jobs - s0);
-    GeoTable<NG> gt;
-    fill_geo(c, gt, job0 + s0, n, true, h_list);
-    EvalParams q = p;
-    q.job0 = job0 + s0;
-    const dim3 grid = NID_GRID(n, (ns + T / 32 - 1) / (T / 32));
-    switch (T) {
-      case 128: k_hist_span<NG, 128><<<grid, 128, sm, c->stream>>>(q, gt); break;
-      case 64: k_hist_span<NG, 64><<<grid, 64, sm, c->stream>>>(q, gt); break;
-      default: k_hist_span<NG, 32><<<grid, 32, sm, c->stream>>>(q, gt); break;
-    }
-    c->launches++;
-  }
-}
-template <int NG>
-static void launch_jac_span_chunks(nid_ctx* c, const EvalParams& p, int ns, int job0, int n_jobs, const int* h_list) {
-  const int T = pick_block(c, ns, n_jobs, NID_JAC_TMAX);
-  const size_t sm = jac_span_smem(c, T);
-  for (int s0 = 0; s0 < n_jobs; s0 += NG) {
-    const int n = std::min(NG, n_jobs - s0);
-    GeoTable<NG> gt;
-    fill_geo(c, gt, job0 + s0, n, false, h_list);
-    EvalParams q = p;
-    q.job0 = job0 + s0;
-    const dim3 grid = NID_GRID(n, (ns + T / 32 - 1) / (T / 32));
-    switch (T) {
-      case 64: k_jac_span<NG, 64><<<grid, 64, sm, c->stream>>>(q, gt); break;
-      default: k_jac_span<NG, 32><<<grid, 32, sm, c->stream>>>(q, gt); break;
-    }
-    c->launches++;
-  }
-}
 #define NID_GEO_SMALL 8
 #define NID_GEO_LARGE 96
 static void launch_hist_w(nid_ctx* c, const EvalParams& p, int ns, int job0, int n_jobs, const int* h_list) {
-  if (c->span_mode) {
-    if (n_jobs <= NID_GEO_SMALL) launch_hist_span_chunks<NID_GEO_SMALL>(c, p, ns, job0, n_jobs, h_list);
-    else launch_hist_span_chunks<NID_GEO_LARGE>(c, p, ns, job0, n_jobs, h_list);
-  } else if (c->sell_points) {
+  if (c->sell_points) {
     if (n_jobs <= NID_GEO_SMALL) launch_hist_chunks<true, NID_GEO_SMALL>(c, p, ns, job0, n_jobs, h_list);
     else launch_hist_chunks<true, NID_GEO_LARGE>(c, p, ns, job0, n_jobs, h_list);
   } else {
@@ -2518,10 +1943,7 @@ static void launch_hist_w(nid_ctx* c, const EvalParams& p, int ns, int job0, int
   }
 }
 static void launch_jac_w(nid_ctx* c, const EvalParams& p, int ns, int job0, int n_jobs, const int* h_list) {
-  if (c->span_mode) {
-    if (n_jobs <= NID_GEO_SMALL) launch_jac_span_chunks<NID_GEO_SMALL>(c, p, ns, job0, n_jobs, h_list);
-    else launch_jac_span_chunks<NID_GEO_LARGE>(c, p, ns, job0, n_jobs, h_list);
-  } else if (c->sell_points) {
+  if (c->sell_points) {
     if (n_jobs <= NID_GEO_SMALL) launch_jac_chunks<true, NID_GEO_SMALL>(c, p, ns, job0, n_jobs, h_list);
     else launch_jac_chunks<true, NID_GEO_LARGE>(c, p, ns, job0, n_jobs, h_list);
   } else {
@@ -2544,10 +1966,7 @@ int launch_sorted_pass1(nid_ctx* c, const int* d_list, const int* h_list, int fi
     NID_LAUNCH_CHECK(c, "k_hist_sell");
   }
   ktime_mark(c, 1);
-  if (c->span_mode) {
-    const int units = c->ncell * n;
-    k_assemble_span<<<(units + NID_ASMW_WARPS - 1) / NID_ASMW_WARPS, NID_ASMW_WARPS * 32, assemble_warp_smem(c), c->stream>>>(p, tables, n);
-  } else if (assemble_warp(c)) {
+  if (assemble_warp(c)) {
     const int units = c->ncell * n;
     if (units <= 2 * c->sm_count * NID_ASMW_WARPS)
       k_assemble_warp<NID_ASMW_BATCH_LAT><<<(units + NID_ASMW_WARPS - 1) / NID_ASMW_WARPS, NID_ASMW_WARPS * 32, assemble_warp_smem(c), c->stream>>>(p, tables, n);
@@ -2690,7 +2109,7 @@ static int capture_latency_graph(nid_ctx* c, LatencyGraph* g, int nslots, const 
 // One round of the latency mode over the slots h_list[0 .. nslots) (every slot of the solve, each exactly once).
 int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h_list, size_t h2d_bytes, double delta, double* gn_out) {
   const int ns = c->max_nslices_prepared;
-  const bool graph_ok = c->opt_lm_graph && !c->opt_time_kernels && ns > 0 && nslots <= NID_GEO_SMALL && !c->span_mode;
+  const bool graph_ok = c->opt_lm_graph && !c->opt_time_kernels && ns > 0 && nslots <= NID_GEO_SMALL;
   if (!graph_ok) {
     cudaError_t e = cudaMemcpyAsync(c->poses, c->h_poses, h2d_bytes, cudaMemcpyHostToDevice, c->stream);
     if (e != cudaSuccess) return check_cuda(e, "H2D poses + list");
@@ -2785,7 +2204,7 @@ int launch_warp_sample_jobs(nid_ctx* c, int n_jobs, float4* d_out, bool u16) {
     fill_geo_k1(c, gt, s0, n);
     EvalParams q = p;
     q.job0 = s0;
-    const dim3 grid = NID_WS_ORDER ? dim3(chunks, n) : dim3(n, chunks);
+    const dim3 grid(n, chunks);
     if (u16) k_warp_sample_jobs<NID_GEO_LARGE, true><<<grid, 128, 0, c->stream>>>(q, gt, nullptr, c->depth16, c->depth_factor, d_out);
     else k_warp_sample_jobs<NID_GEO_LARGE, false><<<grid, 128, 0, c->stream>>>(q, gt, c->depth, nullptr, nullptr, d_out);
     NID_LAUNCH_CHECK(c, "k_warp_sample_jobs");
@@ -2799,7 +2218,6 @@ int sorted_init(nid_ctx* c) {
 #define NID_SMEM_ATTR(k, bytes)                                                                     \
   e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(bytes));            \
   if (e != cudaSuccess) return check_cuda(e, "smem attr " #k);
-#if NID_CARVEOUT
   // shared-memory carve-out of the pixel kernels: what their resident CTAs need and no more, the rest of the 256 KB
   // stays L1 for the target-image gathers. (hint only; per kernel: threads T, CTAs per SM = warps per SM * 32 / T)
 #define NID_CARVE(k, bytes, ctas)                                                                                  \
@@ -2807,9 +2225,6 @@ int sorted_init(nid_ctx* c) {
     const int pct = (int)std::min<size_t>(100, (((bytes) + 1024) * (size_t)(ctas) * 100 + 228 * 1024 - 1) / (228 * 1024)); \
     cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, pct);                                   \
   }
-#else
-#define NID_CARVE(k, bytes, ctas)
-#endif
 #define NID_SMEM_ATTR_PX(PTS, NG)                                           \
   NID_SMEM_ATTR((k_hist_sell<PTS, NG, 256>), hist_sell_smem(c, 256));       \
   NID_SMEM_ATTR((k_hist_sell<PTS, NG, 128>), hist_sell_smem(c, 128));       \
@@ -2839,18 +2254,6 @@ int sorted_init(nid_ctx* c) {
   if (c->bins <= 32) {
     NID_SMEM_ATTR(k_assemble_warp<NID_ASMW_BATCH>, assemble_warp_smem(c));
     NID_SMEM_ATTR(k_assemble_warp<NID_ASMW_BATCH_LAT>, assemble_warp_smem(c));
-    NID_SMEM_ATTR(k_assemble_span, assemble_warp_smem(c));
-  }
-  if (NID_FEW_BINS(c->bins)) {
-#define NID_SMEM_ATTR_SPAN(NG)                                              \
-  NID_SMEM_ATTR((k_hist_span<NG, 128>), hist_span_smem(c, 128));            \
-  NID_SMEM_ATTR((k_hist_span<NG, 64>), hist_span_smem(c, 64));              \
-  NID_SMEM_ATTR((k_hist_span<NG, 32>), hist_span_smem(c, 32));              \
-  NID_SMEM_ATTR((k_jac_span<NG, 64>), jac_span_smem(c, 64));                \
-  NID_SMEM_ATTR((k_jac_span<NG, 32>), jac_span_smem(c, 32));
-    NID_SMEM_ATTR_SPAN(NID_GEO_SMALL)
-    NID_SMEM_ATTR_SPAN(NID_GEO_LARGE)
-#undef NID_SMEM_ATTR_SPAN
   }
 #undef NID_SMEM_ATTR
   return NID_OK;

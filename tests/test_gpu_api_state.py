@@ -317,10 +317,12 @@ def test_latency_mode_graph_survives_changes_of_the_context(nid, orc, make_pair)
 
 
 @pytest.mark.parametrize("cell,bins,rows,cols", [(8, 10, 240, 320), (16, 10, 480, 640), (4, 16, 120, 160), (5, 20, 200, 250)])
-def test_span_tasks_and_class_tasks_agree(nid, orc, make_pair, cell, bins, rows, cols):
-    """Small cells take tasks per reference span (16 accumulations per pixel, long tasks) instead of tasks per reference
-    intensity (4 accumulations, one task per intensity): both against the oracle, and against each other, at the
-    prepare pose and away from it; pixels without a reference sample (out of bounds at prepare) included."""
+def test_small_and_odd_cells_against_the_oracle_with_pixels_out_of_bounds_at_prepare(nid, orc, make_pair, cell, bins, rows,
+                                                                                    cols):
+    """Small cells (1200 to 2000 pixels: a handful of pixels per reference intensity, short tasks) at odd cell and bin
+    counts, prepared at a pose that puts part of the frame out of bounds, so that many valid pixels have no reference
+    sample: against the oracle at the prepare pose and away from it, histograms included, and the cost-only evaluation
+    equal to the cost of the cost+Jacobian one, bit for bit."""
     p = make_pair(1004, rows, cols, invalid_depth_frac=0.05)
     pose0 = orc.reference_perturbation(p.T_wc1)
     shift = orc.se3_mul(orc.se3_exp(np.array([0, 0.05, 0, 0, 0, 0])), pose0)  # part of the frame starts out of bounds
@@ -328,38 +330,29 @@ def test_span_tasks_and_class_tasks_agree(nid, orc, make_pair, cell, bins, rows,
     P.set_quirks(0, 1)
     nco, hrefo = P.prepare(shift)
     act = ~np.isnan(hrefo)
-    res = {}
-    for mode in (2, 1):
-        ctx = nid.Context(rows, cols, cell, bins, max_jobs=2)
-        ctx.set_option("sorted_mode", mode)
-        ctx.set_option("keep_hist", 1)
-        ctx.set_pair(0, p.depth0, p.im0, p.im1, p.T_wc0, p.intr)
-        nc, href = ctx.prepare(0, orc.se3_to_mat16(shift))
-        assert np.array_equal(nc, nco)
-        out = []
-        for pose in (shift, orc.se3_mul(orc.se3_exp(np.array([0.002, -0.03, 0.0015, 0.004, -0.003, 0.002])), shift)):
-            Ht, Hj, J = ctx.eval(0, orc.se3_to_mat16(pose), True)
-            Hto, Hjo, erro, Jo = P.eval(pose, True)
-            np.testing.assert_allclose(Ht[act], Hto[act], rtol=1e-11)
-            np.testing.assert_allclose(Hj[act], Hjo[act], rtol=1e-11)
-            scale = np.abs(Jo[act]).max(axis=1, keepdims=True)
-            assert np.max(np.abs(J[act] - Jo[act]) / scale) < 1e-8
-            assert np.all(np.isnan(Ht[~act])) and np.all(np.isnan(J[~act]))
-            c0 = int(np.where(act)[0][0])
-            pt, pj = ctx.debug_hist(0, c0)
-            pto, pjo = P.last_hist(c0)
-            np.testing.assert_allclose(pj, pjo, rtol=1e-10, atol=1e-16)
-            np.testing.assert_allclose(pt, pto, rtol=1e-10, atol=1e-16)
-            out.append((Ht, Hj, J))
-        # cost-only flavour and a solve on this kind of tasks
-        Ht2, Hj2, _ = ctx.eval(0, orc.se3_to_mat16(shift), False)
-        assert np.array_equal(Ht2[act], out[0][0][act]) and np.array_equal(Hj2[act], out[0][1][act])
-        res[mode] = out
-        ctx.close()
-    for a, b in zip(res[1], res[2]):
-        np.testing.assert_allclose(a[0][act], b[0][act], rtol=1e-12)
-        np.testing.assert_allclose(a[1][act], b[1][act], rtol=1e-12)
-        np.testing.assert_allclose(a[2][act], b[2][act], rtol=1e-8, atol=1e-11)
+    ctx = nid.Context(rows, cols, cell, bins, max_jobs=2)
+    ctx.set_option("keep_hist", 1)
+    ctx.set_pair(0, p.depth0, p.im0, p.im1, p.T_wc0, p.intr)
+    nc, href = ctx.prepare(0, orc.se3_to_mat16(shift))
+    assert np.array_equal(nc, nco)
+    out = []
+    for pose in (shift, orc.se3_mul(orc.se3_exp(np.array([0.002, -0.03, 0.0015, 0.004, -0.003, 0.002])), shift)):
+        Ht, Hj, J = ctx.eval(0, orc.se3_to_mat16(pose), True)
+        Hto, Hjo, erro, Jo = P.eval(pose, True)
+        np.testing.assert_allclose(Ht[act], Hto[act], rtol=1e-11)
+        np.testing.assert_allclose(Hj[act], Hjo[act], rtol=1e-11)
+        scale = np.abs(Jo[act]).max(axis=1, keepdims=True)
+        assert np.max(np.abs(J[act] - Jo[act]) / scale) < 1e-8
+        assert np.all(np.isnan(Ht[~act])) and np.all(np.isnan(J[~act]))
+        c0 = int(np.where(act)[0][0])
+        pt, pj = ctx.debug_hist(0, c0)
+        pto, pjo = P.last_hist(c0)
+        np.testing.assert_allclose(pj, pjo, rtol=1e-10, atol=1e-16)
+        np.testing.assert_allclose(pt, pto, rtol=1e-10, atol=1e-16)
+        out.append((Ht, Hj, J))
+    Ht2, Hj2, _ = ctx.eval(0, orc.se3_to_mat16(shift), False)
+    assert np.array_equal(Ht2[act], out[0][0][act]) and np.array_equal(Hj2[act], out[0][1][act])
+    ctx.close()
 
 
 def test_every_cell_inactive(nid, orc, make_pair):

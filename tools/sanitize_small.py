@@ -5,14 +5,12 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 nid = importlib.import_module("nid-pose-estimation_b200")
 synth = importlib.import_module("nid-pose-estimation_b200.synth")
 from oracle import binding as orc
-for (rows, cols, cell, bins, mode) in ((120, 160, 2, 16, 0), (120, 160, 4, 10, 0), (96, 128, 1, 9, 0), (120, 160, 2, 40, 0),
-                                       (120, 160, 4, 10, 2), (100, 130, 3, 6, 0), (120, 160, 8, 32, 0)):
+for (rows, cols, cell, bins) in ((120, 160, 2, 16), (120, 160, 4, 10), (96, 128, 1, 9), (120, 160, 2, 40), (100, 130, 3, 6),
+                                 (120, 160, 8, 32)):
     p = synth.make_pair(1000, rows, cols, invalid_depth_frac=0.03)
     pose0 = orc.reference_perturbation(p.T_wc1)
     M0 = orc.se3_to_mat16(pose0)
     ctx = nid.Context(rows, cols, cell, bins, n_pairs=3, max_jobs=12)
-    if mode:
-        ctx.set_option("sorted_mode", mode)
     for s in range(2):
         ctx.set_pair(s, p.depth0, p.im0, p.im1, p.T_wc0, p.intr)
         ctx.prepare(s, M0)
@@ -40,4 +38,4 @@ for (rows, cols, cell, bins, mode) in ((120, 160, 2, 16, 0), (120, 160, 4, 10, 0
     ctx.prepare(1, M0)
     ctx.eval(1, M0, True)
     ctx.close()
-    print("ok", rows, cols, cell, bins, mode)
+    print("ok", rows, cols, cell, bins)
