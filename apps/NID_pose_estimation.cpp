@@ -4,6 +4,12 @@
 // replaced by the C-ABI of include/nid_b200.h: nid_set_pair (Calculate3Dpoint), nid_prepare (CudaComputeHref),
 // nid_solve (optimizer.optimize). Optional extra keys: cell (16), bin_num (10), iterations (10), use_gpu is
 // accepted and must be 1: there is no CPU path in this build.
+// pyramid_levels (1): with L > 1 the solve is coarse-to-fine, for starting poses farther from the answer than the
+// reference's perturbation. Level l (1..L-1) halves the resolution l times (nid_set_pairs_downsampled) with cell
+// max(1, cell >> l), so that a cell keeps its pixel count; nid_solve_pyramid_jobs solves levels L-1 .. 1 with `iterations`
+// each, then level 0 is prepared and solved at the pose they hand down, exactly as with L == 1. One extra line per
+// coarse level reports its outer iterations; every other printed line and the CSV row keep their formats.
+#include <algorithm>
 #include <chrono>
 #include <cstdio>
 #include <fstream>
@@ -26,6 +32,11 @@ int main(int argc, char** argv) {
   try {
     const nidio::Config cfg = nidio::read_config(argv[1]);
     const int cell = cfg.integer("cell", 16), bins = cfg.integer("bin_num", 10), iters = cfg.integer("iterations", 10);
+    const int levels = cfg.integer("pyramid_levels", 1);
+    if (levels < 1 || levels > 8) {
+      std::fprintf(stderr, "pyramid_levels must be in [1, 8]\n");
+      return 2;
+    }
     if (cfg.has("use_gpu") && cfg.integer("use_gpu") == 0) {
       std::fprintf(stderr, "use_gpu: 0 requested, but this build has no CPU evaluation path\n");
       return 2;
@@ -65,6 +76,28 @@ int main(int argc, char** argv) {
     if (nid_create(&ctx, 0, P.rows, P.cols, cell, bins, 3, 1, 1) != NID_OK) die("nid_create");
     if (nid_set_option(ctx, "task_px", 16) != NID_OK) die("nid_set_option");  // one pair, one solve: latency-bound (nid_b200.h)
     if (nid_set_pair(ctx, 0, P.depth0.data(), P.im0.data(), P.im1.data(), P.T_wc0.data(), P.intr) != NID_OK) die("nid_set_pair");
+    double pose7[7] = {est.t[0], est.t[1], est.t[2], est.q[0], est.q[1], est.q[2], est.q[3]};
+    if (levels > 1) {
+      // coarse levels 1 .. L-1, each derived on the device from the one above it
+      std::vector<nid_ctx*> lv(levels, nullptr);
+      lv[0] = ctx;
+      for (int l = 1; l < levels; l++) {
+        if (nid_create(&lv[l], 0, P.rows >> l, P.cols >> l, std::max(1, cell >> l), bins, 3, 1, 1) != NID_OK) die("nid_create (pyramid level)");
+        if (nid_set_option(lv[l], "task_px", 16) != NID_OK) die("nid_set_option");
+        if (nid_set_pairs_downsampled(lv[l], 0, lv[l - 1], 0, 1) != NID_OK) die("nid_set_pairs_downsampled");
+      }
+      std::vector<int> its(levels - 1, iters), lstats(3 * (levels - 1));
+      if (nid_solve_pyramid_jobs(lv.data() + 1, levels - 1, 1, nullptr, pose7, its.data(), std::sqrt(0.95), lstats.data()) != NID_OK)
+        die("nid_solve_pyramid_jobs");
+      for (int l = levels - 1; l >= 1; l--)
+        std::cout << "pyramid level " << l << " (" << (P.rows >> l) << "x" << (P.cols >> l) << "): outer iterations " << lstats[3 * (l - 1)]
+                  << std::endl;
+      for (int l = 1; l < levels; l++) nid_destroy(lv[l]);
+      nidhost::Pose7 pc;
+      for (int i = 0; i < 3; i++) pc.t[i] = pose7[i];
+      for (int i = 0; i < 4; i++) pc.q[i] = pose7[3 + i];
+      nidhost::pose_to_mat16(pc, M0);  // level 0 is prepared at the pose the coarse levels handed down
+    }
     std::vector<int> counter(cell * cell);
     std::vector<double> Href(cell * cell);
     if (nid_prepare(ctx, 0, M0, counter.data(), Href.data()) != NID_OK) die("nid_prepare");
@@ -72,7 +105,6 @@ int main(int argc, char** argv) {
     for (double h : Href) edges += !std::isnan(h);  // edges whose Href is NaN are put on level 1 (:323-325)
 
     std::cout << "enter optimization ............. 0" << std::endl;
-    double pose7[7] = {est.t[0], est.t[1], est.t[2], est.q[0], est.q[1], est.q[2], est.q[3]};
     std::vector<double> trace(10 * (size_t)std::max(iters, 1));
     int stats[3] = {0, 0, 0};
     const auto t_opt = std::chrono::steady_clock::now();

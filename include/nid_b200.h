@@ -79,6 +79,18 @@ int nid_set_pair(nid_ctx* ctx, int pair, const double* depth, const uint8_t* im0
  * until nid_sync or the next blocking call on this context (nid_prepare_pairs is one). */
 int nid_set_pairs_u16(nid_ctx* ctx, int pair0, int n, const uint16_t* depth_raw, const uint8_t* im0, const uint8_t* im1,
                       const double* T_wc0, const double* intr);
+/* Coarse levels for coarse-to-fine solves. Fill pair slots [dst_pair0, dst_pair0 + n) of dst with the 2x2-downsampled pairs
+ * [src_pair0, src_pair0 + n) of src, device to device. Destination pixel (i, j) covers source pixels (2i..2i+1, 2j..2j+1);
+ * an odd last source row or column is dropped. Images: (a+b+c+d+2)>>2. Depth: the mean of the valid samples (0.01 <= z
+ * <= 100; NaN and Inf are invalid), summed in row-major order of the 2x2 block, 0 (invalid) when none is valid. Intrinsics
+ * fx/2, fy/2, (cx-0.5)/2, (cy-0.5)/2 (a coarse pixel centre sits at fine coordinate 2j + 0.5); T_wc0 is copied; the
+ * destination holds fp64 depth. dst must have rows == src rows / 2 and cols == src cols / 2 (cell and bins are free) and
+ * live on the same device; levels chain (level 2 from level 1 from level 0).
+ * ASYNCHRONOUS on dst's stream, ordered after all work queued on src so far; later work on src (a refill of the source
+ * slots by nid_set_pairs_u16, say) is ordered after it. The slots must be prepared (nid_prepare*) before they are evaluated
+ * or solved. NID_ERR_ARG: geometry, ranges, devices, NULL; NID_ERR_STATE: a source pair not set, or either context
+ * holding caller-supplied world points (nid_set_pair_points). */
+int nid_set_pairs_downsampled(nid_ctx* dst, int dst_pair0, const nid_ctx* src, int src_pair0, int n);
 /* Reference-frame reuse (tracking against a key frame): replace only the target image of a pair that has been
  * set; depth, reference image and world points stay on the device. The pair must be prepared again
  * (nid_prepare at the new initial pose: the in-bounds set, n_c and H_ref depend on it, CudaComputeHref.cu:33-135). */
@@ -141,6 +153,18 @@ int nid_solve(nid_ctx* ctx, int pair, double pose7[7], int max_iters, double hub
 /* n independent solves in lockstep, pair job_pair[j] (NULL: pair j), poses7 [n][7] in/out, stats [n][3]. */
 int nid_solve_jobs(nid_ctx* ctx, int n, const int* job_pair, double* poses7, int max_iters,
                    double huber_delta, int* stats);
+/* Coarse-to-fine optimize(): levels[0] is the finest context, levels[n_levels-1] the coarsest (1 <= n_levels <= 8; build the
+ * coarse levels with nid_set_pairs_downsampled). For l = n_levels-1 .. 0: prepare pairs job_pair[j] of levels[l] at the
+ * current poses (nid_prepare_pairs), then nid_solve_jobs(levels[l], ..., max_iters[l], ...) and hand the poses down. Job pairs
+ * must be distinct (a pair is prepared at one pose); NULL means pair j. A level with max_iters[l] == 0 is skipped (its stats
+ * are 0). n_levels == 1 is exactly nid_prepare_pairs + nid_solve_jobs. stats (may be NULL): [n][n_levels][3] as in nid_solve.
+ * poses7 and stats are written only on success. Validated before any work: every level non-NULL, n <= max_jobs and every
+ * job's pair set at every level (NID_ERR_STATE if not), pairs distinct.
+ * A job without an active cell at a level (every cell under NID_MIN_CELL_POINTS in-bounds points at the prepare pose, as on
+ * a level too coarse for its cell grid) has chi2 == 0 and a zero Gauss-Newton system there: the LM schedule rejects its
+ * first trial (no decrease) and stops, so that level reports {1, 1, 1} and hands the pose down unchanged. */
+int nid_solve_pyramid_jobs(nid_ctx* const* levels, int n_levels, int n, const int* job_pair, double* poses7,
+                           const int* max_iters, double huber_delta, int* stats);
 
 /* a12: hard-binned NID of NID_standard_property (no B-spline, normaliser = in-bounds count of this
  * pose). total[n_jobs] = sqrt(sum_c nid_c^2); nid_cells [n_jobs][cell^2] may be NULL. */

@@ -68,6 +68,8 @@ def lib():
         L.nid_eval_gn.argtypes = [C.c_void_p, C.c_int, _dp, C.c_double, _dp, _dp, _dp, _dp, _dp]
         L.nid_solve.argtypes = [C.c_void_p, C.c_int, _dp, C.c_int, C.c_double, _dp, _ip]
         L.nid_solve_jobs.argtypes = [C.c_void_p, C.c_int, _ip, _dp, C.c_int, C.c_double, _ip]
+        L.nid_set_pairs_downsampled.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int]
+        L.nid_solve_pyramid_jobs.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_int, _ip, _dp, _ip, C.c_double, _ip]
         L.nid_hard_eval_jobs.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp]
         L.nid_warp_sample.argtypes = [C.c_void_p, C.c_int, _dp, _fp]
         L.nid_warp_sample_f64.argtypes = [C.c_void_p, C.c_int, _dp, _dp]
@@ -160,6 +162,11 @@ class Context:
         href = np.zeros((n, self.ncell))
         _chk(lib().nid_prepare_pairs(self._h, pair0, n, _d(T), nc.ctypes.data_as(_ip), _d(href)))
         return nc, href
+
+    def set_pairs_downsampled(self, pair0, src, src_pair0, n=1):
+        """Fill pairs [pair0, pair0 + n) with the 2x2-downsampled pairs [src_pair0, src_pair0 + n) of Context `src`
+        (device to device, asynchronous; prepare before use)."""
+        _chk(lib().nid_set_pairs_downsampled(self._h, pair0, src._h if src is not None else None, src_pair0, n))
 
     def set_target(self, pair, im1):
         """Replace only the target image of a pair (reference-frame reuse); prepare() must be called again."""
@@ -312,6 +319,21 @@ class Context:
 
     def set_option(self, key: str, value: int):
         _chk(lib().nid_set_option(self._h, key.encode(), int(value)))
+
+
+def solve_pyramid_jobs(levels, poses7, job_pair=None, max_iters=None, delta=np.sqrt(0.95)):
+    """Coarse-to-fine solve over Contexts `levels` (finest first): nid_solve_pyramid_jobs. max_iters: one count per level
+    (default 10 each). Returns (poses [n, 7], stats [n, n_levels, 3])."""
+    L = len(levels)
+    poses = _f64(poses7).copy().reshape(-1, 7)
+    n = poses.shape[0]
+    hs = (C.c_void_p * L)(*[None if c is None else c._h.value for c in levels])
+    its = np.ascontiguousarray([10] * L if max_iters is None else max_iters, dtype=np.int32)
+    jp = None if job_pair is None else np.ascontiguousarray(job_pair, dtype=np.int32)
+    stats = np.zeros((n, L, 3), dtype=np.int32)
+    _chk(lib().nid_solve_pyramid_jobs(hs, L, n, None if jp is None else jp.ctypes.data_as(_ip), _d(poses),
+                                      its.ctypes.data_as(_ip), float(delta), stats.ctypes.data_as(_ip)))
+    return poses, stats
 
 
 def exported_symbols_in_header():

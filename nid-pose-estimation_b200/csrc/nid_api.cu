@@ -390,6 +390,7 @@ int nid_destroy(nid_ctx* c) {
   if (c->h_arena) cudaFreeHost(c->h_arena);
   if (c->h_res) cudaFreeHost(c->h_res);
   for (int i = 0; i < 2; i++) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
+  for (int i = 0; i < 2; i++) if (c->ds_ev[i]) cudaEventDestroy(c->ds_ev[i]);
   for (int i = 0; i < 5; i++) if (c->kev[i]) cudaEventDestroy(c->kev[i]);
   cudaStreamDestroy(c->stream);
   if (c->stream2) cudaStreamDestroy(c->stream2);
@@ -465,6 +466,62 @@ int nid_set_pairs_u16(nid_ctx* c, int pair0, int n, const uint16_t* depth_raw, c
   CU(cudaMemcpyAsync(c->im1 + (size_t)pair0 * N, im1, N * n, cudaMemcpyDefault, c->stream), "H2D im1");
   OKR(update_textures(c, pair0, n));
   for (int i = 0; i < n; i++) c->pair_set[pair0 + i] = 1;
+  return NID_OK;  // (asynchronous: see the header)
+}
+
+// A coarser level of pairs that already live on the device: k_downsample2 writes depth and images, the intrinsics are
+// derived on the host from the source's mirror, T_wc0 is copied device to device; then the ordinary world points and
+// target textures. dst's stream waits for the source's queued work, and the source's stream waits for the kernel, so a
+// refill of the source slot issued right after this call cannot overwrite what is being read.
+int nid_set_pairs_downsampled(nid_ctx* dst, int dst_pair0, const nid_ctx* src, int src_pair0, int n) {
+  if (!dst || !src) { set_error("NULL context"); return NID_ERR_ARG; }
+  if (dst->rows != src->rows / 2 || dst->cols != src->cols / 2) {
+    set_error("destination geometry must be (source rows / 2, source cols / 2)");
+    return NID_ERR_ARG;
+  }
+  if (n < 1 || n > dst->n_pairs || n > src->n_pairs || dst_pair0 < 0 || src_pair0 < 0 || dst_pair0 > dst->n_pairs - n ||
+      src_pair0 > src->n_pairs - n) {
+    set_error("pair range out of bounds");
+    return NID_ERR_ARG;
+  }
+  if (dst->device != src->device) { set_error("source and destination contexts live on different devices"); return NID_ERR_ARG; }
+  if (src->sell_points || dst->sell_points) {
+    set_error("downsampling needs depth pairs on both sides, not caller-supplied world points (nid_set_pair_points)");
+    return NID_ERR_STATE;
+  }
+  for (int i = 0; i < n; i++)
+    if (!src->pair_set[src_pair0 + i]) { set_error("source pair not set"); return NID_ERR_STATE; }
+  CU(cudaSetDevice(dst->device), "cudaSetDevice");
+  for (int i = 0; i < 2; i++)
+    if (!dst->ds_ev[i]) CU(cudaEventCreateWithFlags(&dst->ds_ev[i], cudaEventDisableTiming), "cudaEventCreate (downsample)");
+  double* a = nullptr;
+  OKR(arena_take(dst, sizeof(double) * 5 * n, (void**)&a));
+  double *acam = a, *afac = a + 4 * (size_t)n;
+  for (int i = 0; i < n; i++) {
+    // a coarse pixel centre j sits at fine coordinate 2j + 0.5 (the reference samples pixel j at u = j)
+    const double* k = src->h_cam.data() + 4 * (size_t)(src_pair0 + i);
+    acam[4 * i] = k[0] * 0.5; acam[4 * i + 1] = k[1] * 0.5;
+    acam[4 * i + 2] = (k[2] - 0.5) * 0.5; acam[4 * i + 3] = (k[3] - 0.5) * 0.5;
+    afac[i] = 1.0;  // (unused: the destination holds fp64 depth)
+  }
+  CU(cudaEventRecord(dst->ds_ev[0], src->stream), "record source event");
+  CU(cudaStreamWaitEvent(dst->stream, dst->ds_ev[0], 0), "wait for the source");
+  CU(cudaMemcpyAsync(dst->cam + 4 * (size_t)dst_pair0, acam, sizeof(double) * 4 * n, cudaMemcpyHostToDevice, dst->stream), "H2D intr");
+  CU(cudaMemcpyAsync(dst->depth_factor + dst_pair0, afac, sizeof(double) * n, cudaMemcpyHostToDevice, dst->stream), "H2D depth factor");
+  CU(cudaMemcpyAsync(dst->Twc0 + 16 * (size_t)dst_pair0, src->Twc0 + 16 * (size_t)src_pair0, sizeof(double) * 16 * n,
+                     cudaMemcpyDeviceToDevice, dst->stream), "D2D Twc0");
+  memcpy(dst->h_cam.data() + 4 * (size_t)dst_pair0, acam, sizeof(double) * 4 * n);
+  memcpy(dst->h_Twc0.data() + 16 * (size_t)dst_pair0, src->h_Twc0.data() + 16 * (size_t)src_pair0, sizeof(double) * 16 * n);
+  OKR(launch_downsample2(dst, dst_pair0, src, src_pair0, n));
+  OKR(launch_points(dst, dst_pair0, n, false));
+  OKR(update_textures(dst, dst_pair0, n));
+  CU(cudaEventRecord(dst->ds_ev[1], dst->stream), "record destination event");
+  CU(cudaStreamWaitEvent(src->stream, dst->ds_ev[1], 0), "order the source after the kernel");
+  for (int i = 0; i < n; i++) {
+    dst->pair_set[dst_pair0 + i] = 1;
+    dst->pair_prepared[dst_pair0 + i] = 0;
+    dst->pair_u16[dst_pair0 + i] = 0;
+  }
   return NID_OK;  // (asynchronous: see the header)
 }
 
@@ -1095,6 +1152,55 @@ int nid_solve(nid_ctx* c, int pair, double pose7[7], int max_iters, double delta
   int r = nid_solve_jobs(c, 1, &pair, pose7, max_iters, delta, stats);
   c->lm_trace = nullptr;
   return r;
+}
+
+// Coarse-to-fine: every level is prepared at the poses the coarser level handed down (the in-bounds set and n_c depend on
+// the prepare pose), then solved. The pairs of a run of consecutive job pairs are prepared in one nid_prepare_pairs call.
+int nid_solve_pyramid_jobs(nid_ctx* const* levels, int n_levels, int n, const int* job_pair, double* poses7, const int* max_iters,
+                           double delta, int* stats) {
+  if (!levels || n_levels < 1 || n_levels > 8 || n < 1 || !poses7 || !max_iters) { set_error("bad argument"); return NID_ERR_ARG; }
+  std::vector<int> jp(n);
+  for (int j = 0; j < n; j++) jp[j] = job_pair ? job_pair[j] : j;
+  for (int l = 0; l < n_levels; l++) {
+    const nid_ctx* c = levels[l];
+    if (!c) { set_error("NULL level context"); return NID_ERR_ARG; }
+    if (max_iters[l] < 0) { set_error("max_iters must be >= 0"); return NID_ERR_ARG; }
+    if (n > c->max_jobs) { set_error("more jobs than a level's max_jobs"); return NID_ERR_ARG; }
+    for (int j = 0; j < n; j++) {
+      if (jp[j] < 0 || jp[j] >= c->n_pairs) { set_error("job_pair out of range"); return NID_ERR_ARG; }
+      if (!c->pair_set[jp[j]]) { set_error("job pair not set at every level"); return NID_ERR_STATE; }
+    }
+  }
+  {
+    std::vector<int> s = jp;
+    std::sort(s.begin(), s.end());
+    if (std::adjacent_find(s.begin(), s.end()) != s.end()) {
+      set_error("job pairs must be distinct (a pair is prepared at one pose)");
+      return NID_ERR_ARG;
+    }
+  }
+  std::vector<double> cur(poses7, poses7 + 7 * (size_t)n), T(16 * (size_t)n);
+  std::vector<int> st(3 * (size_t)n), all(3 * (size_t)n * n_levels, 0);
+  for (int l = n_levels - 1; l >= 0; l--) {
+    if (max_iters[l] == 0) continue;
+    nid_ctx* c = levels[l];
+    for (int j = 0; j < n; j++) {
+      nidhost::Pose7 p;
+      memcpy(p.t, &cur[7 * (size_t)j], sizeof(double) * 3);
+      memcpy(p.q, &cur[7 * (size_t)j + 3], sizeof(double) * 4);
+      nidhost::pose_to_mat16(p, &T[16 * (size_t)j]);
+    }
+    for (int j0 = 0, j1; j0 < n; j0 = j1) {
+      for (j1 = j0 + 1; j1 < n && jp[j1] == jp[j1 - 1] + 1; j1++) {}
+      OKR(nid_prepare_pairs(c, jp[j0], j1 - j0, &T[16 * (size_t)j0], nullptr, nullptr));
+    }
+    OKR(nid_solve_jobs(c, n, jp.data(), cur.data(), max_iters[l], delta, st.data()));
+    for (int j = 0; j < n; j++)
+      for (int k = 0; k < 3; k++) all[((size_t)j * n_levels + l) * 3 + k] = st[3 * (size_t)j + k];
+  }
+  memcpy(poses7, cur.data(), sizeof(double) * 7 * (size_t)n);
+  if (stats) memcpy(stats, all.data(), sizeof(int) * all.size());
+  return NID_OK;
 }
 
 int nid_hard_eval_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const double* poses, double* total, double* nid_cells) {

@@ -207,6 +207,9 @@ struct nid_ctx {
   double* lm_trace = nullptr;  // set by nid_solve for the duration of one call
   int lm_trace_cap = 0;
   cudaEvent_t ev[2] = {nullptr, nullptr};
+  // nid_set_pairs_downsampled into this context: [0] recorded on the source's stream before the kernel, [1] on this
+  // context's stream after it (created on first use)
+  cudaEvent_t ds_ev[2] = {nullptr, nullptr};
   int opt_time_kernels = 0;
   cudaEvent_t kev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
   double kernel_ms[4] = {0, 0, 0, 0};  // k_hist, k_jac, k_jac_final, k_entropy
@@ -338,6 +341,7 @@ int launch_href(nid_ctx* c, int pair0, int n);
 // kernel launchers (nid_kernels.cu)
 int launch_build_lut(nid_ctx* c);
 int launch_points(nid_ctx* c, int pair0, int n, bool u16);
+int launch_downsample2(nid_ctx* dst, int dst_pair0, const nid_ctx* src, int src_pair0, int n);
 int launch_prepare(nid_ctx* c, int pair0, int n, const double* d_poses16);
 int launch_ref_weights(nid_ctx* c, int pair);
 int launch_points_aos(nid_ctx* c, int pair, double* d_out);

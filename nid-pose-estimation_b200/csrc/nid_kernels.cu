@@ -65,6 +65,34 @@ __global__ void k_points(int rows, int cols, int pair0, double* __restrict__ dep
   }
 }
 
+// 2x2 downsampling of a pair (nid_set_pairs_downsampled): destination pixel (i, j) of pair blockIdx.y covers source
+// pixels (2i..2i+1, 2j..2j+1); an odd last source row or column is dropped. Images: (a + b + c + d + 2) >> 2, exact in
+// integers. Depth: the mean of the valid samples (the test of k_points, with NaN and Inf invalid too), summed in the fixed
+// order (2i,2j), (2i,2j+1), (2i+1,2j), (2i+1,2j+1) without contraction; 0 (invalid) when no sample is valid.
+// The pointers are those of the first source / destination pair of the batch.
+__global__ void k_downsample2(int src_cols, int rows, int cols, const double* __restrict__ src_depth,
+                              const uint8_t* __restrict__ src_im0, const uint8_t* __restrict__ src_im1, size_t src_N,
+                              double* __restrict__ dst_depth, uint8_t* __restrict__ dst_im0, uint8_t* __restrict__ dst_im1,
+                              size_t dst_N) {
+  const int N = rows * cols;
+  const size_t sb = (size_t)blockIdx.y * src_N, db = (size_t)blockIdx.y * dst_N;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) {
+    const int r = i / cols, c = i % cols;
+    const size_t s[4] = {sb + (size_t)(2 * r) * src_cols + 2 * c, sb + (size_t)(2 * r) * src_cols + 2 * c + 1,
+                         sb + (size_t)(2 * r + 1) * src_cols + 2 * c, sb + (size_t)(2 * r + 1) * src_cols + 2 * c + 1};
+    dst_im0[db + i] = (uint8_t)(((unsigned)src_im0[s[0]] + src_im0[s[1]] + src_im0[s[2]] + src_im0[s[3]] + 2) >> 2);
+    dst_im1[db + i] = (uint8_t)(((unsigned)src_im1[s[0]] + src_im1[s[1]] + src_im1[s[2]] + src_im1[s[3]] + 2) >> 2);
+    double sum = 0.0;
+    int n = 0;
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+      const double z = src_depth[s[k]];
+      if (z >= 0.01 && z <= 100) { sum = __dadd_rn(sum, z); n++; }
+    }
+    dst_depth[db + i] = n ? __ddiv_rn(sum, (double)n) : 0.0;
+  }
+}
+
 __global__ void k_points_aos(int N, const double* __restrict__ pwx, const double* __restrict__ pwy,
                              const double* __restrict__ pwz, double* __restrict__ out) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) {
@@ -598,6 +626,15 @@ int launch_points(nid_ctx* c, int pair0, int n, bool u16) {
   if (u16) k_points<true><<<grid, 256, 0, c->stream>>>(c->rows, c->cols, pair0, c->depth, c->depth16, c->depth_factor, c->Twc0, c->cam, c->pwx, c->pwy, c->pwz);
   else k_points<false><<<grid, 256, 0, c->stream>>>(c->rows, c->cols, pair0, c->depth, nullptr, nullptr, c->Twc0, c->cam, c->pwx, c->pwy, c->pwz);
   NID_LAUNCH_CHECK(c, "k_points");
+  return NID_OK;
+}
+
+int launch_downsample2(nid_ctx* dst, int dst_pair0, const nid_ctx* src, int src_pair0, int n) {
+  const dim3 grid(grid_for(dst->N, 256, std::max(8, dst->sm_count * 8 / n)), n);
+  const size_t sb = (size_t)src_pair0 * src->N, db = (size_t)dst_pair0 * dst->N;
+  k_downsample2<<<grid, 256, 0, dst->stream>>>(src->cols, dst->rows, dst->cols, src->depth + sb, src->im0 + sb, src->im1 + sb,
+                                               (size_t)src->N, dst->depth + db, dst->im0 + db, dst->im1 + db, (size_t)dst->N);
+  NID_LAUNCH_CHECK(dst, "k_downsample2");
   return NID_OK;
 }
 
