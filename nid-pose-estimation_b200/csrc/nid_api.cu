@@ -44,7 +44,9 @@ static int strips_for(const nid_ctx* c, int n_jobs) {
     S = (int)((want + per - 1) / per);
     S = std::max(1, std::min(S, std::min(c->rb, 32)));
   }
-  // the natural-order kernels write n_jobs * S (job, strip) partials: never more than the buffers hold
+  // the natural-order kernels write n_jobs * S (job, strip) partials: never more than the buffers hold. They index them
+  // by (slot * ncell + cell) * S + strip, so pass 1 and pass 2 of the same slots must use the same S: n_jobs is the
+  // number of slots a job set addresses (JobSet::slots), not the length of its list.
   if (c->part_slots > 0 && n_jobs > 0) S = (int)std::max<size_t>(1, std::min<size_t>((size_t)S, c->part_slots / (size_t)n_jobs));
   return S;
 }
@@ -741,11 +743,27 @@ int nid_stage_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const double* po
   return stage_jobs(c, n_jobs, job_pair, poses);
 }
 
+// cost (+ Jacobian) of the staged jobs 0 .. n - 1
+static int eval_range(nid_ctx* c, int n, int want_jac) {
+  OKR(ensure_job_buffers(c));
+  const JobSet js{nullptr, nullptr, 0, n, n};
+  OKR(launch_pass1(c, js, want_jac ? Pass2::all : Pass2::none));
+  if (!want_jac) {
+    const int slot[2] = {0, 3};
+    ktime_collect(c, 2, slot);
+    return NID_OK;
+  }
+  OKR(launch_pass2(c, js));
+  const int sorted_slot[4] = {0, 3, 1, 2}, natural_slot[4] = {0, -1, 1, 2};  // (natural: no cost tail between marks 1 and 2)
+  ktime_collect(c, 4, use_sorted(c) ? sorted_slot : natural_slot);
+  return NID_OK;
+}
+
 int nid_eval_staged(nid_ctx* c, int n_jobs, int want_jac) {
   if (!c || n_jobs < 1 || n_jobs > c->max_jobs) { set_error("bad argument"); return NID_ERR_ARG; }
   if (n_jobs > c->staged_jobs) { set_error("nid_eval_staged: more jobs than the last nid_stage_jobs staged"); return NID_ERR_STATE; }
   CU(cudaSetDevice(c->device), "cudaSetDevice");
-  return launch_eval(c, n_jobs, want_jac);
+  return eval_range(c, n_jobs, want_jac);
 }
 
 int nid_fetch_results(nid_ctx* c, int n_jobs, int want_jac, double* Ht, double* Hj, double* der) {
@@ -759,7 +777,7 @@ int nid_eval_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const double* pos
   if (!c || !poses) { set_error("bad argument"); return NID_ERR_ARG; }
   CU(cudaSetDevice(c->device), "cudaSetDevice");
   OKR(stage_jobs(c, n_jobs, job_pair, poses));
-  OKR(launch_eval(c, n_jobs, want_jac));
+  OKR(eval_range(c, n_jobs, want_jac));
   return fetch(c, n_jobs, want_jac, Ht, Hj, der);
 }
 
@@ -772,8 +790,8 @@ int nid_eval_gn(nid_ctx* c, int pair, const double T_cw1[16], double delta, doub
   if (!c || !T_cw1) { set_error("bad argument"); return NID_ERR_ARG; }
   CU(cudaSetDevice(c->device), "cudaSetDevice");
   OKR(stage_jobs(c, 1, &pair, T_cw1));
-  OKR(launch_eval(c, 1, 1));
-  OKR(launch_gn(c, 1, delta));
+  OKR(eval_range(c, 1, 1));
+  OKR(launch_gn(c, JobSet{nullptr, nullptr, 0, 1, 1}, delta, 1));
   double* h = c->h_out;
   const size_t nc = c->ncell;
   CU(cudaMemcpyAsync(h, c->gn, sizeof(double) * 44, cudaMemcpyDeviceToHost, c->stream), "D2H gn");
@@ -999,38 +1017,13 @@ static int solve_speculative(nid_ctx* c, std::vector<LM>& st, int n, int max_ite
 // then :98), and the sorted kernels are deterministic, so the histograms, err and tables in the slot are bit for bit
 // what a recomputation would produce. The reference evaluates them again (CudaComputeH(true) repeats the cost half);
 // skipping that repeats nothing observable and saves a third of the device work of a solve (option "lm_reuse").
-int nid_solve_jobs(nid_ctx* c, int n, const int* job_pair, double* poses7, int max_iters, double delta, int* stats) {
-  if (!c || n < 1 || n > c->max_jobs || !poses7) { set_error("bad argument"); return NID_ERR_ARG; }
-  CU(cudaSetDevice(c->device), "cudaSetDevice");
-  std::vector<LM> st(n);
-  for (int j = 0; j < n; j++) {
-    LM& s = st[j];
-    s.pair = job_pair ? job_pair[j] : j;
-    if (s.pair < 0 || s.pair >= c->n_pairs) { set_error("job_pair out of range"); return NID_ERR_ARG; }
-    if (!c->pair_prepared[s.pair] || (use_sorted(c) && !c->pair_sorted[s.pair])) { set_error("pair not prepared"); return NID_ERR_STATE; }
-    memcpy(s.est.t, poses7 + 7 * j, sizeof(double) * 3);
-    memcpy(s.est.q, poses7 + 7 * j + 3, sizeof(double) * 4);
-    s.phase = max_iters > 0 ? 0 : 2;
-  }
-  OKR(ensure_job_buffers(c));
-  c->staged_jobs = 0;  // the solver rewrites the staged poses and job table
+// The natural-order kernels sum with shared-memory atomics, so their histograms are not bit-reproducible: there every
+// active job is on list 1.
+static int solve_lockstep(nid_ctx* c, std::vector<LM>& st, int n, int max_iters, double delta) {
   const bool sorted = use_sorted(c);
   const bool reuse = sorted && c->opt_lm_reuse;
-  if (sorted && n <= 4 && c->opt_lm_spec >= 2) {
-    const int K = std::min(c->opt_lm_spec, c->job_cap / n);
-    if (K >= 2) {
-      for (int j = 0; j < n; j++) c->h_job_pair[j] = st[j].pair;
-      int r = solve_speculative(c, st, n, max_iters, delta, K);
-      if (r != NID_OK) return r;
-      for (int j = 0; j < n; j++) {
-        memcpy(poses7 + 7 * j, st[j].est.t, sizeof(double) * 3);
-        memcpy(poses7 + 7 * j + 3, st[j].est.q, sizeof(double) * 4);
-        if (stats) { stats[3 * j] = st[j].it; stats[3 * j + 1] = st[j].jac_evals; stats[3 * j + 2] = st[j].cost_evals; }
-      }
-      return NID_OK;
-    }
-  }
-  // (the natural-order kernels size their per-job partial buffers by the job count of a launch: one range there)
+  // (the natural-order kernels index their partial buffers by (slot, cell, strip): two halves in flight would need the
+  // same strip count S)
   const int nh = (n >= 8 && sorted) ? 2 : 1;
   if (nh == 2 && !c->stream2) {
     CU(cudaStreamCreateWithFlags(&c->stream2, cudaStreamNonBlocking), "cudaStreamCreate (LM)");
@@ -1075,68 +1068,57 @@ int nid_solve_jobs(nid_ctx* c, int n, const int* job_pair, double* poses7, int m
     int* d2 = d1 + cnt;
     CU(cudaMemcpyAsync(d1, l1, sizeof(int) * 2 * cnt, cudaMemcpyHostToDevice, h.stream), "H2D job lists");
     c->stream = h.stream;  // the launchers issue on the context's current stream
+    const JobSet js1{d1, l1, 0, h.n1, n}, js2{d2, l2, 0, h.n2, n};  // (slots: the solve's, the same in every round)
     int r = NID_OK;
-    if (sorted) {
-      if (h.n1 > 0) r = launch_sorted_pass1(c, d1, l1, 0, h.n1, 1);
-      if (r == NID_OK && h.n2 > 0) r = launch_sorted_pass2(c, d2, l2, 0, h.n2);
-      if (r == NID_OK && h.n2 > 0) r = launch_gn_list(c, d2, 0, h.n2, delta, 1);
-      if (r == NID_OK && h.n1 > 0) r = launch_gn_list(c, d1, 0, h.n1, delta, 0);  // chi2 of the trial poses (and, harmlessly, again of full jobs)
-    } else {
-      // natural-order kernels: contiguous ranges, everything recomputed -- jobs are compacted into the slots [lo, lo + na)
-      r = NID_ERR_STATE;
-    }
+    if (h.n1 > 0) r = launch_pass1(c, js1, Pass2::some);
+    if (r == NID_OK && h.n2 > 0) r = launch_pass2(c, js2);
+    if (r == NID_OK && h.n2 > 0) r = launch_gn(c, js2, delta, 1);
+    if (r == NID_OK && h.n1 > 0) r = launch_gn(c, js1, delta, 0);  // chi2 of the trial poses (and, harmlessly, again of full jobs)
     c->stream = main_stream;
     if (r != NID_OK) return r;
     CU(cudaMemcpyAsync(c->h_out + 44 * (size_t)h.lo, c->gn + 44 * (size_t)h.lo, sizeof(double) * 44 * cnt, cudaMemcpyDeviceToHost, h.stream),
        "D2H gn");
     return NID_OK;
   };
-  // natural-order path: the round-1 scheme (compacted contiguous ranges, full evaluations)
-  std::vector<int> order;
-  auto issue_natural = [&](Half& h) -> int {
-    order.clear();
-    int nj = 0;
-    for (int j = h.lo; j < h.hi; j++) if (st[j].phase == 0) { order.push_back(j); nj++; }
-    for (int j = h.lo; j < h.hi; j++) if (st[j].phase == 1) order.push_back(j);
-    h.na = (int)order.size();
-    if (h.na == 0) return NID_OK;
-    for (int k = 0; k < h.na; k++) {
-      nidhost::pose_to_mat16(st[order[k]].est, c->h_poses + 16 * (size_t)k);
-      c->h_job_pair[k] = st[order[k]].pair;
-    }
-    CU(cudaMemcpyAsync(c->poses, c->h_poses, sizeof(double) * 16 * h.na, cudaMemcpyHostToDevice, h.stream), "H2D poses");
-    CU(cudaMemcpyAsync(c->job_pair, c->h_job_pair, sizeof(int) * h.na, cudaMemcpyHostToDevice, h.stream), "H2D job_pair");
-    const int r = launch_eval_mixed(c, 0, nj, h.na - nj, delta);
-    if (r != NID_OK) return r;
-    CU(cudaMemcpyAsync(c->h_out, c->gn, sizeof(double) * 44 * h.na, cudaMemcpyDeviceToHost, h.stream), "D2H gn");
-    return NID_OK;
-  };
-  if (!sorted) {
-    Half& h = H[0];
-    rc = issue_natural(h);
-    while (rc == NID_OK && h.na > 0) {
+  for (int i = 0; i < nh && rc == NID_OK; i++) rc = issue(H[i]);
+  while (rc == NID_OK && (H[0].na > 0 || (nh == 2 && H[1].na > 0))) {
+    for (int i = 0; i < nh && rc == NID_OK; i++) {
+      Half& h = H[i];
+      if (h.na == 0) continue;
       if (cudaStreamSynchronize(h.stream) != cudaSuccess) { rc = check_cuda(cudaGetLastError(), "sync lm"); break; }
-      const std::vector<int> done = order;
-      for (int k = 0; k < (int)done.size(); k++) lm_absorb(c, st[done[k]], c->h_out + 44 * (size_t)k, n, max_iters);
-      rc = issue_natural(h);
-    }
-  } else {
-    for (int i = 0; i < nh && rc == NID_OK; i++) rc = issue(H[i]);
-    while (rc == NID_OK && (H[0].na > 0 || (nh == 2 && H[1].na > 0))) {
-      for (int i = 0; i < nh && rc == NID_OK; i++) {
-        Half& h = H[i];
-        if (h.na == 0) continue;
-        if (cudaStreamSynchronize(h.stream) != cudaSuccess) { rc = check_cuda(cudaGetLastError(), "sync lm"); break; }
-        for (int j = h.lo; j < h.hi; j++)
-          if (st[j].phase != 2) lm_absorb(c, st[j], c->h_out + 44 * (size_t)j, n, max_iters);
-        rc = issue(h);
-      }
+      for (int j = h.lo; j < h.hi; j++)
+        if (st[j].phase != 2) lm_absorb(c, st[j], c->h_out + 44 * (size_t)j, n, max_iters);
+      rc = issue(h);
     }
   }
   c->stream = main_stream;
   if (nh == 2) cudaStreamSynchronize(c->stream2);
   cudaStreamSynchronize(main_stream);
-  if (rc != NID_OK) return rc;
+  return rc;
+}
+
+int nid_solve_jobs(nid_ctx* c, int n, const int* job_pair, double* poses7, int max_iters, double delta, int* stats) {
+  if (!c || n < 1 || n > c->max_jobs || !poses7) { set_error("bad argument"); return NID_ERR_ARG; }
+  CU(cudaSetDevice(c->device), "cudaSetDevice");
+  std::vector<LM> st(n);
+  for (int j = 0; j < n; j++) {
+    LM& s = st[j];
+    s.pair = job_pair ? job_pair[j] : j;
+    if (s.pair < 0 || s.pair >= c->n_pairs) { set_error("job_pair out of range"); return NID_ERR_ARG; }
+    if (!c->pair_prepared[s.pair] || (use_sorted(c) && !c->pair_sorted[s.pair])) { set_error("pair not prepared"); return NID_ERR_STATE; }
+    memcpy(s.est.t, poses7 + 7 * j, sizeof(double) * 3);
+    memcpy(s.est.q, poses7 + 7 * j + 3, sizeof(double) * 4);
+    s.phase = max_iters > 0 ? 0 : 2;
+  }
+  OKR(ensure_job_buffers(c));
+  c->staged_jobs = 0;  // the solver rewrites the staged poses and job table
+  const int K = std::min(c->opt_lm_spec, c->job_cap / n);
+  if (use_sorted(c) && n <= 4 && K >= 2) {
+    for (int j = 0; j < n; j++) c->h_job_pair[j] = st[j].pair;
+    OKR(solve_speculative(c, st, n, max_iters, delta, K));
+  } else {
+    OKR(solve_lockstep(c, st, n, max_iters, delta));
+  }
   for (int j = 0; j < n; j++) {
     memcpy(poses7 + 7 * j, st[j].est.t, sizeof(double) * 3);
     memcpy(poses7 + 7 * j + 3, st[j].est.q, sizeof(double) * 4);

@@ -309,10 +309,12 @@ inline void ktime_mark(nid_ctx* c, int i) {
   if (!c->kev[i]) cudaEventCreate(&c->kev[i]);
   cudaEventRecord(c->kev[i], c->stream);
 }
+// adds the interval between marks i and i + 1 to the bucket slot[i] (-1: no kernel ran in it)
 inline void ktime_collect(nid_ctx* c, int n, const int* slot) {
   if (!c->opt_time_kernels) return;
   cudaEventSynchronize(c->kev[n]);
   for (int i = 0; i < n; i++) {
+    if (slot[i] < 0) continue;
     float ms = 0.f;
     cudaEventElapsedTime(&ms, c->kev[i], c->kev[i + 1]);
     c->kernel_ms[slot[i]] += ms;
@@ -322,17 +324,27 @@ inline void ktime_collect(nid_ctx* c, int n, const int* slot) {
 bool use_sorted(const nid_ctx* c);
 int ensure_job_buffers(nid_ctx* c);
 
+// The evaluation, on either kernel family (use_sorted picks it), of a set of job slots: d_list[first .. first + n)
+// (h_list: the host copy of d_list), or the slots first .. first + n - 1 when d_list is null. `slots` is the number of
+// slots the set addresses (first + n for a range, the solve's slot count in the LM); pass 1 and pass 2 of the same jobs
+// must be given the same value (see strips_for).
+struct JobSet { const int* d_list; const int* h_list; int first, n; int slots; };
+// Will pass 2 run on none, some or all of the jobs of a pass 1? Sorted: unless none, the assembly also writes the scaled
+// log tables pass 2 reads. Natural: with all, k_jac writes the cost and pass 1 skips k_entropy.
+enum class Pass2 { none, some, all };
+// nid_sorted.cu: pass 1 writes the histograms and the cost (ht, hj, err) between timer marks 0, 1, 2; pass 2 the Jacobian
+// (der) of jobs whose pass 1 has run, up to marks 3, 4. nid_kernels.cu: the Gauss-Newton block (gn), chi2 after pass 1,
+// with want_jac also H and b after pass 2.
+int launch_pass1(nid_ctx* c, const JobSet& js, Pass2 p2);
+int launch_pass2(nid_ctx* c, const JobSet& js);
+int launch_gn(nid_ctx* c, const JobSet& js, double delta, int want_jac);
+
 // sorted path (nid_sorted.cu)
 int sorted_init(nid_ctx* c);
 int launch_count_classes(nid_ctx* c, int pair);
 int launch_layout_and_scatter(nid_ctx* c, int pair0, int n);
 int launch_pack(nid_ctx* c, int pair0, int n);
 int launch_pack_k1(nid_ctx* c, int pair, unsigned short* d_out);
-int launch_eval_sorted(nid_ctx* c, int job0, int n_jobs, int n_jobs_total, int want_jac);
-// the two halves of an evaluation on explicit job lists (d_list / h_list: device and host copies, entries [first, first + n))
-int launch_sorted_pass1(nid_ctx* c, const int* d_list, const int* h_list, int first, int n, int tables);
-int launch_sorted_pass2(nid_ctx* c, const int* d_list, const int* h_list, int first, int n);
-int launch_gn_list(nid_ctx* c, const int* d_list, int first, int n, double delta, int want_jac);
 int launch_sorted_tail_gn(nid_ctx* c, const int* d_list, const int* h_list, int first, int n, double delta, double* gn_out);
 int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h_list, size_t h2d_bytes, double delta, double* gn_out);
 void destroy_latency_graph(nid_ctx* c);
@@ -345,15 +357,10 @@ int launch_downsample2(nid_ctx* dst, int dst_pair0, const nid_ctx* src, int src_
 int launch_prepare(nid_ctx* c, int pair0, int n, const double* d_poses16);
 int launch_ref_weights(nid_ctx* c, int pair);
 int launch_points_aos(nid_ctx* c, int pair, double* d_out);
-int launch_eval(nid_ctx* c, int n_jobs, int want_jac);
-int launch_eval_natural(nid_ctx* c, int n_jobs, int want_jac);
-int launch_gn(nid_ctx* c, int n_jobs, double delta);
 int launch_hard(nid_ctx* c, int n_jobs);
 int launch_warp_sample(nid_ctx* c, int pair, const double* d_pose16, int f64);
 int launch_warp_sample_jobs(nid_ctx* c, int n_jobs, float4* d_out, bool u16);
 int launch_check_integral(nid_ctx* c, const double* d_src, uint8_t* d_dst, int is_ref);
-int launch_chi2(nid_ctx* c, int n_jobs, double delta);
-int launch_eval_mixed(nid_ctx* c, int base, int nj, int nt, double delta);
 int launch_points_soa(nid_ctx* c, int pair, const double* d_in);
 int launch_import_flags(nid_ctx* c, int pair, const double* d_bsv);
 }  // namespace nid

@@ -1952,16 +1952,37 @@ static void launch_jac_w(nid_ctx* c, const EvalParams& p, int ns, int job0, int 
   }
 }
 
-// Pass 1 + assembly (histograms, entropies, err; with `tables` also the scaled log tables pass 2 needs) of the n jobs
-// d_list[first .. first + n) (d_list == nullptr: jobs first .. first + n - 1); h_list is the host copy of d_list.
-int launch_sorted_pass1(nid_ctx* c, const int* d_list, const int* h_list, int first, int n, int tables) {
-  EvalParams p = make_params(c, n);
-  p.job0 = first;
-  p.job_list = d_list;
+// the natural-order kernels (nid_kernels.cu)
+__global__ void k_hist(EvalParams p);
+__global__ void k_entropy(EvalParams p);
+__global__ void k_jac(EvalParams p);
+__global__ void k_jac_final(EvalParams p, int n_jobs);
+
+// Pass 1 of the jobs of js. Sorted: pixel kernel + assembly (histograms, entropies, err; unless p2 == none also the
+// scaled log tables pass 2 needs). Natural: strip histograms, then the cost tail k_entropy unless k_jac will write it.
+int launch_pass1(nid_ctx* c, const JobSet& js, Pass2 p2) {
+  EvalParams p = make_params(c, js.slots);
+  p.job0 = js.first;
+  p.job_list = js.d_list;
+  const int n = js.n;
+  if (!use_sorted(c)) {
+    const size_t smem = sizeof(double) * p.hist_stride;
+    ktime_mark(c, 0);
+    k_hist<<<dim3(p.S, p.ncell, n), 256, smem, c->stream>>>(p);
+    NID_LAUNCH_CHECK(c, "k_hist");
+    ktime_mark(c, 1);
+    if (p2 != Pass2::all) {
+      k_entropy<<<dim3(p.ncell, n), 256, smem, c->stream>>>(p);
+      NID_LAUNCH_CHECK(c, "k_entropy");
+    }
+    ktime_mark(c, 2);
+    return NID_OK;
+  }
+  const int tables = p2 != Pass2::none;
   const int ns = c->max_nslices_prepared;
   ktime_mark(c, 0);
   if (ns > 0) {  // (no slices at all: every cell of every prepared pair is inactive; the assembly reports NaN)
-    launch_hist_w(c, p, ns, first, n, h_list);
+    launch_hist_w(c, p, ns, js.first, n, js.h_list);
     c->launches--;
     NID_LAUNCH_CHECK(c, "k_hist_sell");
   }
@@ -1986,14 +2007,24 @@ int launch_sorted_pass1(nid_ctx* c, const int* d_list, const int* h_list, int fi
   return NID_OK;
 }
 
-// Pass 2 + Jacobian tail of the same kind of job list; the jobs' tables must be those of their current poses.
-int launch_sorted_pass2(nid_ctx* c, const int* d_list, const int* h_list, int first, int n) {
-  EvalParams p = make_params(c, n);
-  p.job0 = first;
-  p.job_list = d_list;
+// Pass 2 + Jacobian tail of the jobs of js; their pass 1 must have run at their current poses (sorted: with the tables).
+int launch_pass2(nid_ctx* c, const JobSet& js) {
+  EvalParams p = make_params(c, js.slots);
+  p.job0 = js.first;
+  p.job_list = js.d_list;
+  const int n = js.n;
+  if (!use_sorted(c)) {
+    k_jac<<<dim3(p.S, p.ncell, n), 256, sizeof(double) * p.hist_stride, c->stream>>>(p);
+    NID_LAUNCH_CHECK(c, "k_jac");
+    ktime_mark(c, 3);
+    k_jac_final<<<(n * p.ncell * 6 + 255) / 256, 256, 0, c->stream>>>(p, n);
+    NID_LAUNCH_CHECK(c, "k_jac_final");
+    ktime_mark(c, 4);
+    return NID_OK;
+  }
   const int ns = c->max_nslices_prepared;
   if (ns > 0) {
-    launch_jac_w(c, p, ns, first, n, h_list);
+    launch_jac_w(c, p, ns, js.first, n, js.h_list);
     c->launches--;
     NID_LAUNCH_CHECK(c, "k_jac_sell");
   }
@@ -2075,7 +2106,7 @@ static int capture_latency_graph(nid_ctx* c, LatencyGraph* g, int nslots, const 
   int r = NID_OK;
   e = cudaMemcpyAsync(c->poses, c->h_poses, h2d_bytes, cudaMemcpyHostToDevice, c->stream);
   if (e != cudaSuccess) r = check_cuda(e, "H2D poses + list (capture)");
-  if (r == NID_OK) r = launch_sorted_pass1(c, d_list, h_list, 0, nslots, 1);
+  if (r == NID_OK) r = launch_pass1(c, JobSet{d_list, h_list, 0, nslots, nslots}, Pass2::some);
   if (r == NID_OK) r = launch_sorted_tail_gn(c, d_list, h_list, 0, nslots, delta, gn_out);
   e = cudaStreamEndCapture(c->stream, &g->graph);
   if (r != NID_OK) return r;
@@ -2113,7 +2144,7 @@ int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h
   if (!graph_ok) {
     cudaError_t e = cudaMemcpyAsync(c->poses, c->h_poses, h2d_bytes, cudaMemcpyHostToDevice, c->stream);
     if (e != cudaSuccess) return check_cuda(e, "H2D poses + list");
-    int r = launch_sorted_pass1(c, d_list, h_list, 0, nslots, 1);
+    int r = launch_pass1(c, JobSet{d_list, h_list, 0, nslots, nslots}, Pass2::some);
     if (r != NID_OK) return r;
     return launch_sorted_tail_gn(c, d_list, h_list, 0, nslots, delta, gn_out);
   }
@@ -2144,22 +2175,6 @@ int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h
   const cudaError_t e = cudaGraphLaunch(g->exec, c->stream);
   if (e != cudaSuccess) return check_cuda(e, "cudaGraphLaunch");
   c->launches += 4;
-  return NID_OK;
-}
-
-int launch_eval_sorted(nid_ctx* c, int job0, int n_jobs, int n_jobs_total, int want_jac) {
-  (void)n_jobs_total;
-  int r = launch_sorted_pass1(c, nullptr, nullptr, job0, n_jobs, want_jac);
-  if (r != NID_OK) return r;
-  if (want_jac) {
-    r = launch_sorted_pass2(c, nullptr, nullptr, job0, n_jobs);
-    if (r != NID_OK) return r;
-    const int slot[4] = {0, 3, 1, 2};
-    ktime_collect(c, 4, slot);
-  } else {
-    const int slot[2] = {0, 3};
-    ktime_collect(c, 2, slot);
-  }
   return NID_OK;
 }
 
