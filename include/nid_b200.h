@@ -153,6 +153,23 @@ int nid_solve(nid_ctx* ctx, int pair, double pose7[7], int max_iters, double hub
 /* n independent solves in lockstep, pair job_pair[j] (NULL: pair j), poses7 [n][7] in/out, stats [n][3]. */
 int nid_solve_jobs(nid_ctx* ctx, int n, const int* job_pair, double* poses7, int max_iters,
                    double huber_delta, int* stats);
+/* Joint solves: n_groups independent problems; group g has group_size[g] >= 1 jobs (pairs) that share ONE unknown pose
+ * (a rig of cameras on one body, or several reference keyframes of one target frame). Jobs are listed group after group;
+ * job i uses pair job_pair[i] (NULL: pair i); the same pair may appear in several jobs. poses7 [n_groups][7] in/out is the
+ * group's pose T_bw as {t, q}. Job i is evaluated at T_cw1 = T_cb[i] * T_bw; T_cb [n_jobs][16] is column-major rigid
+ * camera-from-body (NULL: identity for every job, i.e. several pairs observed from one camera pose). One optimize(max_iters)
+ * per group over the cell edges of all its jobs: chi2, H and b are the sums over the jobs in job order, each job's Jacobian
+ * taken w.r.t. the body update T_bw <- exp(xi) * T_bw (J_body = J_cam * Ad(T_cb)). stats [n_groups][3] as in nid_solve,
+ * counting evaluations of the whole group; trace (may be NULL) [n_groups][max_iters][10] as in nid_solve (rows past a
+ * group's outer iterations are not written). Every job's pair must be prepared, at T_cb[i] * (initial T_bw) for the
+ * reference's semantics. sum(group_size) <= max_jobs. Runs in latency mode (see "lm_speculate") when there are at most 4
+ * groups and room for 2 trial poses of every job. A group of one job with T_cb NULL is exactly nid_solve_jobs of that job.
+ * Validated before any work; poses7, stats and trace are written only on success. NID_ERR_ARG: n_groups < 1, a group size
+ * < 1, more jobs than max_jobs, NULL poses7 or group_size, a job_pair out of range, a T_cb that is not rigid (bottom row
+ * not exactly (0,0,0,1), or R^T R != I to 1e-9, or det R < 0). NID_ERR_STATE: a job's pair not prepared.
+ * A group whose jobs have no active cell has chi2 == 0 and a zero system: it reports {1, 1, 1} and keeps its pose. */
+int nid_solve_groups(nid_ctx* ctx, int n_groups, const int* group_size, const int* job_pair, const double* T_cb,
+                     double* poses7, int max_iters, double huber_delta, int* stats, double* trace);
 /* Coarse-to-fine optimize(): levels[0] is the finest context, levels[n_levels-1] the coarsest (1 <= n_levels <= 8; build the
  * coarse levels with nid_set_pairs_downsampled). For l = n_levels-1 .. 0: prepare pairs job_pair[j] of levels[l] at the
  * current poses (nid_prepare_pairs), then nid_solve_jobs(levels[l], ..., max_iters[l], ...) and hand the poses down. Job pairs

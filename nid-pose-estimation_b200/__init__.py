@@ -68,6 +68,7 @@ def lib():
         L.nid_eval_gn.argtypes = [C.c_void_p, C.c_int, _dp, C.c_double, _dp, _dp, _dp, _dp, _dp]
         L.nid_solve.argtypes = [C.c_void_p, C.c_int, _dp, C.c_int, C.c_double, _dp, _ip]
         L.nid_solve_jobs.argtypes = [C.c_void_p, C.c_int, _ip, _dp, C.c_int, C.c_double, _ip]
+        L.nid_solve_groups.argtypes = [C.c_void_p, C.c_int, _ip, _ip, _dp, _dp, C.c_int, C.c_double, _ip, _dp]
         L.nid_set_pairs_downsampled.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int]
         L.nid_solve_pyramid_jobs.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_int, _ip, _dp, _ip, C.c_double, _ip]
         L.nid_hard_eval_jobs.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp]
@@ -261,6 +262,28 @@ class Context:
         _chk(lib().nid_solve_jobs(self._h, n, None if jp is None else jp.ctypes.data_as(_ip), _d(poses), max_iters,
                                   float(delta), stats.ctypes.data_as(_ip)))
         return poses, stats
+
+    def solve_groups(self, poses7, group_sizes, job_pair=None, T_cb=None, max_iters=10, delta=np.sqrt(0.95)):
+        """Joint solves (nid_solve_groups): group g's group_sizes[g] jobs share the pose poses7[g] (T_bw); job i is
+        evaluated at T_cb[i] @ T_bw (T_cb [n_jobs, 16] column-major, None: identity). Returns (poses [n, 7], stats [n, 3],
+        trace [n, max_iters, 10]); the trace rows past stats[g, 0] are zero."""
+        poses = _f64(poses7).copy().reshape(-1, 7)
+        n = poses.shape[0]
+        gs = np.ascontiguousarray(group_sizes, dtype=np.int32).reshape(-1)
+        jp = None if job_pair is None else np.ascontiguousarray(job_pair, dtype=np.int32)
+        E = None if T_cb is None else _f64(T_cb)
+        if gs.size != n:
+            raise ValueError(f"{n} poses but {gs.size} group sizes")
+        if jp is not None and jp.size != int(gs.sum()):
+            raise ValueError(f"{int(gs.sum())} jobs but {jp.size} job pairs")
+        if E is not None and E.size != 16 * int(gs.sum()):
+            raise ValueError(f"{int(gs.sum())} jobs but {E.size} doubles of T_cb")
+        stats = np.zeros((n, 3), dtype=np.int32)
+        trace = np.zeros((n, max(max_iters, 0), 10))
+        _chk(lib().nid_solve_groups(self._h, n, gs.ctypes.data_as(_ip), None if jp is None else jp.ctypes.data_as(_ip),
+                                    None if E is None else _d(E), _d(poses), max_iters, float(delta),
+                                    stats.ctypes.data_as(_ip), _d(trace)))
+        return poses, stats, trace
 
     # ---- a12
     def hard_eval_jobs(self, poses, job_pair=None):

@@ -204,8 +204,6 @@ struct nid_ctx {
   int opt_asm_wide = 1;  // 1024-thread assembly when there are fewer (cell, job) units than SMs
   int opt_lm_spec = 4;         // latency mode of nid_solve_jobs (few problems): trial poses evaluated per round and problem
   int opt_lm_reuse = 1;        // a cost+Jacobian job at the pose of the accepted trial reuses that trial's histograms and tables
-  double* lm_trace = nullptr;  // set by nid_solve for the duration of one call
-  int lm_trace_cap = 0;
   cudaEvent_t ev[2] = {nullptr, nullptr};
   // nid_set_pairs_downsampled into this context: [0] recorded on the source's stream before the kernel, [1] on this
   // context's stream after it (created on first use)

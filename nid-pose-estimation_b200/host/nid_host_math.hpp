@@ -147,6 +147,92 @@ inline Pose7 pose_exp(const double xi[6]) {  // se3quat.h:223-257
   return pose_from_Rt(R, t);
 }
 
+// 6x6 adjoint (row-major) of a rigid column-major 4x4 E = [R t; 0 1] for xi = (omega, upsilon):
+// E * exp(xi) * E^-1 = exp(Ad * xi), Ad = [[R, 0], [t^ R, R]].
+inline void adjoint6(const double E[16], double Ad[36]) {
+  double R[3][3], tx[3][3];
+  for (int r = 0; r < 3; r++)
+    for (int c = 0; c < 3; c++) R[r][c] = E[4 * c + r];
+  const double* t = E + 12;
+  tx[0][0] = 0; tx[0][1] = -t[2]; tx[0][2] = t[1];
+  tx[1][0] = t[2]; tx[1][1] = 0; tx[1][2] = -t[0];
+  tx[2][0] = -t[1]; tx[2][1] = t[0]; tx[2][2] = 0;
+  for (int r = 0; r < 3; r++)
+    for (int c = 0; c < 3; c++) {
+      double s = 0;
+      for (int k = 0; k < 3; k++) s += tx[r][k] * R[k][c];
+      Ad[6 * r + c] = R[r][c];
+      Ad[6 * r + c + 3] = 0.0;
+      Ad[6 * (r + 3) + c] = s;
+      Ad[6 * (r + 3) + c + 3] = R[r][c];
+    }
+}
+
+// A Gauss-Newton block {chi2, H[36] row-major, b[6], n_active} of a camera whose pose is E * T, re-expressed for the update
+// T <- exp(xi) * T of the body pose T: J_body = J_cam * Ad(E), so H -> Ad^T H Ad and b -> Ad^T b; chi2 and n_active stay.
+inline void gn_block_to_body(const double Ad[36], const double in[44], double out[44]) {
+  const double* H = in + 1;
+  double HA[36];
+  for (int i = 0; i < 6; i++)
+    for (int j = 0; j < 6; j++) {
+      double s = 0;
+      for (int k = 0; k < 6; k++) s += H[6 * i + k] * Ad[6 * k + j];
+      HA[6 * i + j] = s;
+    }
+  for (int i = 0; i < 6; i++) {
+    for (int j = 0; j < 6; j++) {
+      double s = 0;
+      for (int k = 0; k < 6; k++) s += Ad[6 * k + i] * HA[6 * k + j];
+      out[1 + 6 * i + j] = s;
+    }
+    double s = 0;
+    for (int k = 0; k < 6; k++) s += Ad[6 * k + i] * in[37 + k];
+    out[37 + i] = s;
+  }
+  out[0] = in[0];
+  out[43] = in[43];
+}
+
+// The block of a group of n jobs sharing one pose: the sum of the jobs' blocks in job order (blocks[44 * i ..]), each first
+// taken to the body frame when Ad is given (Ad[36 * i ..] per job). The first block is copied, not added to zero, so that a
+// group of one without Ad returns its job's block bit for bit.
+inline void gn_combine(int n, const double* blocks, const double* Ad, double out[44]) {
+  double tmp[44];
+  for (int i = 0; i < n; i++) {
+    const double* g = blocks + 44 * (size_t)i;
+    if (Ad) {
+      gn_block_to_body(Ad + 36 * (size_t)i, g, tmp);
+      g = tmp;
+    }
+    if (i == 0) std::memcpy(out, g, sizeof(double) * 44);
+    else for (int k = 0; k < 44; k++) out[k] += g[k];
+  }
+}
+
+// Is m a rigid column-major 4x4: bottom row exactly (0, 0, 0, 1), R^T R = I to tol per entry, det R > 0?
+inline bool is_rigid(const double m[16], double tol = 1e-9) {
+  if (!(m[3] == 0.0 && m[7] == 0.0 && m[11] == 0.0 && m[15] == 1.0)) return false;
+  for (int i = 0; i < 16; i++) if (!std::isfinite(m[i])) return false;
+  for (int a = 0; a < 3; a++)
+    for (int b = 0; b < 3; b++) {
+      double s = 0;
+      for (int r = 0; r < 3; r++) s += m[4 * a + r] * m[4 * b + r];
+      if (std::fabs(s - (a == b ? 1.0 : 0.0)) > tol) return false;
+    }
+  const double det = m[0] * (m[5] * m[10] - m[9] * m[6]) - m[4] * (m[1] * m[10] - m[9] * m[2]) + m[8] * (m[1] * m[6] - m[5] * m[2]);
+  return det > 0;
+}
+
+// out = A * B for column-major 4x4 (out may not alias A or B)
+inline void mat16_mul(const double A[16], const double B[16], double out[16]) {
+  for (int c = 0; c < 4; c++)
+    for (int r = 0; r < 4; r++) {
+      double s = 0;
+      for (int k = 0; k < 4; k++) s += A[4 * k + r] * B[4 * c + k];
+      out[4 * c + r] = s;
+    }
+}
+
 // Huber, robust_kernel_impl.cpp:78-90 with the `float dsqr` of robust_kernel_impl.h:84
 inline void huber(double e2, double delta, double rho[3]) {
   const double dsqr = (double)(float)(delta * delta);
