@@ -203,6 +203,9 @@ int nid_warp_sample_f64(nid_ctx* ctx, int pair, const double T_cw1[16], double* 
 int nid_debug_hist(nid_ctx* ctx, int job, int cell_index, double* P_t, double* P_j);
 /* number of kernels launched by this context so far */
 long long nid_launch_count(nid_ctx* ctx);
+/* number of CUDA resources (device and pinned buffers, streams, events, arrays, textures, graphs) held by all
+ * contexts of the process: a context releases every one of them in nid_destroy, and a failed nid_create holds none */
+long long nid_live_resources(void);
 /* accumulated device time (ms) and launch count per kernel since "time_kernels" was set:
  * [0] pass-1 histogram kernel, [1] pass-2 Jacobian kernel, [2] Jacobian tail, [3] entropy tail */
 int nid_kernel_times(nid_ctx* ctx, double ms[4], long long calls[4]);

@@ -78,6 +78,8 @@ def lib():
         L.nid_debug_hist.argtypes = [C.c_void_p, C.c_int, C.c_int, _dp, _dp]
         L.nid_launch_count.restype = C.c_longlong
         L.nid_launch_count.argtypes = [C.c_void_p]
+        L.nid_live_resources.restype = C.c_longlong
+        L.nid_live_resources.argtypes = []
         L.nid_set_option.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
         L.nid_kernel_times.argtypes = [C.c_void_p, _dp, C.POINTER(C.c_longlong)]
         L.nid_stream.restype = C.c_void_p
@@ -357,6 +359,11 @@ def solve_pyramid_jobs(levels, poses7, job_pair=None, max_iters=None, delta=np.s
     _chk(lib().nid_solve_pyramid_jobs(hs, L, n, None if jp is None else jp.ctypes.data_as(_ip), _d(poses),
                                       its.ctypes.data_as(_ip), float(delta), stats.ctypes.data_as(_ip)))
     return poses, stats
+
+
+def live_resources() -> int:
+    """CUDA resources held by all contexts of the process (nid_live_resources)."""
+    return int(lib().nid_live_resources())
 
 
 def exported_symbols_in_header():

@@ -6,6 +6,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <atomic>
 #include <limits>
 #include <string>
 #include <chrono>
@@ -65,7 +66,7 @@ EvalParams make_params(nid_ctx* c, int n_jobs) {
   p.lut_w = c->lut_w; p.lut_k = c->lut_k;
   p.poses = c->poses; p.job_pair = c->job_pair;
   const bool sorted = use_sorted(c);
-  p.part = c->part; p.jpart = sorted ? c->jpart_s : c->jpart; p.hist = c->opt_keep_hist ? c->hist : nullptr;
+  p.part = c->part; p.jpart = sorted ? c->jpart_s : c->jpart; p.hist = c->opt_keep_hist ? c->hist.get() : nullptr;
   p.ht = c->ht; p.hj = c->hj; p.err = c->err; p.der = c->der; p.gn = c->gn;
   p.sd0 = c->sd0; p.sd1 = c->sd1; p.sd2 = c->sd2; p.sid = c->sid;
   p.stage_bulk = (c->opt_stage_bulk < 0 ? (long long)c->rb * c->cb < NID_SMALL_CELL_PX : c->opt_stage_bulk) ? 1 : 0;
@@ -90,36 +91,37 @@ bool use_sorted(const nid_ctx* c) {
   return true;
 }
 
-template <typename T>
-static int dalloc(T** p, size_t n, const char* what) {
-  cudaError_t e = cudaMalloc((void**)p, sizeof(T) * (n ? n : 1));
-  if (e != cudaSuccess) return check_cuda(e, what);
-  return NID_OK;
+std::atomic<long long> live_handles{0};
+
+// Replaces a buffer by one of n elements. The old buffer is released only after the context stream has drained: work
+// queued on it may still read the buffer.
+template <typename B>
+static int regrow(nid_ctx* c, B& buf, size_t n, const char* sync_what, const char* what) {
+  CU(cudaStreamSynchronize(c->stream), sync_what);
+  return buf.alloc(n, what);
 }
 
 // per-job scratch of the active path, allocated on first use / grown when a pair with more tasks is prepared
 int ensure_job_buffers(nid_ctx* c) {
   const size_t J = c->job_cap, NC = c->ncell;
   const size_t hs = (size_t)c->bins * c->bins + c->bins;
-  if (c->opt_keep_hist && !c->hist) OKR(dalloc(&c->hist, J * NC * hs, "hist"));
+  if (c->opt_keep_hist && !c->hist) OKR(c->hist.alloc(J * NC * hs, "hist"));
   if (use_sorted(c)) {
     const size_t need = (size_t)std::max(c->max_ntasks_prepared, 1);
     if (c->g_stride < need) {
-      CU(cudaStreamSynchronize(c->stream), "sync before growing job buffers");
-      if (c->G) cudaFree(c->G);
-      c->G = nullptr;
-      OKR(dalloc(&c->G, J * need * c->bins, "G"));
+      c->g_stride = 0;
+      OKR(regrow(c, c->G, J * need * c->bins, "sync before growing job buffers", "G"));
       c->g_stride = need;
     }
-    if (!c->jpart_s) OKR(dalloc(&c->jpart_s, J * (size_t)c->max_slices * 6, "jpart_s"));  // one partial per slice
+    if (!c->jpart_s) OKR(c->jpart_s.alloc(J * (size_t)c->max_slices * 6, "jpart_s"));  // one partial per slice
     if (!c->wv) {
-      OKR(dalloc(&c->wv, J * NC * (size_t)nid::wv_stride(c->bins), "wv"));
+      OKR(c->wv.alloc(J * NC * (size_t)nid::wv_stride(c->bins), "wv"));
       CU(cudaMemset(c->wv, 0, sizeof(double) * J * NC * (size_t)nid::wv_stride(c->bins)), "memset wv");  // (the padding is copied, never used)
     }
   } else if (!c->part) {
     c->part_slots = J + 2 * (size_t)c->sm_count + 64;
-    OKR(dalloc(&c->part, c->part_slots * NC * hs, "part"));
-    OKR(dalloc(&c->jpart, c->part_slots * NC * 6, "jpart"));
+    OKR(c->part.alloc(c->part_slots * NC * hs, "part"));
+    OKR(c->jpart.alloc(c->part_slots * NC * 6, "jpart"));
   }
   return NID_OK;
 }
@@ -131,7 +133,7 @@ static int update_textures(nid_ctx* c, int pair0, int n) {
     const int nb = std::min(c->setup_batch, pair0 + n - p0);
     OKR(launch_pack(c, p0, nb));
     for (int i = 0; i < nb; i++)
-      CU(cudaMemcpy2DToArrayAsync(c->tex2_arrays[p0 + i], 0, 0, c->d_pack + (size_t)i * c->N, sizeof(unsigned) * c->cols,
+      CU(cudaMemcpy2DToArrayAsync(c->tex2[p0 + i].array, 0, 0, c->d_pack + (size_t)i * c->N, sizeof(unsigned) * c->cols,
                                   sizeof(unsigned) * c->cols, c->rows, cudaMemcpyDeviceToDevice, c->stream), "packed im1 -> texture array");
   }
   return NID_OK;
@@ -143,11 +145,9 @@ static int update_texture(nid_ctx* c, int pair) { return update_textures(c, pair
 static int arena_take(nid_ctx* c, size_t bytes, void** out) {
   bytes = (bytes + 63) & ~(size_t)63;
   if (bytes > c->h_arena_cap) {
-    CU(cudaStreamSynchronize(c->stream), "sync before growing the staging arena");
-    if (c->h_arena) cudaFreeHost(c->h_arena);
-    c->h_arena = nullptr; c->h_arena_cap = 0; c->h_arena_used = 0;
     const size_t cap = std::max(bytes * 4, (size_t)1 << 20);
-    CU(cudaMallocHost((void**)&c->h_arena, cap), "pinned staging arena");
+    c->h_arena_cap = 0; c->h_arena_used = 0;
+    OKR(regrow(c, c->h_arena, cap, "sync before growing the staging arena", "pinned staging arena"));
     c->h_arena_cap = cap;
   }
   if (c->h_arena_used + bytes > c->h_arena_cap) {
@@ -232,7 +232,7 @@ int nid_create(nid_ctx** out, int device, int rows, int cols, int cell, int bins
   }
   if (device < 0 || device >= ndev) { set_error("device index out of range"); return NID_ERR_ARG; }
   CU(cudaSetDevice(device), "cudaSetDevice");
-  nid_ctx* c = new nid_ctx();
+  auto c = std::make_unique<nid_ctx>();  // (released on every error return: the members free what was allocated)
   c->device = device; c->rows = rows; c->cols = cols; c->cell = cell; c->bins = bins; c->degree = degree;
   c->N = rows * cols; c->ncell = cell * cell; c->rb = rows / cell; c->cb = cols / cell;
   c->n_pairs = n_pairs; c->max_jobs = max_jobs;
@@ -240,14 +240,15 @@ int nid_create(nid_ctx** out, int device, int rows, int cols, int cell, int bins
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device), "cudaGetDeviceProperties");
   c->sm_count = prop.multiProcessorCount;
-  CU(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking), "cudaStreamCreate");
+  OKR(c->streams[0].create("cudaStreamCreate"));
+  c->stream = c->streams[0];
   const size_t N = c->N, P = n_pairs, J = c->job_cap, NC = c->ncell;
   const size_t hs = (size_t)bins * bins + bins;
-  OKR(dalloc(&c->pwx, P * N, "pwx")); OKR(dalloc(&c->pwy, P * N, "pwy")); OKR(dalloc(&c->pwz, P * N, "pwz"));
-  OKR(dalloc(&c->im0, P * N, "im0")); OKR(dalloc(&c->im1, P * N, "im1")); OKR(dalloc(&c->inb0, P * N, "inb0"));
-  OKR(dalloc(&c->n_c, P * NC, "n_c")); OKR(dalloc(&c->href, P * NC, "href"));
-  OKR(dalloc(&c->cam, P * 4, "cam")); OKR(dalloc(&c->Twc0, P * 16, "Twc0"));
-  OKR(dalloc(&c->cnt, P * NC * NID_NCLS, "cnt"));
+  OKR(c->pwx.alloc(P * N, "pwx")); OKR(c->pwy.alloc(P * N, "pwy")); OKR(c->pwz.alloc(P * N, "pwz"));
+  OKR(c->im0.alloc(P * N, "im0")); OKR(c->im1.alloc(P * N, "im1")); OKR(c->inb0.alloc(P * N, "inb0"));
+  OKR(c->n_c.alloc(P * NC, "n_c")); OKR(c->href.alloc(P * NC, "href"));
+  OKR(c->cam.alloc(P * 4, "cam")); OKR(c->Twc0.alloc(P * 16, "Twc0"));
+  OKR(c->cnt.alloc(P * NC * NID_NCLS, "cnt"));
   // pixels per task, by geometry only (never by the capacity of the context: a shard of a job must compute the same
   // bits as the whole job). Measured at 640x480, 96 evaluations in flight: 4x4 cells 144k evaluations/s with 32-pixel
   // tasks, 137k with 24, 126k with 16 (twice the task rows to assemble); 8x8 cells 112k / 110k / 103k; the reference's
@@ -261,22 +262,22 @@ int nid_create(nid_ctx** out, int device, int rows, int cols, int cell, int bins
   c->max_slices = c->max_tasks / 32 + (int)NC + 1;
   // pixel slots per pair: every task is padded to a multiple of 4 and every cell's slices to their longest task
   c->sell_cap = (N + 3 * (size_t)c->max_tasks + NC * 32 * (size_t)(NID_TASK_PX_MAX + 4) + 255) / 128 * 128;
-  OKR(dalloc(&c->depth, P * N, "depth"));
-  OKR(dalloc(&c->sl_off, P * ((size_t)c->max_slices + 1), "sl_off"));
-  OKR(dalloc(&c->sl_task, P * (size_t)c->max_slices * 32, "sl_task"));
-  OKR(dalloc(&c->sl_desc, P * (size_t)c->max_slices * 32, "sl_desc"));
-  OKR(dalloc(&c->task_cls, P * (size_t)c->max_tasks, "task_cls"));
-  OKR(dalloc(&c->sl_cell, P * (size_t)c->max_slices, "sl_cell"));
-  OKR(dalloc(&c->task_pos, P * (size_t)c->max_tasks, "task_pos"));
-  OKR(dalloc(&c->nslices, P, "nslices"));
+  OKR(c->depth.alloc(P * N, "depth"));
+  OKR(c->sl_off.alloc(P * ((size_t)c->max_slices + 1), "sl_off"));
+  OKR(c->sl_task.alloc(P * (size_t)c->max_slices * 32, "sl_task"));
+  OKR(c->sl_desc.alloc(P * (size_t)c->max_slices * 32, "sl_desc"));
+  OKR(c->task_cls.alloc(P * (size_t)c->max_tasks, "task_cls"));
+  OKR(c->sl_cell.alloc(P * (size_t)c->max_slices, "sl_cell"));
+  OKR(c->task_pos.alloc(P * (size_t)c->max_tasks, "task_pos"));
+  OKR(c->nslices.alloc(P, "nslices"));
   CU(cudaMemset(c->nslices, 0, sizeof(int) * P), "memset nslices");
   c->h_nslices.assign(P, 0);
-  OKR(dalloc(&c->tasks, P * (size_t)c->max_tasks, "tasks"));
-  OKR(dalloc(&c->ntasks, P, "ntasks"));
+  OKR(c->tasks.alloc(P * (size_t)c->max_tasks, "tasks"));
+  OKR(c->ntasks.alloc(P, "ntasks"));
   CU(cudaMemset(c->ntasks, 0, sizeof(int) * P), "memset ntasks");
-  OKR(dalloc(&c->cell_task_start, P * (NC + 1), "cell_task_start"));
-  OKR(dalloc(&c->cell_slice_start, P * (NC + 1), "cell_slice_start"));
-  OKR(dalloc(&c->cls_task_start, P * NC * (NID_NCLS + 1), "cls_task_start"));
+  OKR(c->cell_task_start.alloc(P * (NC + 1), "cell_task_start"));
+  OKR(c->cell_slice_start.alloc(P * (NC + 1), "cell_slice_start"));
+  OKR(c->cls_task_start.alloc(P * NC * (NID_NCLS + 1), "cls_task_start"));
   {
     // first class of every span: k_r(v) = floor(v' (B-3)/255), v' = 254.999 for v = 255, is monotone in v
     const int NS = bins - 3;
@@ -285,117 +286,72 @@ int nid_create(nid_ctx** out, int device, int rows, int cols, int cell, int bins
     for (int v = 255; v >= 0; v--)
       for (int k = 0; k <= kr(v) && k <= NS; k++) ss[k] = v;
     ss[NS] = 256;
-    OKR(dalloc(&c->span_start, ss.size(), "span_start"));
+    OKR(c->span_start.alloc(ss.size(), "span_start"));
     CU(cudaMemcpy(c->span_start, ss.data(), sizeof(int) * ss.size(), cudaMemcpyHostToDevice), "H2D span_start");
   }
   c->h_ntasks.assign(P, 0);
   // packed target images as gather-able textures (tex2Dgather needs a CUDA array created with cudaArrayTextureGather)
   {
-    bool ok = true;
     // packed I | Gx | Gy texels, 32 bit
-    c->tex2_arrays.assign(P, nullptr);
-    c->h_tex2.assign(P, 0);
-    cudaChannelFormatDesc cd2 = cudaCreateChannelDesc<unsigned int>();
-    for (size_t i = 0; i < P && ok; i++) {
-      if (cudaMallocArray(&c->tex2_arrays[i], &cd2, cols, rows, cudaArrayTextureGather) != cudaSuccess) { ok = false; break; }
-      cudaResourceDesc rd;
-      memset(&rd, 0, sizeof(rd));
-      rd.resType = cudaResourceTypeArray;
-      rd.res.array.array = c->tex2_arrays[i];
-      cudaTextureDesc td;
-      memset(&td, 0, sizeof(td));
-      td.addressMode[0] = td.addressMode[1] = cudaAddressModeClamp;
-      td.filterMode = cudaFilterModePoint;
-      td.readMode = cudaReadModeElementType;
-      td.normalizedCoords = 0;
-      if (cudaCreateTextureObject(&c->h_tex2[i], &rd, &td, nullptr) != cudaSuccess) ok = false;
+    c->tex2.resize(P);
+    std::vector<cudaTextureObject_t> h_tex2(P);
+    for (size_t i = 0; i < P; i++) {
+      if (c->tex2[i].create(cudaCreateChannelDesc<unsigned int>(), cols, rows, "packed target") != NID_OK) {
+        cudaGetLastError();
+        set_error("could not create the packed gather textures for the target images");
+        return NID_ERR_CUDA;
+      }
+      h_tex2[i] = c->tex2[i].tex;
     }
-    if (!ok) {
-      cudaGetLastError();
-      set_error("could not create the packed gather textures for the target images");
-      return NID_ERR_CUDA;
-    }
-    OKR(dalloc(&c->d_tex2, P, "d_tex2"));
-    OKR(dalloc(&c->d_k1tex, P, "d_k1tex"));
+    OKR(c->d_tex2.alloc(P, "d_tex2"));
+    OKR(c->d_k1tex.alloc(P, "d_k1tex"));
     CU(cudaMemset(c->d_k1tex, 0, sizeof(cudaTextureObject_t) * P), "memset k1tex");
-    c->k1_arrays.assign(P, nullptr);
-    c->h_k1tex.assign(P, 0);
+    c->k1tex.resize(P);
     c->k1_ready.assign(P, 0);
-    CU(cudaMemcpy(c->d_tex2, c->h_tex2.data(), sizeof(cudaTextureObject_t) * P, cudaMemcpyHostToDevice), "H2D tex2 handles");
+    CU(cudaMemcpy(c->d_tex2, h_tex2.data(), sizeof(cudaTextureObject_t) * P, cudaMemcpyHostToDevice), "H2D tex2 handles");
     c->setup_batch = (int)std::min<size_t>(P, 32);
-    OKR(dalloc(&c->d_pack, N * (size_t)c->setup_batch, "d_pack"));
-    OKR(dalloc(&c->lay_tot, (size_t)c->setup_batch * NC * 3, "lay_tot"));
-    OKR(dalloc(&c->lay_base, (size_t)c->setup_batch * NC * 3, "lay_base"));
-    OKR(dalloc(&c->prep_poses, (size_t)c->setup_batch * 16, "prep_poses"));
-    OKR(dalloc(&c->depth_factor, P, "depth_factor"));
+    OKR(c->d_pack.alloc(N * (size_t)c->setup_batch, "d_pack"));
+    OKR(c->lay_tot.alloc((size_t)c->setup_batch * NC * 3, "lay_tot"));
+    OKR(c->lay_base.alloc((size_t)c->setup_batch * NC * 3, "lay_base"));
+    OKR(c->prep_poses.alloc((size_t)c->setup_batch * 16, "prep_poses"));
+    OKR(c->depth_factor.alloc(P, "depth_factor"));
     c->pair_u16.assign(P, 0);
-    OKR(dalloc(&c->fp1, P * N, "fp1"));
+    OKR(c->fp1.alloc(P * N, "fp1"));
     c->h_Twc0.assign(P * 16, 0.0);
     c->h_cam.assign(P * 4, 1.0);
   }
-  OKR(dalloc(&c->d_depth, N, "d_depth")); OKR(dalloc(&c->d_img64, N, "d_img64")); OKR(dalloc(&c->d_flag, 2, "d_flag"));
+  OKR(c->d_depth.alloc(N, "d_depth")); OKR(c->d_img64.alloc(N, "d_img64")); OKR(c->d_flag.alloc(2, "d_flag"));
   CU(cudaMemset(c->d_flag, 0, sizeof(int) * 2), "memset flag");
-  OKR(dalloc(&c->lut_w, 256 * 4, "lut_w")); OKR(dalloc(&c->lut_k, 256, "lut_k"));
-  OKR(dalloc(&c->poses, J * 16, "poses")); OKR(dalloc(&c->job_pair, J, "job_pair"));
+  OKR(c->lut_w.alloc(256 * 4, "lut_w")); OKR(c->lut_k.alloc(256, "lut_k"));
+  OKR(c->pose_buf.alloc(J * 16, "poses")); OKR(c->job_pair.alloc(J, "job_pair"));
+  c->poses = c->pose_buf;
   CU(cudaMemset(c->job_pair, 0, sizeof(int) * J), "memset job_pair");
   CU(cudaMemset(c->poses, 0, sizeof(double) * 16 * J), "memset poses");
-  OKR(dalloc(&c->aux_pose, 16, "aux_pose"));
+  OKR(c->aux_pose.alloc(16, "aux_pose"));
   (void)hs;
-  OKR(dalloc(&c->ht, J * NC, "ht")); OKR(dalloc(&c->hj, J * NC, "hj")); OKR(dalloc(&c->err, J * NC, "err"));
-  OKR(dalloc(&c->der, J * NC * 6, "der")); OKR(dalloc(&c->gn, J * 44, "gn"));
-  OKR(dalloc(&c->hard, J * (NC + 1), "hard"));
-  CU(cudaMallocHost((void**)&c->h_poses_ring, sizeof(double) * 16 * J * NID_STAGE_RING), "pinned poses");
-  CU(cudaMallocHost((void**)&c->h_job_pair_ring, sizeof(int) * J * NID_STAGE_RING), "pinned job_pair");
+  OKR(c->ht.alloc(J * NC, "ht")); OKR(c->hj.alloc(J * NC, "hj")); OKR(c->err.alloc(J * NC, "err"));
+  OKR(c->der.alloc(J * NC * 6, "der")); OKR(c->gn.alloc(J * 44, "gn"));
+  OKR(c->hard.alloc(J * (NC + 1), "hard"));
+  OKR(c->h_poses_ring.alloc(16 * J * NID_STAGE_RING, "pinned poses"));
+  OKR(c->h_job_pair_ring.alloc(J * NID_STAGE_RING, "pinned job_pair"));
   memset(c->h_poses_ring, 0, sizeof(double) * 16 * J * NID_STAGE_RING);
   memset(c->h_job_pair_ring, 0, sizeof(int) * J * NID_STAGE_RING);
   c->h_poses = c->h_poses_ring;
   c->h_job_pair = c->h_job_pair_ring;
-  for (int i = 0; i < NID_STAGE_RING; i++) CU(cudaEventCreateWithFlags(&c->stage_ev[i], cudaEventDisableTiming), "cudaEventCreate (staging)");
-  CU(cudaMallocHost((void**)&c->h_aux_pose, sizeof(double) * 16), "pinned aux pose");
-  CU(cudaMallocHost((void**)&c->h_out, sizeof(double) * J * (NC * 8 + 44)), "pinned out");
+  for (auto& e : c->stage_ev) OKR(e.create(cudaEventDisableTiming, "cudaEventCreate (staging)"));
+  OKR(c->h_aux_pose.alloc(16, "pinned aux pose"));
+  OKR(c->h_out.alloc(J * (NC * 8 + 44), "pinned out"));
   c->pair_set.assign(P, 0);
   c->pair_prepared.assign(P, 0);
   c->pair_sorted.assign(P, 0);
-  OKR(launch_build_lut(c));
-  OKR(sorted_init(c));
+  OKR(launch_build_lut(c.get()));
+  OKR(sorted_init(c.get()));
   CU(cudaStreamSynchronize(c->stream), "sync after lut");
-  *out = c;
+  *out = c.release();
   return NID_OK;
 }
 
 int nid_destroy(nid_ctx* c) {
-  if (!c) return NID_OK;
-  cudaSetDevice(c->device);
-  cudaStreamSynchronize(c->stream);
-  void* ptrs[] = {c->pwx, c->pwy, c->pwz, c->im0, c->im1, c->inb0, c->n_c, c->href, c->cam, c->Twc0, c->cnt, c->d_depth,
-                  c->d_img64, c->d_flag, c->d_pix, c->d_pix4, c->d_pix4_jobs, c->chunk_cnt, c->d_bsv, c->d_bsi, c->lut_w, c->lut_k, c->poses,
-                  c->job_pair, c->aux_pose, c->part, c->jpart, c->hist, c->ht, c->hj, c->err, c->der, c->gn, c->hard,
-                  c->depth, c->sd0, c->sd1, c->sd2, c->sid, c->sl_off, c->sl_task, c->sl_desc, c->task_cls, c->sl_cell, c->nslices, c->task_pos,
-                  c->lay_tot, c->lay_base, c->prep_poses, c->depth16, c->depth_factor, c->d_tex2, c->d_pack, c->tasks, c->ntasks, c->cell_task_start, c->cell_slice_start, c->G, c->jpart_s, c->fp1, c->cls_task_start, c->span_start, c->wv};
-  for (auto t : c->h_k1tex) if (t) cudaDestroyTextureObject(t);
-  for (auto arr : c->k1_arrays) if (arr) cudaFreeArray(arr);
-  if (c->d_k1tex) cudaFree(c->d_k1tex);
-  if (c->d_k1pack) cudaFree(c->d_k1pack);
-  for (auto t : c->h_tex2) if (t) cudaDestroyTextureObject(t);
-  for (auto arr : c->tex2_arrays) if (arr) cudaFreeArray(arr);
-  for (void* p : ptrs) if (p) cudaFree(p);
-  if (c->h_poses_ring) cudaFreeHost(c->h_poses_ring);
-  if (c->h_job_pair_ring) cudaFreeHost(c->h_job_pair_ring);
-  if (c->h_aux_pose) cudaFreeHost(c->h_aux_pose);
-  if (c->h_lm_lists) cudaFreeHost(c->h_lm_lists);
-  destroy_latency_graph(c);
-  if (c->h_lm_stage) cudaFreeHost(c->h_lm_stage);
-  if (c->d_lm_stage) cudaFree(c->d_lm_stage);
-  if (c->d_lm_lists) cudaFree(c->d_lm_lists);
-  for (int i = 0; i < NID_STAGE_RING; i++) if (c->stage_ev[i]) cudaEventDestroy(c->stage_ev[i]);
-  if (c->h_out) cudaFreeHost(c->h_out);
-  if (c->h_arena) cudaFreeHost(c->h_arena);
-  if (c->h_res) cudaFreeHost(c->h_res);
-  for (int i = 0; i < 2; i++) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
-  for (int i = 0; i < 2; i++) if (c->ds_ev[i]) cudaEventDestroy(c->ds_ev[i]);
-  for (int i = 0; i < 5; i++) if (c->kev[i]) cudaEventDestroy(c->kev[i]);
-  cudaStreamDestroy(c->stream);
-  if (c->stream2) cudaStreamDestroy(c->stream2);
   delete c;
   return NID_OK;
 }
@@ -417,7 +373,7 @@ static int set_pairs_geometry(nid_ctx* c, int pair0, int n, const double* depth6
   CU(cudaSetDevice(c->device), "cudaSetDevice");
   const size_t N = c->N;
   if (depth16) {
-    if (!c->depth16) OKR(dalloc(&c->depth16, (size_t)c->n_pairs * N, "depth16"));
+    if (!c->depth16) OKR(c->depth16.alloc((size_t)c->n_pairs * N, "depth16"));
     CU(cudaMemcpyAsync(c->depth16 + (size_t)pair0 * N, depth16, sizeof(uint16_t) * N * n, cudaMemcpyDefault, c->stream), "H2D depth (u16)");
   } else {
     CU(cudaMemcpyAsync(c->depth + (size_t)pair0 * N, depth64, sizeof(double) * N * n, cudaMemcpyDefault, c->stream), "H2D depth");
@@ -495,7 +451,7 @@ int nid_set_pairs_downsampled(nid_ctx* dst, int dst_pair0, const nid_ctx* src, i
     if (!src->pair_set[src_pair0 + i]) { set_error("source pair not set"); return NID_ERR_STATE; }
   CU(cudaSetDevice(dst->device), "cudaSetDevice");
   for (int i = 0; i < 2; i++)
-    if (!dst->ds_ev[i]) CU(cudaEventCreateWithFlags(&dst->ds_ev[i], cudaEventDisableTiming), "cudaEventCreate (downsample)");
+    if (!dst->ds_ev[i]) OKR(dst->ds_ev[i].create(cudaEventDisableTiming, "cudaEventCreate (downsample)"));
   double* a = nullptr;
   OKR(arena_take(dst, sizeof(double) * 5 * n, (void**)&a));
   double *acam = a, *afac = a + 4 * (size_t)n;
@@ -579,7 +535,7 @@ int nid_set_pair_points(nid_ctx* c, int pair, const double* points_3d, const dou
   CU(cudaSetDevice(c->device), "cudaSetDevice");
   if (points_3d) {
     if (!intr) { set_error("intr required with points"); return NID_ERR_ARG; }
-    if (!c->d_pix) OKR(dalloc(&c->d_pix, (size_t)8 * c->N, "d_pix"));
+    if (!c->d_pix) OKR(c->d_pix.alloc((size_t)8 * c->N, "d_pix"));
     CU(cudaMemcpyAsync(c->d_pix, points_3d, sizeof(double) * 3 * c->N, cudaMemcpyDefault, c->stream), "H2D points3d");
     CU(cudaMemcpyAsync(c->cam + 4 * pair, intr, sizeof(double) * 4, cudaMemcpyDefault, c->stream), "H2D intr");
     memcpy(c->h_cam.data() + 4 * (size_t)pair, intr, sizeof(double) * 4);
@@ -601,7 +557,7 @@ int nid_import_prepare(nid_ctx* c, int pair, const double* bs_value, const int* 
   if (!c || pair < 0 || pair >= c->n_pairs || !bs_value || !bs_counter || !Href) { set_error("bad argument"); return NID_ERR_ARG; }
   if (!c->pair_set[pair]) { set_error("pair not set"); return NID_ERR_STATE; }
   CU(cudaSetDevice(c->device), "cudaSetDevice");
-  if (!c->d_bsv) { OKR(dalloc(&c->d_bsv, (size_t)4 * c->N, "d_bsv")); OKR(dalloc(&c->d_bsi, (size_t)c->N, "d_bsi")); }
+  if (!c->d_bsv) { OKR(c->d_bsv.alloc((size_t)4 * c->N, "d_bsv")); OKR(c->d_bsi.alloc((size_t)c->N, "d_bsi")); }
   CU(cudaMemcpyAsync(c->d_bsv, bs_value, sizeof(double) * 4 * c->N, cudaMemcpyDefault, c->stream), "H2D bs_value");
   OKR(launch_import_flags(c, pair, c->d_bsv));
   CU(cudaMemcpyAsync(c->n_c + pair * c->ncell, bs_counter, sizeof(int) * c->ncell, cudaMemcpyDefault, c->stream), "H2D n_c");
@@ -627,7 +583,7 @@ int nid_get_points3d(nid_ctx* c, int pair, double* points_3d) {
   if (!c || pair < 0 || pair >= c->n_pairs || !points_3d) { set_error("bad argument"); return NID_ERR_ARG; }
   if (!c->pair_set[pair]) { set_error("pair not set"); return NID_ERR_STATE; }
   CU(cudaSetDevice(c->device), "cudaSetDevice");
-  if (!c->d_pix) OKR(dalloc(&c->d_pix, (size_t)8 * c->N, "d_pix"));
+  if (!c->d_pix) OKR(c->d_pix.alloc((size_t)8 * c->N, "d_pix"));
   OKR(launch_points_aos(c, pair, c->d_pix));
   CU(cudaMemcpyAsync(points_3d, c->d_pix, sizeof(double) * 3 * c->N, cudaMemcpyDefault, c->stream), "copy points3d");
   CU(cudaStreamSynchronize(c->stream), "sync points3d");
@@ -641,16 +597,16 @@ static int build_sorted_layout(nid_ctx* c, int pair0, int n) {
   for (int i = 0; i < n; i++) c->pair_sorted[pair0 + i] = 0;
   if (!use_sorted(c)) return NID_OK;  // the natural-order kernels need none of this
   if (!c->sd0) {
-    OKR(dalloc(&c->sd0, (size_t)c->n_pairs * c->sell_cap, "sd0"));
-    OKR(dalloc(&c->sid, (size_t)c->n_pairs * c->sell_cap, "sid"));
+    OKR(c->sd0.alloc((size_t)c->n_pairs * c->sell_cap, "sd0"));
+    OKR(c->sid.alloc((size_t)c->n_pairs * c->sell_cap, "sid"));
   }
   if (c->sell_points && !c->sd1) {
-    OKR(dalloc(&c->sd1, (size_t)c->n_pairs * c->sell_cap, "sd1"));
-    OKR(dalloc(&c->sd2, (size_t)c->n_pairs * c->sell_cap, "sd2"));
+    OKR(c->sd1.alloc((size_t)c->n_pairs * c->sell_cap, "sd1"));
+    OKR(c->sd2.alloc((size_t)c->n_pairs * c->sell_cap, "sd2"));
   }
   if (!c->chunk_cnt) {
     const size_t nchunks = ((size_t)c->rb * c->cb + 255) / 256;
-    OKR(dalloc(&c->chunk_cnt, (size_t)c->setup_batch * c->ncell * nchunks * NID_NCLS, "chunk_cnt"));
+    OKR(c->chunk_cnt.alloc((size_t)c->setup_batch * c->ncell * nchunks * NID_NCLS, "chunk_cnt"));
   }
   for (int p0 = pair0; p0 < pair0 + n; p0 += c->setup_batch)
     OKR(launch_layout_and_scatter(c, p0, std::min(c->setup_batch, pair0 + n - p0)));
@@ -662,13 +618,11 @@ static int finish_sorted_layout(nid_ctx* c, int pair0, int n, int* bs_counter, d
   const size_t NC = c->ncell;
   const size_t bytes = (size_t)n * (NC * (sizeof(double) + sizeof(int)) + 2 * sizeof(int)) + sizeof(int) + 64;
   if (c->h_res_cap < bytes) {
-    CU(cudaStreamSynchronize(c->stream), "sync before growing the result buffer");
-    if (c->h_res) cudaFreeHost(c->h_res);
-    c->h_res = nullptr; c->h_res_cap = 0;
-    CU(cudaMallocHost((void**)&c->h_res, bytes * 2), "pinned prepare results");
+    c->h_res_cap = 0;
+    OKR(regrow(c, c->h_res, bytes * 2, "sync before growing the result buffer", "pinned prepare results"));
     c->h_res_cap = bytes * 2;
   }
-  double* h_href = (double*)c->h_res;
+  double* h_href = (double*)c->h_res.get();
   int* h_nc = (int*)(h_href + (size_t)n * NC);
   int* h_nt = h_nc + (size_t)n * NC;
   int* h_ns = h_nt + n;
@@ -729,7 +683,7 @@ int nid_get_ref_weights(nid_ctx* c, int pair, double* bs_value, int* bs_index) {
   if (!c || pair < 0 || pair >= c->n_pairs) { set_error("bad argument"); return NID_ERR_ARG; }
   if (!c->pair_prepared[pair]) { set_error("pair not prepared"); return NID_ERR_STATE; }
   CU(cudaSetDevice(c->device), "cudaSetDevice");
-  if (!c->d_bsv) { OKR(dalloc(&c->d_bsv, (size_t)4 * c->N, "d_bsv")); OKR(dalloc(&c->d_bsi, (size_t)c->N, "d_bsi")); }
+  if (!c->d_bsv) { OKR(c->d_bsv.alloc((size_t)4 * c->N, "d_bsv")); OKR(c->d_bsi.alloc((size_t)c->N, "d_bsi")); }
   OKR(launch_ref_weights(c, pair));
   if (bs_value) CU(cudaMemcpyAsync(bs_value, c->d_bsv, sizeof(double) * 4 * c->N, cudaMemcpyDefault, c->stream), "D2H bs_value");
   if (bs_index) CU(cudaMemcpyAsync(bs_index, c->d_bsi, sizeof(int) * c->N, cudaMemcpyDefault, c->stream), "D2H bs_index");
@@ -931,16 +885,16 @@ static int solve_speculative(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs,
   // kernels read both from there for the duration of the solve
   const int nslots = n_jobs * K;
   const size_t stage_bytes = sizeof(double) * 16 * (size_t)c->job_cap + sizeof(int) * (size_t)c->job_cap;
-  if (!c->h_lm_stage) {
-    CU(cudaMallocHost((void**)&c->h_lm_stage, stage_bytes), "pinned LM staging");
-    CU(cudaMalloc((void**)&c->d_lm_stage, stage_bytes), "LM staging");
+  if (!c->d_lm_stage) {
+    OKR(c->h_lm_stage.alloc(stage_bytes, "pinned LM staging"));
+    OKR(c->d_lm_stage.alloc(stage_bytes, "LM staging"));
   }
   struct Swap {  // restores the context's pose buffers on every way out
     nid_ctx* c; double* poses; double* h_poses;
     ~Swap() { c->poses = poses; c->h_poses = h_poses; }
   } swap{c, c->poses, c->h_poses};
-  c->poses = reinterpret_cast<double*>(c->d_lm_stage);
-  c->h_poses = reinterpret_cast<double*>(c->h_lm_stage);
+  c->poses = reinterpret_cast<double*>(c->d_lm_stage.get());
+  c->h_poses = reinterpret_cast<double*>(c->h_lm_stage.get());
   int* const list = reinterpret_cast<int*>(c->h_poses + 16 * (size_t)nslots);
   int* const d_list = reinterpret_cast<int*>(c->poses + 16 * (size_t)nslots);
   auto slot_of = [&](int j, int k, int g) { return st[j].slot0 * K + k * st[j].nj + g; };
@@ -1048,12 +1002,10 @@ static int solve_lockstep(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs, in
   // (the natural-order kernels index their partial buffers by (slot, cell, strip): two halves in flight would need the
   // same strip count S)
   const int nh = (n >= 8 && sorted) ? 2 : 1;
-  if (nh == 2 && !c->stream2) {
-    CU(cudaStreamCreateWithFlags(&c->stream2, cudaStreamNonBlocking), "cudaStreamCreate (LM)");
-  }
-  if (!c->h_lm_lists) {
-    CU(cudaMallocHost((void**)&c->h_lm_lists, sizeof(int) * 2 * (size_t)c->job_cap), "pinned LM lists");
-    OKR(dalloc(&c->d_lm_lists, 2 * (size_t)c->job_cap, "LM lists"));
+  if (nh == 2 && !c->streams[1]) OKR(c->streams[1].create("cudaStreamCreate (LM)"));
+  if (!c->d_lm_lists) {
+    OKR(c->h_lm_lists.alloc(2 * (size_t)c->job_cap, "pinned LM lists"));
+    OKR(c->d_lm_lists.alloc(2 * (size_t)c->job_cap, "LM lists"));
   }
   CU(cudaStreamSynchronize(c->stream), "sync before LM");
   // half h owns the problems [p0, p1), their slots [lo, hi) and the list storage [2 lo, 2 hi): list 1 then list 2
@@ -1063,7 +1015,7 @@ static int solve_lockstep(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs, in
   };
   Half H[2];
   H[0] = half(0, nh == 2 ? n / 2 : n, c->stream);
-  H[1] = half(n / 2, n, c->stream2);
+  H[1] = half(n / 2, n, c->streams[1]);
   cudaStream_t const main_stream = c->stream;
   for (int j = 0; j < n; j++)
     for (int g = 0; g < st[j].nj; g++) c->h_job_pair[st[j].slot0 + g] = st[j].pairs[g];
@@ -1124,7 +1076,7 @@ static int solve_lockstep(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs, in
     }
   }
   c->stream = main_stream;
-  if (nh == 2) cudaStreamSynchronize(c->stream2);
+  if (nh == 2) cudaStreamSynchronize(c->streams[1]);
   cudaStreamSynchronize(main_stream);
   return rc;
 }
@@ -1268,8 +1220,8 @@ static int warp_sample_common(nid_ctx* c, int pair, const double T_cw1[16], int 
   if (!c || pair < 0 || pair >= c->n_pairs || !T_cw1) { set_error("bad argument"); return NID_ERR_ARG; }
   if (!c->pair_set[pair]) { set_error("pair not set"); return NID_ERR_STATE; }
   CU(cudaSetDevice(c->device), "cudaSetDevice");
-  if (f64 && !c->d_pix) OKR(dalloc(&c->d_pix, (size_t)8 * c->N, "d_pix"));
-  if (!f64 && !c->d_pix4) OKR(dalloc(&c->d_pix4, (size_t)4 * c->N, "d_pix4"));
+  if (f64 && !c->d_pix) OKR(c->d_pix.alloc((size_t)8 * c->N, "d_pix"));
+  if (!f64 && !c->d_pix4) OKR(c->d_pix4.alloc((size_t)4 * c->N, "d_pix4"));
   memcpy(c->h_aux_pose, T_cw1, sizeof(double) * 16);  // (both callers synchronise before returning)
   CU(cudaMemcpyAsync(c->aux_pose, c->h_aux_pose, sizeof(double) * 16, cudaMemcpyHostToDevice, c->stream), "H2D pose");
   return launch_warp_sample(c, pair, c->aux_pose, f64);
@@ -1286,25 +1238,15 @@ int nid_warp_sample(nid_ctx* c, int pair, const double T_cw1[16], float* out) {
 // and filled the first time the pair is used by nid_warp_sample_jobs after its target image changed.
 static int ensure_k1_texture(nid_ctx* c, int pair) {
   if (c->k1_ready[pair]) return NID_OK;
-  if (!c->k1_arrays[pair]) {
-    cudaChannelFormatDesc cd = cudaCreateChannelDescHalf();
-    CU(cudaMallocArray(&c->k1_arrays[pair], &cd, c->cols, 3 * c->rows, cudaArrayTextureGather), "cudaMallocArray (kernel-1 planes)");
-    cudaResourceDesc rd;
-    memset(&rd, 0, sizeof(rd));
-    rd.resType = cudaResourceTypeArray;
-    rd.res.array.array = c->k1_arrays[pair];
-    cudaTextureDesc td;
-    memset(&td, 0, sizeof(td));
-    td.addressMode[0] = td.addressMode[1] = cudaAddressModeClamp;
-    td.filterMode = cudaFilterModePoint;
-    td.readMode = cudaReadModeElementType;
-    td.normalizedCoords = 0;
-    CU(cudaCreateTextureObject(&c->h_k1tex[pair], &rd, &td, nullptr), "cudaCreateTextureObject (kernel-1 planes)");
-    CU(cudaMemcpyAsync(c->d_k1tex + pair, &c->h_k1tex[pair], sizeof(cudaTextureObject_t), cudaMemcpyHostToDevice, c->stream), "H2D k1 texture handle");
+  nid::GatherTexture& t = c->k1tex[pair];
+  if (!t.tex) {
+    OKR(t.create(cudaCreateChannelDescHalf(), c->cols, 3 * c->rows, "kernel-1 planes"));
+    CU(cudaMemcpyAsync(c->d_k1tex + pair, t.tex.handle_address(), sizeof(cudaTextureObject_t), cudaMemcpyHostToDevice, c->stream),
+       "H2D k1 texture handle");
   }
-  if (!c->d_k1pack) OKR(dalloc(&c->d_k1pack, (size_t)3 * c->N, "d_k1pack"));
+  if (!c->d_k1pack) OKR(c->d_k1pack.alloc((size_t)3 * c->N, "d_k1pack"));
   OKR(launch_pack_k1(c, pair, c->d_k1pack));
-  CU(cudaMemcpy2DToArrayAsync(c->k1_arrays[pair], 0, 0, c->d_k1pack, sizeof(unsigned short) * c->cols, sizeof(unsigned short) * c->cols,
+  CU(cudaMemcpy2DToArrayAsync(t.array, 0, 0, c->d_k1pack, sizeof(unsigned short) * c->cols, sizeof(unsigned short) * c->cols,
                               3 * c->rows, cudaMemcpyDeviceToDevice, c->stream), "fp16 planes -> texture array");
   c->k1_ready[pair] = 1;
   return NID_OK;
@@ -1315,7 +1257,7 @@ int nid_warp_sample_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const doub
   CU(cudaSetDevice(c->device), "cudaSetDevice");
   if (n_jobs < 1 || n_jobs > c->max_jobs) { set_error("n_jobs out of range"); return NID_ERR_ARG; }
   if (c->sell_points) { set_error("nid_warp_sample_jobs needs depth pairs (nid_set_pair), not caller-supplied points"); return NID_ERR_UNSUPPORTED; }
-  if (!c->d_pix4_jobs) OKR(dalloc(&c->d_pix4_jobs, (size_t)4 * c->N * c->max_jobs, "d_pix4_jobs"));
+  if (!c->d_pix4_jobs) OKR(c->d_pix4_jobs.alloc((size_t)4 * c->N * c->max_jobs, "d_pix4_jobs"));
   OKR(stage_jobs(c, n_jobs, job_pair, poses, 1));
   c->staged_jobs = 0;  // (not evaluation jobs: the pairs need not be prepared)
   // pairs uploaded as raw 16-bit depth are read as such (2 B/px); a mixed batch falls back to the fp64 planes, which
@@ -1325,7 +1267,7 @@ int nid_warp_sample_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const doub
     u16 = u16 && c->pair_u16[c->h_job_pair[j]];
     OKR(ensure_k1_texture(c, c->h_job_pair[j]));
   }
-  OKR(launch_warp_sample_jobs(c, n_jobs, (float4*)c->d_pix4_jobs, u16));
+  OKR(launch_warp_sample_jobs(c, n_jobs, (float4*)c->d_pix4_jobs.get(), u16));
   if (out) CU(cudaMemcpyAsync(out, c->d_pix4_jobs, sizeof(float) * 4 * c->N * (size_t)n_jobs, cudaMemcpyDefault, c->stream), "D2H pix4 jobs");
   CU(cudaStreamSynchronize(c->stream), "sync warp_sample_jobs");
   return NID_OK;
@@ -1352,6 +1294,8 @@ int nid_debug_hist(nid_ctx* c, int job, int cell_index, double* P_t, double* P_j
 
 long long nid_launch_count(nid_ctx* c) { return c ? c->launches : 0; }
 
+long long nid_live_resources(void) { return live_handles.load(); }
+
 int nid_kernel_times(nid_ctx* c, double ms[4], long long calls[4]) {
   if (!c || !ms || !calls) { set_error("bad argument"); return NID_ERR_ARG; }
   for (int i = 0; i < 4; i++) { ms[i] = c->kernel_ms[i]; calls[i] = c->kernel_calls[i]; }
@@ -1363,7 +1307,7 @@ void* nid_stream(nid_ctx* c) { return c ? (void*)c->stream : nullptr; }
 int nid_event_record(nid_ctx* c, int slot) {
   if (!c || slot < 0 || slot > 1) { set_error("bad argument"); return NID_ERR_ARG; }
   CU(cudaSetDevice(c->device), "cudaSetDevice");
-  if (!c->ev[slot]) CU(cudaEventCreate(&c->ev[slot]), "cudaEventCreate");
+  if (!c->ev[slot]) OKR(c->ev[slot].create(cudaEventDefault, "cudaEventCreate"));
   CU(cudaEventRecord(c->ev[slot], c->stream), "cudaEventRecord");
   return NID_OK;
 }

@@ -2,10 +2,12 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <memory>
 #include <string>
 #include <vector>
 
 #include "../../include/nid_b200.h"
+#include "nid_handles.h"
 
 #define NID_NCLS 257  /* reference-intensity classes 0..255 + 256 = valid point without reference sample */
 #define NID_SORTED_MIN_BINS 6  /* the two 3x3 end blocks of the basis fold must not overlap */
@@ -82,7 +84,12 @@ struct EvalParams {
 
 }  // namespace nid
 
-namespace nid { struct LatencyGraph; }
+namespace nid {
+struct LatencyGraph;
+struct LatencyGraphDelete { void operator()(LatencyGraph* g) const; };  // (nid_sorted.cu)
+}  // namespace nid
+// A context owns every handle it holds (nid_handles.h); `stream`, `poses`, `h_poses` and `h_job_pair` are views that are
+// pointed elsewhere at run time, their storage is owned by separate members.
 struct nid_ctx {
   int device = 0;
   int rows = 0, cols = 0, cell = 0, bins = 0, degree = 3;
@@ -90,113 +97,108 @@ struct nid_ctx {
   int n_pairs = 0, max_jobs = 0;
   int job_cap = 0;             // job slots actually allocated: max(max_jobs, NID_MIN_JOB_SLOTS) (speculative LM trials need a few)
   int sm_count = 148;
-  cudaStream_t stream = nullptr;
-  int* chunk_cnt = nullptr;    // [setup_batch][ncell][chunks of 256 px][NID_NCLS] scratch of the regrouping scatter
+  // [0] the context stream, [1] the second stream of the ping-pong LM driver (nid_solve_jobs), created on first use
+  nid::Stream streams[2];
+  cudaStream_t stream = nullptr;  // the stream the launchers issue on: streams[0], or the stream of a lock-step LM half
+  nid::DeviceBuffer<int> chunk_cnt;    // [setup_batch][ncell][chunks of 256 px][NID_NCLS] scratch of the regrouping scatter
   // batched pair set-up (nid_set_pairs_u16 / nid_prepare_pairs): up to setup_batch pairs per launch
   int setup_batch = 1;
-  int* lay_tot = nullptr;      // [setup_batch][ncell][3] tasks, slices, pixel slots of every cell
-  int* lay_base = nullptr;     // [setup_batch][ncell][3] their exclusive scans over the cells of a pair
-  double* prep_poses = nullptr;  // [setup_batch][16] initial poses of the batch
-  uint16_t* depth16 = nullptr; // [n_pairs][N] raw 16-bit depth (allocated by the first nid_set_pairs_u16)
-  double* depth_factor = nullptr;  // [n_pairs]
+  nid::DeviceBuffer<int> lay_tot;     // [setup_batch][ncell][3] tasks, slices, pixel slots of every cell
+  nid::DeviceBuffer<int> lay_base;    // [setup_batch][ncell][3] their exclusive scans over the cells of a pair
+  nid::DeviceBuffer<double> prep_poses;  // [setup_batch][16] initial poses of the batch
+  nid::DeviceBuffer<uint16_t> depth16; // [n_pairs][N] raw 16-bit depth (allocated by the first nid_set_pairs_u16)
+  nid::DeviceBuffer<double> depth_factor;  // [n_pairs]
   std::vector<char> pair_u16;  // the pair's depth16 plane is valid
-  char* h_arena = nullptr;     // pinned bump arena for the small per-pair arrays of the asynchronous set-up calls
+  nid::PinnedBuffer<char> h_arena;    // pinned bump arena for the small per-pair arrays of the asynchronous set-up calls
   size_t h_arena_cap = 0, h_arena_used = 0;
-  char* h_res = nullptr;       // pinned results of nid_prepare_pairs (n_c, H_ref, task and slice counts)
+  nid::PinnedBuffer<char> h_res;      // pinned results of nid_prepare_pairs (n_c, H_ref, task and slice counts)
   size_t h_res_cap = 0;
-  cudaStream_t stream2 = nullptr;  // second stream of the ping-pong LM driver (nid_solve_jobs)
   long long launches = 0;
 
   // per pair
-  double *pwx = nullptr, *pwy = nullptr, *pwz = nullptr;
-  uint8_t *im0 = nullptr, *im1 = nullptr, *inb0 = nullptr;
-  int* n_c = nullptr;
-  double* href = nullptr;
-  double* cam = nullptr;
-  double* Twc0 = nullptr;      // [n_pairs][16]
-  unsigned int* cnt = nullptr; // [n_pairs][ncell][NID_NCLS] pixel counts per reference class at prepare
+  nid::DeviceBuffer<double> pwx, pwy, pwz;
+  nid::DeviceBuffer<uint8_t> im0, im1, inb0;
+  nid::DeviceBuffer<int> n_c;
+  nid::DeviceBuffer<double> href, cam;
+  nid::DeviceBuffer<double> Twc0;     // [n_pairs][16]
+  nid::DeviceBuffer<unsigned int> cnt; // [n_pairs][ncell][NID_NCLS] pixel counts per reference class at prepare
   // sorted path, per pair
-  double* depth = nullptr;     // [n_pairs][N] reference depth as uploaded (depth form)
-  double *sd0 = nullptr, *sd1 = nullptr, *sd2 = nullptr;
-  unsigned* sid = nullptr;
+  nid::DeviceBuffer<double> depth;    // [n_pairs][N] reference depth as uploaded (depth form)
+  nid::DeviceBuffer<double> sd0, sd1, sd2;
+  nid::DeviceBuffer<unsigned> sid;
   size_t sell_cap = 0;
-  int* sl_desc = nullptr;
-  unsigned short* task_cls = nullptr;
-  int *sl_off = nullptr, *sl_task = nullptr, *sl_cell = nullptr, *nslices = nullptr, *task_pos = nullptr;
+  nid::DeviceBuffer<int> sl_desc;
+  nid::DeviceBuffer<unsigned short> task_cls;
+  nid::DeviceBuffer<int> sl_off, sl_task, sl_cell, nslices, task_pos;
   int max_slices = 0;
   std::vector<int> h_nslices;
   int max_nslices_prepared = 0;
   int task_px = 32;            // L: pixels per task
   bool sell_points = false;    // pairs carry caller-supplied world points (nid_set_pair_points)
-  int2* tasks = nullptr;
-  int* ntasks = nullptr;
-  int* cell_task_start = nullptr;
-  int* cell_slice_start = nullptr;
-  int* cls_task_start = nullptr;
-  int* span_start = nullptr;
-  double* wv = nullptr;
+  nid::DeviceBuffer<int2> tasks;
+  nid::DeviceBuffer<int> ntasks, cell_task_start, cell_slice_start, cls_task_start, span_start;
+  nid::DeviceBuffer<double> wv;
   int max_tasks = 0;
   std::vector<int> h_ntasks;
   int max_ntasks_prepared = 0;
   // sorted path, per job (grown on demand)
-  double *G = nullptr, *jpart_s = nullptr;
-  std::vector<cudaArray_t> tex2_arrays;
-  std::vector<cudaTextureObject_t> h_tex2;
-  cudaTextureObject_t* d_tex2 = nullptr;
+  nid::DeviceBuffer<double> G, jpart_s;
+  std::vector<nid::GatherTexture> tex2;  // [n_pairs] packed target textures
+  nid::DeviceBuffer<cudaTextureObject_t> d_tex2;
   // kernel 1 (nid_warp_sample_jobs): fp16 target planes, created and filled on first use per pair
-  std::vector<cudaArray_t> k1_arrays;
-  std::vector<cudaTextureObject_t> h_k1tex;
-  cudaTextureObject_t* d_k1tex = nullptr;
+  std::vector<nid::GatherTexture> k1tex;
+  nid::DeviceBuffer<cudaTextureObject_t> d_k1tex;
   std::vector<char> k1_ready;
-  unsigned short* d_k1pack = nullptr;  // [3N] scratch
-  unsigned* fp1 = nullptr;     // [n_pairs][N]
+  nid::DeviceBuffer<unsigned short> d_k1pack;  // [3N] scratch
+  nid::DeviceBuffer<unsigned> fp1;    // [n_pairs][N]
   std::vector<double> h_Twc0, h_cam;  // host copies per pair (geometry tables are built on the host)
-  unsigned* d_pack = nullptr;  // [setup_batch][N] scratch for the packed textures
+  nid::DeviceBuffer<unsigned> d_pack;  // [setup_batch][N] scratch for the packed textures
   size_t g_stride = 0;
   int opt_path = 0;            // 0 auto, 1 natural-order atomics (v1), 2 sorted
   int opt_keep_hist = 0;
   std::vector<char> pair_set, pair_prepared, pair_sorted;
   // staging
-  double* d_depth = nullptr;   // [N] scratch
-  double* d_img64 = nullptr;   // [N] scratch for the f64 image entry point
-  int* d_flag = nullptr;
-  double* d_pix = nullptr;     // [8N] scratch for nid_warp_sample_f64
-  float* d_pix4 = nullptr;     // [4N] scratch for nid_warp_sample
-  float* d_pix4_jobs = nullptr;  // [max_jobs][4N] output of nid_warp_sample_jobs (allocated on first use)
-  double* d_bsv = nullptr;     // [4N] scratch for nid_get_ref_weights
-  int* d_bsi = nullptr;        // [N]
+  nid::DeviceBuffer<double> d_depth;  // [N] scratch
+  nid::DeviceBuffer<double> d_img64;  // [N] scratch for the f64 image entry point
+  nid::DeviceBuffer<int> d_flag;
+  nid::DeviceBuffer<double> d_pix;    // [8N] scratch for nid_warp_sample_f64
+  nid::DeviceBuffer<float> d_pix4;    // [4N] scratch for nid_warp_sample
+  nid::DeviceBuffer<float> d_pix4_jobs;  // [max_jobs][4N] output of nid_warp_sample_jobs (allocated on first use)
+  nid::DeviceBuffer<double> d_bsv;    // [4N] scratch for nid_get_ref_weights
+  nid::DeviceBuffer<int> d_bsi;       // [N]
   // luts
-  double* lut_w = nullptr;
-  int* lut_k = nullptr;
+  nid::DeviceBuffer<double> lut_w;
+  nid::DeviceBuffer<int> lut_k;
   // per job
-  double* poses = nullptr;
-  int* job_pair = nullptr;
-  double *part = nullptr, *jpart = nullptr, *hist = nullptr;
-  double *ht = nullptr, *hj = nullptr, *err = nullptr, *der = nullptr, *gn = nullptr;
-  double* hard = nullptr;      // [jobs][ncell+1]
+  nid::DeviceBuffer<double> pose_buf;  // [job_cap][16]
+  double* poses = nullptr;  // pose_buf, or the LM staging block of the latency mode
+  nid::DeviceBuffer<int> job_pair;
+  nid::DeviceBuffer<double> part, jpart, hist;
+  nid::DeviceBuffer<double> ht, hj, err, der, gn;
+  nid::DeviceBuffer<double> hard;     // [jobs][ncell+1]
   size_t part_slots = 0;       // capacity in (job,strip) units
   // pinned host mirrors of the staged jobs: a ring of NID_STAGE_RING slots, each guarded by an event recorded after
   // the slot's H2D copies, so that a slot is never rewritten while a copy from it is still pending (the staged
   // API is asynchronous: stage, eval, stage, eval ... without a synchronisation in between)
-  double* h_poses = nullptr;      // current slot: [max_jobs][16]
+  double* h_poses = nullptr;      // current slot: [max_jobs][16] (or the LM staging block)
   int* h_job_pair = nullptr;      // current slot: [max_jobs]
-  double* h_poses_ring = nullptr;
-  int* h_job_pair_ring = nullptr;
-  cudaEvent_t stage_ev[NID_STAGE_RING] = {};
+  nid::PinnedBuffer<double> h_poses_ring;
+  nid::PinnedBuffer<int> h_job_pair_ring;
+  nid::Event stage_ev[NID_STAGE_RING];
   int stage_slot = 0;
   int staged_jobs = 0;            // jobs of the last nid_stage_jobs (nid_eval_staged refuses more)
   // nid_prepare / nid_warp_sample* take their pose through their own scratch (both calls are blocking), so that
   // they never disturb staged jobs
-  double* h_aux_pose = nullptr;   // pinned [16]
-  double* aux_pose = nullptr;     // device [16]
-  double* h_out = nullptr;     // [max_jobs][ncell*8 + 44]
+  nid::PinnedBuffer<double> h_aux_pose;  // [16]
+  nid::DeviceBuffer<double> aux_pose;    // [16]
+  nid::PinnedBuffer<double> h_out;    // [max_jobs][ncell*8 + 44]
   int opt_force_strips = 0;
   // LM driver: per half-batch job lists (pinned mirror + device copy), [2 halves][2 lists][max_jobs]
-  int* h_lm_lists = nullptr;
-  int* d_lm_lists = nullptr;
-  void* h_lm_stage = nullptr;  // latency mode: poses + slot list of a round, pinned / device
-  void* d_lm_stage = nullptr;
-  nid::LatencyGraph* lm_graph = nullptr;  // latency mode: the captured round (nid_sorted.cu)
+  nid::PinnedBuffer<int> h_lm_lists;
+  nid::DeviceBuffer<int> d_lm_lists;
+  nid::PinnedBuffer<char> h_lm_stage;  // latency mode: poses + slot list of a round, pinned / device
+  nid::DeviceBuffer<char> d_lm_stage;
+  std::unique_ptr<nid::LatencyGraph, nid::LatencyGraphDelete> lm_graph;  // latency mode: the captured round
   const void* last_hist_func = nullptr;     // the pixel-kernel instantiations the last launch used (graph node lookup)
   const void* last_jac_func = nullptr;
   int opt_lm_graph = 1;
@@ -204,14 +206,21 @@ struct nid_ctx {
   int opt_asm_wide = 1;  // 1024-thread assembly when there are fewer (cell, job) units than SMs
   int opt_lm_spec = 4;         // latency mode of nid_solve_jobs (few problems): trial poses evaluated per round and problem
   int opt_lm_reuse = 1;        // a cost+Jacobian job at the pose of the accepted trial reuses that trial's histograms and tables
-  cudaEvent_t ev[2] = {nullptr, nullptr};
+  nid::Event ev[2];
   // nid_set_pairs_downsampled into this context: [0] recorded on the source's stream before the kernel, [1] on this
   // context's stream after it (created on first use)
-  cudaEvent_t ds_ev[2] = {nullptr, nullptr};
+  nid::Event ds_ev[2];
   int opt_time_kernels = 0;
-  cudaEvent_t kev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+  nid::Event kev[5];
   double kernel_ms[4] = {0, 0, 0, 0};  // k_hist, k_jac, k_jac_final, k_entropy
   long long kernel_calls[4] = {0, 0, 0, 0};
+
+  // the members release their handles after the streams have drained
+  ~nid_ctx() {
+    cudaSetDevice(device);
+    for (auto& s : streams)
+      if (s) cudaStreamSynchronize(s);
+  }
 };
 
 namespace nid {
@@ -304,7 +313,7 @@ EvalParams make_params(nid_ctx* c, int n_jobs);
 // optional per-kernel stopwatch (option "time_kernels"): events between the launches of one evaluation
 inline void ktime_mark(nid_ctx* c, int i) {
   if (!c->opt_time_kernels) return;
-  if (!c->kev[i]) cudaEventCreate(&c->kev[i]);
+  if (!c->kev[i]) c->kev[i].create(cudaEventDefault, "cudaEventCreate (kernel timer)");
   cudaEventRecord(c->kev[i], c->stream);
 }
 // adds the interval between marks i and i + 1 to the bucket slot[i] (-1: no kernel ran in it)
@@ -345,7 +354,6 @@ int launch_pack(nid_ctx* c, int pair0, int n);
 int launch_pack_k1(nid_ctx* c, int pair, unsigned short* d_out);
 int launch_sorted_tail_gn(nid_ctx* c, const int* d_list, const int* h_list, int first, int n, double delta, double* gn_out);
 int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h_list, size_t h2d_bytes, double delta, double* gn_out);
-void destroy_latency_graph(nid_ctx* c);
 int launch_href(nid_ctx* c, int pair0, int n);
 
 // kernel launchers (nid_kernels.cu)

@@ -714,7 +714,7 @@ int launch_warp_sample(nid_ctx* c, int pair, const double* d_pose16, int f64) {
   EvalParams p = make_params(c, 1);
   int g = grid_for(c->N, 256, c->sm_count * 8);
   if (f64) k_warp_sample<true><<<g, 256, 0, c->stream>>>(p, pair, d_pose16, nullptr, c->d_pix);
-  else k_warp_sample<false><<<g, 256, 0, c->stream>>>(p, pair, d_pose16, (float4*)c->d_pix4, nullptr);
+  else k_warp_sample<false><<<g, 256, 0, c->stream>>>(p, pair, d_pose16, (float4*)c->d_pix4.get(), nullptr);
   NID_LAUNCH_CHECK(c, "k_warp_sample");
   return NID_OK;
 }

@@ -1864,7 +1864,7 @@ static void fill_geo(const nid_ctx* c, GeoTable<NG>& gt, int first, int n, bool 
     double* g = gt.g[i];
     gt.job[i] = job; gt.pair[i] = pair;
     gt.nsl[i] = c->h_nslices[pair];
-    gt.tex[i] = c->h_tex2.empty() ? 0ull : (unsigned long long)c->h_tex2[pair];
+    gt.tex[i] = c->tex2.empty() ? 0ull : (unsigned long long)c->tex2[pair].tex;
     for (int col = 0; col < 4; col++)
       for (int r = 0; r < 3; r++) {
         double m;
@@ -2072,8 +2072,8 @@ int launch_sorted_tail_gn(nid_ctx* c, const int* d_list, const int* h_list, int 
 // The graph is rebuilt whenever anything its nodes captured by value has changed (buffers, layout sizes, options):
 // the signature below is compared at every round.
 struct LatencyGraph {
-  cudaGraph_t graph = nullptr;
-  cudaGraphExec_t exec = nullptr;
+  Graph graph;
+  GraphExec exec;  // (declared after its graph: destroyed first)
   cudaGraphNode_t hist_node = nullptr, jac_node = nullptr;
   cudaKernelNodeParams hist_np{}, jac_np{};
   EvalParams hist_q, jac_q;  // first argument of the two pixel kernels as captured
@@ -2088,19 +2088,12 @@ struct LatencyGraph {
   cudaStream_t stream = nullptr;
 };
 
-void destroy_latency_graph(nid_ctx* c) {
-  LatencyGraph* g = c->lm_graph;
-  if (!g) return;
-  if (g->exec) cudaGraphExecDestroy(g->exec);
-  if (g->graph) cudaGraphDestroy(g->graph);
-  delete g;
-  c->lm_graph = nullptr;
-}
+void LatencyGraphDelete::operator()(LatencyGraph* g) const { delete g; }
 
 static int capture_latency_graph(nid_ctx* c, LatencyGraph* g, int nslots, const int* d_list, const int* h_list, size_t h2d_bytes,
                                  double delta, double* gn_out) {
-  if (g->exec) { cudaGraphExecDestroy(g->exec); g->exec = nullptr; }
-  if (g->graph) { cudaGraphDestroy(g->graph); g->graph = nullptr; }
+  g->exec.reset();
+  g->graph.reset();
   cudaError_t e = cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal);
   if (e != cudaSuccess) return check_cuda(e, "cudaStreamBeginCapture");
   int r = NID_OK;
@@ -2108,7 +2101,9 @@ static int capture_latency_graph(nid_ctx* c, LatencyGraph* g, int nslots, const 
   if (e != cudaSuccess) r = check_cuda(e, "H2D poses + list (capture)");
   if (r == NID_OK) r = launch_pass1(c, JobSet{d_list, h_list, 0, nslots, nslots}, Pass2::some);
   if (r == NID_OK) r = launch_sorted_tail_gn(c, d_list, h_list, 0, nslots, delta, gn_out);
-  e = cudaStreamEndCapture(c->stream, &g->graph);
+  cudaGraph_t graph = nullptr;
+  e = cudaStreamEndCapture(c->stream, &graph);
+  g->graph.reset(graph);
   if (r != NID_OK) return r;
   if (e != cudaSuccess) return check_cuda(e, "cudaStreamEndCapture");
   size_t nn = 0;
@@ -2132,8 +2127,10 @@ static int capture_latency_graph(nid_ctx* c, LatencyGraph* g, int nslots, const 
     }
   }
   if (!g->hist_node || !g->jac_node) { set_error("latency graph: pixel-kernel nodes not found"); return NID_ERR_STATE; }
-  e = cudaGraphInstantiate(&g->exec, g->graph, 0);
+  cudaGraphExec_t exec = nullptr;
+  e = cudaGraphInstantiate(&exec, g->graph, 0);
   if (e != cudaSuccess) return check_cuda(e, "cudaGraphInstantiate");
+  g->exec.reset(exec);
   return NID_OK;
 }
 
@@ -2148,15 +2145,15 @@ int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h
     if (r != NID_OK) return r;
     return launch_sorted_tail_gn(c, d_list, h_list, 0, nslots, delta, gn_out);
   }
-  if (!c->lm_graph) c->lm_graph = new LatencyGraph();
-  LatencyGraph* g = c->lm_graph;
+  if (!c->lm_graph) c->lm_graph.reset(new LatencyGraph());
+  LatencyGraph* g = c->lm_graph.get();
   const EvalParams sig = make_params(c, nslots);
   const bool same = g->exec && memcmp(&sig, &g->sig, sizeof(sig)) == 0 && g->nslots == nslots && g->ns == ns && g->task_px == c->task_px &&
                     g->h2d_bytes == h2d_bytes && g->delta == delta && g->d_list == d_list && g->gn_out == gn_out &&
                     g->h_src == (const void*)c->h_poses && g->stream == c->stream;
   if (!same) {
     const int r = capture_latency_graph(c, g, nslots, d_list, h_list, h2d_bytes, delta, gn_out);
-    if (r != NID_OK) { destroy_latency_graph(c); return r; }
+    if (r != NID_OK) { c->lm_graph.reset(); return r; }
     g->sig = sig; g->nslots = nslots; g->ns = ns; g->task_px = c->task_px; g->h2d_bytes = h2d_bytes; g->delta = delta;
     g->d_list = d_list; g->gn_out = gn_out; g->h_src = c->h_poses; g->stream = c->stream;
     // (the graph just captured holds this round's geometry already)

@@ -60,3 +60,26 @@ def test_every_run_time_option_is_documented_in_the_header():
     hdr = open(os.path.join(ROOT, "include", "nid_b200.h")).read()
     missing = [k for k in sorted(keys) if f'"{k}"' not in hdr]
     assert not missing, missing
+
+
+def test_cuda_resources_are_acquired_and_released_only_by_their_owner_types():
+    """A context's device and pinned buffers, streams, events, arrays, textures and graphs are held by the owner types of
+    csrc/nid_handles.h, which release them in their destructors: no source file allocates or releases one by hand, so a
+    context frees everything it holds on every way out, a nid_create that fails half way included."""
+    import glob
+    import re
+    ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    csrc = os.path.join(ROOT, "nid-pose-estimation_b200", "csrc")
+    release = {"cudaFree", "cudaFreeHost", "cudaFreeArray", "cudaEventDestroy", "cudaStreamDestroy",
+               "cudaDestroyTextureObject", "cudaGraphDestroy", "cudaGraphExecDestroy"}
+    acquire = {"cudaMalloc", "cudaMallocHost", "cudaMallocArray", "cudaCreateTextureObject", "cudaStreamCreate",
+               "cudaStreamCreateWithFlags", "cudaEventCreate", "cudaEventCreateWithFlags"}
+    found = {}
+    for path in sorted(glob.glob(os.path.join(csrc, "*.cu*")) + glob.glob(os.path.join(csrc, "*.h"))):
+        code = re.sub(r'"(?:\\.|[^"\\])*"', '""', open(path).read())  # (error texts name the calls they report)
+        code = re.sub(r"//[^\n]*|/\*.*?\*/", "", code, flags=re.S)
+        names = set(re.findall(r"\bcuda\w+", code)) & (release | acquire)
+        if names:
+            found[os.path.basename(path)] = names
+    assert set(found) == {"nid_handles.h"}, found
+    assert release <= found["nid_handles.h"]
