@@ -64,7 +64,7 @@ EvalParams make_params(nid_ctx* c, int n_jobs) {
   p.im0 = c->im0; p.im1 = c->im1; p.inb0 = c->inb0;
   p.n_c = c->n_c; p.href = c->href; p.cam = c->cam;
   p.lut_w = c->lut_w; p.lut_k = c->lut_k;
-  p.poses = c->poses; p.job_pair = c->job_pair;
+  p.job_pair = c->job_pair;
   const bool sorted = use_sorted(c);
   p.part = c->part; p.jpart = sorted ? c->jpart_s : c->jpart; p.hist = c->opt_keep_hist ? c->hist.get() : nullptr;
   p.ht = c->ht; p.hj = c->hj; p.err = c->err; p.der = c->der; p.gn = c->gn;
@@ -76,6 +76,11 @@ EvalParams make_params(nid_ctx* c, int n_jobs) {
   p.cls_task_start = c->cls_task_start; p.span_start = c->span_start; p.wv = c->wv;
   p.max_tasks = c->max_tasks; p.g_stride = (int)c->g_stride;
   p.G = c->G; p.fp1 = c->fp1; p.tex2 = c->d_tex2; p.k1tex = c->d_k1tex;
+  return p;
+}
+EvalParams make_params(nid_ctx* c, const JobSet& js) {
+  EvalParams p = make_params(c, js.slots);
+  p.job0 = js.first; p.job_list = js.d_list; p.poses = js.d_poses;
   return p;
 }
 
@@ -159,8 +164,26 @@ static int arena_take(nid_ctx* c, size_t bytes, void** out) {
   return NID_OK;
 }
 
-// Staging of n_jobs (pair, pose) jobs: the next slot of the pinned ring is taken (waiting, if need be, for the copies
-// that last read it), filled, and copied to the device asynchronously on the context stream.
+// Takes the next slot of the pinned staging ring, waiting, if need be, for the copies that last read it: its poses
+// [job_cap][16] and pairs [job_cap].
+static int take_stage_slot(nid_ctx* c, double** h_poses, int** h_pair) {
+  const int slot = (c->stage_slot + 1) % NID_STAGE_RING;
+  CU(cudaEventSynchronize(c->stage_ev[slot]), "wait for the staging slot");  // (returns at once for an unrecorded event)
+  c->stage_slot = slot;
+  *h_poses = c->h_poses_ring + (size_t)slot * 16 * c->job_cap;
+  *h_pair = c->h_job_pair_ring + (size_t)slot * c->job_cap;
+  return NID_OK;
+}
+
+// the staged jobs 0 .. n - 1: the slot taken last, pose_buf, the context stream
+static JobSet staged_set(const nid_ctx* c, int n) {
+  const size_t slot = c->stage_slot;
+  return JobSet{nullptr, nullptr, 0, n, n, c->stream, c->pose_buf, c->h_poses_ring + slot * 16 * c->job_cap,
+                c->h_job_pair_ring + slot * c->job_cap};
+}
+
+// Staging of n_jobs (pair, pose) jobs: the next ring slot is taken, filled, and copied to the device asynchronously on
+// the context stream.
 // mode 0: pairs must be prepared (evaluation); 1: pairs must be set (hard-binned NID, kernel 1).
 static int stage_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const double* poses, int mode = 0) {
   if (n_jobs < 1 || n_jobs > c->max_jobs) { set_error("n_jobs out of range"); return NID_ERR_ARG; }
@@ -177,16 +200,14 @@ static int stage_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const double*
       return NID_ERR_STATE;
     }
   }
-  const int slot = (c->stage_slot + 1) % NID_STAGE_RING;
-  CU(cudaEventSynchronize(c->stage_ev[slot]), "wait for the staging slot");  // (returns at once for an unrecorded event)
-  c->stage_slot = slot;
-  c->h_poses = c->h_poses_ring + (size_t)slot * 16 * c->job_cap;
-  c->h_job_pair = c->h_job_pair_ring + (size_t)slot * c->job_cap;
-  for (int j = 0; j < n_jobs; j++) c->h_job_pair[j] = job_pair ? job_pair[j] : 0;
-  memcpy(c->h_poses, poses, sizeof(double) * 16 * n_jobs);
-  CU(cudaMemcpyAsync(c->poses, c->h_poses, sizeof(double) * 16 * n_jobs, cudaMemcpyHostToDevice, c->stream), "H2D poses");
-  CU(cudaMemcpyAsync(c->job_pair, c->h_job_pair, sizeof(int) * n_jobs, cudaMemcpyHostToDevice, c->stream), "H2D job_pair");
-  CU(cudaEventRecord(c->stage_ev[slot], c->stream), "record staging event");
+  double* h_poses;
+  int* h_pair;
+  OKR(take_stage_slot(c, &h_poses, &h_pair));
+  for (int j = 0; j < n_jobs; j++) h_pair[j] = job_pair ? job_pair[j] : 0;
+  memcpy(h_poses, poses, sizeof(double) * 16 * n_jobs);
+  CU(cudaMemcpyAsync(c->pose_buf, h_poses, sizeof(double) * 16 * n_jobs, cudaMemcpyHostToDevice, c->stream), "H2D poses");
+  CU(cudaMemcpyAsync(c->job_pair, h_pair, sizeof(int) * n_jobs, cudaMemcpyHostToDevice, c->stream), "H2D job_pair");
+  CU(cudaEventRecord(c->stage_ev[c->stage_slot], c->stream), "record staging event");
   c->staged_jobs = n_jobs;
   return NID_OK;
 }
@@ -240,8 +261,7 @@ int nid_create(nid_ctx** out, int device, int rows, int cols, int cell, int bins
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device), "cudaGetDeviceProperties");
   c->sm_count = prop.multiProcessorCount;
-  OKR(c->streams[0].create("cudaStreamCreate"));
-  c->stream = c->streams[0];
+  OKR(c->stream.create("cudaStreamCreate"));
   const size_t N = c->N, P = n_pairs, J = c->job_cap, NC = c->ncell;
   const size_t hs = (size_t)bins * bins + bins;
   OKR(c->pwx.alloc(P * N, "pwx")); OKR(c->pwy.alloc(P * N, "pwy")); OKR(c->pwz.alloc(P * N, "pwz"));
@@ -324,9 +344,8 @@ int nid_create(nid_ctx** out, int device, int rows, int cols, int cell, int bins
   CU(cudaMemset(c->d_flag, 0, sizeof(int) * 2), "memset flag");
   OKR(c->lut_w.alloc(256 * 4, "lut_w")); OKR(c->lut_k.alloc(256, "lut_k"));
   OKR(c->pose_buf.alloc(J * 16, "poses")); OKR(c->job_pair.alloc(J, "job_pair"));
-  c->poses = c->pose_buf;
   CU(cudaMemset(c->job_pair, 0, sizeof(int) * J), "memset job_pair");
-  CU(cudaMemset(c->poses, 0, sizeof(double) * 16 * J), "memset poses");
+  CU(cudaMemset(c->pose_buf, 0, sizeof(double) * 16 * J), "memset poses");
   OKR(c->aux_pose.alloc(16, "aux_pose"));
   (void)hs;
   OKR(c->ht.alloc(J * NC, "ht")); OKR(c->hj.alloc(J * NC, "hj")); OKR(c->err.alloc(J * NC, "err"));
@@ -336,8 +355,6 @@ int nid_create(nid_ctx** out, int device, int rows, int cols, int cell, int bins
   OKR(c->h_job_pair_ring.alloc(J * NID_STAGE_RING, "pinned job_pair"));
   memset(c->h_poses_ring, 0, sizeof(double) * 16 * J * NID_STAGE_RING);
   memset(c->h_job_pair_ring, 0, sizeof(int) * J * NID_STAGE_RING);
-  c->h_poses = c->h_poses_ring;
-  c->h_job_pair = c->h_job_pair_ring;
   for (auto& e : c->stage_ev) OKR(e.create(cudaEventDisableTiming, "cudaEventCreate (staging)"));
   OKR(c->h_aux_pose.alloc(16, "pinned aux pose"));
   OKR(c->h_out.alloc(J * (NC * 8 + 44), "pinned out"));
@@ -700,7 +717,7 @@ int nid_stage_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const double* po
 // cost (+ Jacobian) of the staged jobs 0 .. n - 1
 static int eval_range(nid_ctx* c, int n, int want_jac) {
   OKR(ensure_job_buffers(c));
-  const JobSet js{nullptr, nullptr, 0, n, n};
+  const JobSet js = staged_set(c, n);
   OKR(launch_pass1(c, js, want_jac ? Pass2::all : Pass2::none));
   if (!want_jac) {
     const int slot[2] = {0, 3};
@@ -745,7 +762,7 @@ int nid_eval_gn(nid_ctx* c, int pair, const double T_cw1[16], double delta, doub
   CU(cudaSetDevice(c->device), "cudaSetDevice");
   OKR(stage_jobs(c, 1, &pair, T_cw1));
   OKR(eval_range(c, 1, 1));
-  OKR(launch_gn(c, JobSet{nullptr, nullptr, 0, 1, 1}, delta, 1));
+  OKR(launch_gn(c, staged_set(c, 1), delta, 1));
   double* h = c->h_out;
   const size_t nc = c->ncell;
   CU(cudaMemcpyAsync(h, c->gn, sizeof(double) * 44, cudaMemcpyDeviceToHost, c->stream), "D2H gn");
@@ -887,21 +904,20 @@ static int solve_speculative(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs,
   const size_t stage_bytes = sizeof(double) * 16 * (size_t)c->job_cap + sizeof(int) * (size_t)c->job_cap;
   if (!c->d_lm_stage) {
     OKR(c->h_lm_stage.alloc(stage_bytes, "pinned LM staging"));
+    OKR(c->h_lm_pair.alloc(c->job_cap, "pinned LM pairs"));
     OKR(c->d_lm_stage.alloc(stage_bytes, "LM staging"));
   }
-  struct Swap {  // restores the context's pose buffers on every way out
-    nid_ctx* c; double* poses; double* h_poses;
-    ~Swap() { c->poses = poses; c->h_poses = h_poses; }
-  } swap{c, c->poses, c->h_poses};
-  c->poses = reinterpret_cast<double*>(c->d_lm_stage.get());
-  c->h_poses = reinterpret_cast<double*>(c->h_lm_stage.get());
-  int* const list = reinterpret_cast<int*>(c->h_poses + 16 * (size_t)nslots);
-  int* const d_list = reinterpret_cast<int*>(c->poses + 16 * (size_t)nslots);
+  double* const h_poses = reinterpret_cast<double*>(c->h_lm_stage.get());
+  double* const d_poses = reinterpret_cast<double*>(c->d_lm_stage.get());
+  int* const list = reinterpret_cast<int*>(h_poses + 16 * (size_t)nslots);
+  int* const d_list = reinterpret_cast<int*>(d_poses + 16 * (size_t)nslots);
+  int* const h_pair = c->h_lm_pair;
+  const JobSet js{d_list, list, 0, nslots, nslots, c->stream, d_poses, h_poses, h_pair};
   auto slot_of = [&](int j, int k, int g) { return st[j].slot0 * K + k * st[j].nj + g; };
   for (int j = 0; j < n; j++)
     for (int k = 0; k < K; k++)
-      for (int g = 0; g < st[j].nj; g++) c->h_job_pair[slot_of(j, k, g)] = st[j].pairs[g];
-  CU(cudaMemcpyAsync(c->job_pair, c->h_job_pair, sizeof(int) * nslots, cudaMemcpyHostToDevice, c->stream), "H2D job_pair");
+      for (int g = 0; g < st[j].nj; g++) h_pair[slot_of(j, k, g)] = st[j].pairs[g];
+  CU(cudaMemcpyAsync(c->job_pair, h_pair, sizeof(int) * nslots, cudaMemcpyHostToDevice, c->stream), "H2D job_pair");
   CU(cudaStreamSynchronize(c->stream), "sync before LM");
   auto same_pose = [](const nidhost::Pose7& a, const nidhost::Pose7& b) {
     return memcmp(a.t, b.t, sizeof(a.t)) == 0 && memcmp(a.q, b.q, sizeof(a.q)) == 0;
@@ -940,7 +956,7 @@ static int solve_speculative(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs,
         Cand& q = cache[(size_t)j * K + k];
         q.pose = sim.est;
         q.valid = true;
-        for (int g = 0; g < s.nj; g++) stage_pose(s, sim.est, g, c->h_poses + 16 * (size_t)slot_of(j, k, g));
+        for (int g = 0; g < s.nj; g++) stage_pose(s, sim.est, g, h_poses + 16 * (size_t)slot_of(j, k, g));
         nround++;
         if (sim.phase != 1 || sim.qmax + 1 >= 10) break;  // only trial poses have successors; maxTrials = 10
         // the trial after a rejection of this one (lm_absorb's else branch, then lm_start_trial)
@@ -959,14 +975,14 @@ static int solve_speculative(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs,
       for (int k = 0; k < K; k++) {
         if (cache[(size_t)j * K + k].valid) continue;
         for (int g = 0; g < st[j].nj; g++) {
-          double* m = c->h_poses + 16 * (size_t)slot_of(j, k, g);
-          if (k > 0) memcpy(m, c->h_poses + 16 * (size_t)slot_of(j, 0, g), sizeof(double) * 16);
+          double* m = h_poses + 16 * (size_t)slot_of(j, k, g);
+          if (k > 0) memcpy(m, h_poses + 16 * (size_t)slot_of(j, 0, g), sizeof(double) * 16);
           else stage_pose(st[j], st[j].est, g, m);
         }
       }
     }
     for (int i = 0; i < nslots; i++) list[i] = i;
-    OKR(launch_latency_round(c, nslots, d_list, list, sizeof(double) * 16 * nslots + sizeof(int) * nslots, delta, c->h_out));
+    OKR(launch_latency_round(c, js, sizeof(double) * 16 * nslots + sizeof(int) * nslots, delta, c->h_out));
     const double t2 = now();
     CU(cudaStreamSynchronize(c->stream), "sync lm");
     const double t3 = now();
@@ -1002,7 +1018,7 @@ static int solve_lockstep(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs, in
   // (the natural-order kernels index their partial buffers by (slot, cell, strip): two halves in flight would need the
   // same strip count S)
   const int nh = (n >= 8 && sorted) ? 2 : 1;
-  if (nh == 2 && !c->streams[1]) OKR(c->streams[1].create("cudaStreamCreate (LM)"));
+  if (nh == 2 && !c->lm_stream) OKR(c->lm_stream.create("cudaStreamCreate (LM)"));
   if (!c->d_lm_lists) {
     OKR(c->h_lm_lists.alloc(2 * (size_t)c->job_cap, "pinned LM lists"));
     OKR(c->d_lm_lists.alloc(2 * (size_t)c->job_cap, "LM lists"));
@@ -1015,12 +1031,14 @@ static int solve_lockstep(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs, in
   };
   Half H[2];
   H[0] = half(0, nh == 2 ? n / 2 : n, c->stream);
-  H[1] = half(n / 2, n, c->streams[1]);
-  cudaStream_t const main_stream = c->stream;
+  H[1] = half(n / 2, n, c->lm_stream);
+  double* h_poses;
+  int* h_pair;
+  OKR(take_stage_slot(c, &h_poses, &h_pair));
   for (int j = 0; j < n; j++)
-    for (int g = 0; g < st[j].nj; g++) c->h_job_pair[st[j].slot0 + g] = st[j].pairs[g];
-  CU(cudaMemcpyAsync(c->job_pair, c->h_job_pair, sizeof(int) * n_jobs, cudaMemcpyHostToDevice, main_stream), "H2D job_pair");
-  CU(cudaStreamSynchronize(main_stream), "sync job_pair");
+    for (int g = 0; g < st[j].nj; g++) h_pair[st[j].slot0 + g] = st[j].pairs[g];
+  CU(cudaMemcpyAsync(c->job_pair, h_pair, sizeof(int) * n_jobs, cudaMemcpyHostToDevice, c->stream), "H2D job_pair");
+  CU(cudaStreamSynchronize(c->stream), "sync job_pair");
   int rc = NID_OK;
   auto issue = [&](Half& h) -> int {
     int* l1 = c->h_lm_lists + 2 * (size_t)h.lo;
@@ -1030,7 +1048,7 @@ static int solve_lockstep(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs, in
       LM& s = st[j];
       if (s.phase == 2) continue;
       h.na++;
-      for (int g = 0; g < s.nj; g++) stage_pose(s, s.est, g, c->h_poses + 16 * (size_t)(s.slot0 + g));
+      for (int g = 0; g < s.nj; g++) stage_pose(s, s.est, g, h_poses + 16 * (size_t)(s.slot0 + g));
       const bool full = s.phase == 0;
       const bool pass1 = !full || !(reuse && s.slot_holds_est);
       for (int g = 0; g < s.nj; g++) {
@@ -1041,20 +1059,18 @@ static int solve_lockstep(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs, in
     }
     if (h.na == 0) return NID_OK;
     const int cnt = h.hi - h.lo;
-    CU(cudaMemcpyAsync(c->poses + 16 * (size_t)h.lo, c->h_poses + 16 * (size_t)h.lo, sizeof(double) * 16 * cnt, cudaMemcpyHostToDevice, h.stream),
+    CU(cudaMemcpyAsync(c->pose_buf + 16 * (size_t)h.lo, h_poses + 16 * (size_t)h.lo, sizeof(double) * 16 * cnt, cudaMemcpyHostToDevice, h.stream),
        "H2D poses");
     int* d1 = c->d_lm_lists + 2 * (size_t)h.lo;
     int* d2 = d1 + cnt;
     CU(cudaMemcpyAsync(d1, l1, sizeof(int) * 2 * cnt, cudaMemcpyHostToDevice, h.stream), "H2D job lists");
-    c->stream = h.stream;  // the launchers issue on the context's current stream
-    const JobSet js1{d1, l1, 0, h.n1, n_jobs}, js2{d2, l2, 0, h.n2, n_jobs};  // (slots: the solve's, the same in every round)
-    int r = NID_OK;
-    if (h.n1 > 0) r = launch_pass1(c, js1, Pass2::some);
-    if (r == NID_OK && h.n2 > 0) r = launch_pass2(c, js2);
-    if (r == NID_OK && h.n2 > 0) r = launch_gn(c, js2, delta, 1);
-    if (r == NID_OK && h.n1 > 0) r = launch_gn(c, js1, delta, 0);  // chi2 of the trial poses (and, harmlessly, again of full jobs)
-    c->stream = main_stream;
-    if (r != NID_OK) return r;
+    // (slots: the solve's, the same in every round)
+    const JobSet js1{d1, l1, 0, h.n1, n_jobs, h.stream, c->pose_buf, h_poses, h_pair};
+    const JobSet js2{d2, l2, 0, h.n2, n_jobs, h.stream, c->pose_buf, h_poses, h_pair};
+    if (h.n1 > 0) OKR(launch_pass1(c, js1, Pass2::some));
+    if (h.n2 > 0) OKR(launch_pass2(c, js2));
+    if (h.n2 > 0) OKR(launch_gn(c, js2, delta, 1));
+    if (h.n1 > 0) OKR(launch_gn(c, js1, delta, 0));  // chi2 of the trial poses (and, harmlessly, again of full jobs)
     CU(cudaMemcpyAsync(c->h_out + 44 * (size_t)h.lo, c->gn + 44 * (size_t)h.lo, sizeof(double) * 44 * cnt, cudaMemcpyDeviceToHost, h.stream),
        "D2H gn");
     return NID_OK;
@@ -1075,9 +1091,8 @@ static int solve_lockstep(nid_ctx* c, std::vector<LM>& st, int n, int n_jobs, in
       rc = issue(h);
     }
   }
-  c->stream = main_stream;
-  if (nh == 2) cudaStreamSynchronize(c->streams[1]);
-  cudaStreamSynchronize(main_stream);
+  if (nh == 2) cudaStreamSynchronize(c->lm_stream);
+  cudaStreamSynchronize(c->stream);
   return rc;
 }
 
@@ -1205,7 +1220,7 @@ int nid_hard_eval_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const double
   CU(cudaSetDevice(c->device), "cudaSetDevice");
   OKR(stage_jobs(c, n_jobs, job_pair, poses, 1));
   c->staged_jobs = 0;  // (not evaluation jobs: the pairs need not be prepared)
-  OKR(launch_hard(c, n_jobs));
+  OKR(launch_hard(c, staged_set(c, n_jobs)));
   const size_t w = c->ncell + 1;
   CU(cudaMemcpyAsync(c->h_out, c->hard, sizeof(double) * w * n_jobs, cudaMemcpyDeviceToHost, c->stream), "D2H hard");
   CU(cudaStreamSynchronize(c->stream), "sync hard");
@@ -1262,12 +1277,13 @@ int nid_warp_sample_jobs(nid_ctx* c, int n_jobs, const int* job_pair, const doub
   c->staged_jobs = 0;  // (not evaluation jobs: the pairs need not be prepared)
   // pairs uploaded as raw 16-bit depth are read as such (2 B/px); a mixed batch falls back to the fp64 planes, which
   // every pair has
+  const JobSet js = staged_set(c, n_jobs);
   bool u16 = true;
   for (int j = 0; j < n_jobs; j++) {
-    u16 = u16 && c->pair_u16[c->h_job_pair[j]];
-    OKR(ensure_k1_texture(c, c->h_job_pair[j]));
+    u16 = u16 && c->pair_u16[js.h_pair[j]];
+    OKR(ensure_k1_texture(c, js.h_pair[j]));
   }
-  OKR(launch_warp_sample_jobs(c, n_jobs, (float4*)c->d_pix4_jobs.get(), u16));
+  OKR(launch_warp_sample_jobs(c, js, (float4*)c->d_pix4_jobs.get(), u16));
   if (out) CU(cudaMemcpyAsync(out, c->d_pix4_jobs, sizeof(float) * 4 * c->N * (size_t)n_jobs, cudaMemcpyDefault, c->stream), "D2H pix4 jobs");
   CU(cudaStreamSynchronize(c->stream), "sync warp_sample_jobs");
   return NID_OK;

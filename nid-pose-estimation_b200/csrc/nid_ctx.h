@@ -88,8 +88,8 @@ namespace nid {
 struct LatencyGraph;
 struct LatencyGraphDelete { void operator()(LatencyGraph* g) const; };  // (nid_sorted.cu)
 }  // namespace nid
-// A context owns every handle it holds (nid_handles.h); `stream`, `poses`, `h_poses` and `h_job_pair` are views that are
-// pointed elsewhere at run time, their storage is owned by separate members.
+// A context owns every handle it holds (nid_handles.h). The evaluation launchers take the stream and the job table they
+// work on from their JobSet argument, so nothing here is repointed while a call runs.
 struct nid_ctx {
   int device = 0;
   int rows = 0, cols = 0, cell = 0, bins = 0, degree = 3;
@@ -97,9 +97,8 @@ struct nid_ctx {
   int n_pairs = 0, max_jobs = 0;
   int job_cap = 0;             // job slots actually allocated: max(max_jobs, NID_MIN_JOB_SLOTS) (speculative LM trials need a few)
   int sm_count = 148;
-  // [0] the context stream, [1] the second stream of the ping-pong LM driver (nid_solve_jobs), created on first use
-  nid::Stream streams[2];
-  cudaStream_t stream = nullptr;  // the stream the launchers issue on: streams[0], or the stream of a lock-step LM half
+  nid::Stream stream;     // the context stream
+  nid::Stream lm_stream;  // the second half of the lock-step LM driver (nid_solve_jobs), created on first use
   nid::DeviceBuffer<int> chunk_cnt;    // [setup_batch][ncell][chunks of 256 px][NID_NCLS] scratch of the regrouping scatter
   // batched pair set-up (nid_set_pairs_u16 / nid_prepare_pairs): up to setup_batch pairs per launch
   int setup_batch = 1;
@@ -170,8 +169,7 @@ struct nid_ctx {
   nid::DeviceBuffer<double> lut_w;
   nid::DeviceBuffer<int> lut_k;
   // per job
-  nid::DeviceBuffer<double> pose_buf;  // [job_cap][16]
-  double* poses = nullptr;  // pose_buf, or the LM staging block of the latency mode
+  nid::DeviceBuffer<double> pose_buf;  // [job_cap][16] the staged poses
   nid::DeviceBuffer<int> job_pair;
   nid::DeviceBuffer<double> part, jpart, hist;
   nid::DeviceBuffer<double> ht, hj, err, der, gn;
@@ -179,13 +177,12 @@ struct nid_ctx {
   size_t part_slots = 0;       // capacity in (job,strip) units
   // pinned host mirrors of the staged jobs: a ring of NID_STAGE_RING slots, each guarded by an event recorded after
   // the slot's H2D copies, so that a slot is never rewritten while a copy from it is still pending (the staged
-  // API is asynchronous: stage, eval, stage, eval ... without a synchronisation in between)
-  double* h_poses = nullptr;      // current slot: [max_jobs][16] (or the LM staging block)
-  int* h_job_pair = nullptr;      // current slot: [max_jobs]
-  nid::PinnedBuffer<double> h_poses_ring;
-  nid::PinnedBuffer<int> h_job_pair_ring;
+  // API is asynchronous: stage, eval, stage, eval ... without a synchronisation in between). The lock-step LM driver
+  // takes its pinned job table from the ring the same way.
+  nid::PinnedBuffer<double> h_poses_ring;  // [NID_STAGE_RING][job_cap][16]
+  nid::PinnedBuffer<int> h_job_pair_ring;  // [NID_STAGE_RING][job_cap]
   nid::Event stage_ev[NID_STAGE_RING];
-  int stage_slot = 0;
+  int stage_slot = 0;             // the slot taken last: the host mirror of the staged jobs
   int staged_jobs = 0;            // jobs of the last nid_stage_jobs (nid_eval_staged refuses more)
   // nid_prepare / nid_warp_sample* take their pose through their own scratch (both calls are blocking), so that
   // they never disturb staged jobs
@@ -197,6 +194,7 @@ struct nid_ctx {
   nid::PinnedBuffer<int> h_lm_lists;
   nid::DeviceBuffer<int> d_lm_lists;
   nid::PinnedBuffer<char> h_lm_stage;  // latency mode: poses + slot list of a round, pinned / device
+  nid::PinnedBuffer<int> h_lm_pair;    // latency mode: the slot -> pair mirror [job_cap]
   nid::DeviceBuffer<char> d_lm_stage;
   std::unique_ptr<nid::LatencyGraph, nid::LatencyGraphDelete> lm_graph;  // latency mode: the captured round
   const void* last_hist_func = nullptr;     // the pixel-kernel instantiations the last launch used (graph node lookup)
@@ -218,7 +216,7 @@ struct nid_ctx {
   // the members release their handles after the streams have drained
   ~nid_ctx() {
     cudaSetDevice(device);
-    for (auto& s : streams)
+    for (cudaStream_t s : {stream.get(), lm_stream.get()})
       if (s) cudaStreamSynchronize(s);
   }
 };
@@ -308,13 +306,13 @@ __device__ __forceinline__ void gn_block(const EvalParams& p, int job, int want_
 #endif
 void set_error(const std::string& s);
 int check_cuda(cudaError_t e, const char* what);
-EvalParams make_params(nid_ctx* c, int n_jobs);
+EvalParams make_params(nid_ctx* c, int n_jobs);  // (set-up launchers: no pose table)
 
 // optional per-kernel stopwatch (option "time_kernels"): events between the launches of one evaluation
-inline void ktime_mark(nid_ctx* c, int i) {
+inline void ktime_mark(nid_ctx* c, cudaStream_t stream, int i) {
   if (!c->opt_time_kernels) return;
   if (!c->kev[i]) c->kev[i].create(cudaEventDefault, "cudaEventCreate (kernel timer)");
-  cudaEventRecord(c->kev[i], c->stream);
+  cudaEventRecord(c->kev[i], stream);
 }
 // adds the interval between marks i and i + 1 to the bucket slot[i] (-1: no kernel ran in it)
 inline void ktime_collect(nid_ctx* c, int n, const int* slot) {
@@ -334,8 +332,16 @@ int ensure_job_buffers(nid_ctx* c);
 // The evaluation, on either kernel family (use_sorted picks it), of a set of job slots: d_list[first .. first + n)
 // (h_list: the host copy of d_list), or the slots first .. first + n - 1 when d_list is null. `slots` is the number of
 // slots the set addresses (first + n for a range, the solve's slot count in the LM); pass 1 and pass 2 of the same jobs
-// must be given the same value (see strips_for).
-struct JobSet { const int* d_list; const int* h_list; int first, n; int slots; };
+// must be given the same value (see strips_for). The launches go on `stream`. Slot s is evaluated at the pose
+// d_poses[s] for the pair c->job_pair[s]; h_poses and h_pair are their host mirrors, which the geometry tables are
+// built from.
+struct JobSet {
+  const int* d_list; const int* h_list; int first, n; int slots;
+  cudaStream_t stream;
+  double* d_poses;  // [slots][16] (the latency round copies its staging block here)
+  const double* h_poses; const int* h_pair;
+};
+EvalParams make_params(nid_ctx* c, const JobSet& js);
 // Will pass 2 run on none, some or all of the jobs of a pass 1? Sorted: unless none, the assembly also writes the scaled
 // log tables pass 2 reads. Natural: with all, k_jac writes the cost and pass 1 skips k_entropy.
 enum class Pass2 { none, some, all };
@@ -352,8 +358,8 @@ int launch_count_classes(nid_ctx* c, int pair);
 int launch_layout_and_scatter(nid_ctx* c, int pair0, int n);
 int launch_pack(nid_ctx* c, int pair0, int n);
 int launch_pack_k1(nid_ctx* c, int pair, unsigned short* d_out);
-int launch_sorted_tail_gn(nid_ctx* c, const int* d_list, const int* h_list, int first, int n, double delta, double* gn_out);
-int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h_list, size_t h2d_bytes, double delta, double* gn_out);
+int launch_sorted_tail_gn(nid_ctx* c, const JobSet& js, double delta, double* gn_out);
+int launch_latency_round(nid_ctx* c, const JobSet& js, size_t h2d_bytes, double delta, double* gn_out);
 int launch_href(nid_ctx* c, int pair0, int n);
 
 // kernel launchers (nid_kernels.cu)
@@ -363,9 +369,9 @@ int launch_downsample2(nid_ctx* dst, int dst_pair0, const nid_ctx* src, int src_
 int launch_prepare(nid_ctx* c, int pair0, int n, const double* d_poses16);
 int launch_ref_weights(nid_ctx* c, int pair);
 int launch_points_aos(nid_ctx* c, int pair, double* d_out);
-int launch_hard(nid_ctx* c, int n_jobs);
+int launch_hard(nid_ctx* c, const JobSet& js);
 int launch_warp_sample(nid_ctx* c, int pair, const double* d_pose16, int f64);
-int launch_warp_sample_jobs(nid_ctx* c, int n_jobs, float4* d_out, bool u16);
+int launch_warp_sample_jobs(nid_ctx* c, const JobSet& js, float4* d_out, bool u16);
 int launch_check_integral(nid_ctx* c, const double* d_src, uint8_t* d_dst, int is_ref);
 int launch_points_soa(nid_ctx* c, int pair, const double* d_in);
 int launch_import_flags(nid_ctx* c, int pair, const double* d_bsv);

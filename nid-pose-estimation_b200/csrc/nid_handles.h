@@ -1,7 +1,6 @@
 // Owning handles of the CUDA resources a context holds. Every handle is released by the destructor of its owner, so a
 // context releases everything it acquired -- also when nid_create fails half way. An owner converts to its raw handle
-// (device and pinned buffers read like the raw pointers they hold); code that repoints a handle at run time keeps a plain
-// pointer beside the owner (see nid_ctx).
+// (device and pinned buffers read like the raw pointers they hold).
 #pragma once
 #include <cuda_runtime.h>
 #include <stddef.h>

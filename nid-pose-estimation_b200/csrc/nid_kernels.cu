@@ -689,23 +689,21 @@ int launch_ref_weights(nid_ctx* c, int pair) {
 }
 
 int launch_gn(nid_ctx* c, const JobSet& js, double delta, int want_jac) {
-  EvalParams p = make_params(c, js.slots);
+  EvalParams p = make_params(c, js);
   p.huber_delta = delta;
   p.huber_dsqr = (double)(float)(delta * delta);  // `float dsqr`, robust_kernel_impl.h:84
-  p.job0 = js.first;
-  p.job_list = js.d_list;
-  k_gn<<<js.n, 128, 0, c->stream>>>(p, want_jac);
+  k_gn<<<js.n, 128, 0, js.stream>>>(p, want_jac);
   NID_LAUNCH_CHECK(c, want_jac ? "k_gn" : "k_gn(chi2)");
   return NID_OK;
 }
 
-int launch_hard(nid_ctx* c, int n_jobs) {
-  EvalParams p = make_params(c, n_jobs);
+int launch_hard(nid_ctx* c, const JobSet& js) {
+  EvalParams p = make_params(c, js);
   size_t smem = sizeof(unsigned int) * (p.bins * p.bins + 2 * p.bins + 1);
-  dim3 g(p.ncell, n_jobs);
-  k_hard<<<g, 256, smem, c->stream>>>(p, c->hard);
+  dim3 g(p.ncell, js.n);
+  k_hard<<<g, 256, smem, js.stream>>>(p, c->hard);
   NID_LAUNCH_CHECK(c, "k_hard");
-  k_hard_total<<<(n_jobs + 127) / 128, 128, 0, c->stream>>>(n_jobs, p.ncell, c->hard);
+  k_hard_total<<<(js.n + 127) / 128, 128, 0, js.stream>>>(js.n, p.ncell, c->hard);
   NID_LAUNCH_CHECK(c, "k_hard_total");
   return NID_OK;
 }

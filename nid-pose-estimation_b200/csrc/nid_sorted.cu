@@ -1851,14 +1851,14 @@ size_t assemble_smem(const nid_ctx* c, int threads) {
   return sizeof(double) * ((size_t)5 * c->bins * c->bins + c->bins + threads + (size_t)NID_NCLS * c->bins + (NID_FEW_BINS(c->bins) ? 1024 : 0));
 }
 
-// Host side of the geometry table: job (first + i) -> gt.g[i] from the staged poses (pinned mirror), the pair's
+// Host side of the geometry table: job s0 + i of js -> gt.g[i] from the host mirrors of its pose and pair, the pair's
 // T_wc0 and intrinsics. pass1: rows 0 and 1 of M pre-multiplied by fx, fy.
 template <int NG>
-static void fill_geo(const nid_ctx* c, GeoTable<NG>& gt, int first, int n, bool pass1, const int* h_list = nullptr) {
+static void fill_geo(const nid_ctx* c, GeoTable<NG>& gt, const JobSet& js, int s0, int n, bool pass1) {
   for (int i = 0; i < n; i++) {
-    const int job = h_list ? h_list[first + i] : first + i;
-    const double* T1 = c->h_poses + 16 * (size_t)job;
-    const int pair = c->h_job_pair[job];
+    const int job = js.h_list ? js.h_list[js.first + s0 + i] : js.first + s0 + i;
+    const double* T1 = js.h_poses + 16 * (size_t)job;
+    const int pair = js.h_pair[job];
     const double* T0 = c->h_Twc0.data() + 16 * (size_t)pair;
     const double* cam = c->h_cam.data() + 4 * (size_t)pair;
     double* g = gt.g[i];
@@ -1882,43 +1882,44 @@ static void fill_geo(const nid_ctx* c, GeoTable<NG>& gt, int first, int n, bool 
 }
 
 template <bool PTS, int NG>
-static void launch_hist_chunks(nid_ctx* c, const EvalParams& p, int ns, int job0, int n_jobs, const int* h_list) {
+static int launch_hist_chunks(nid_ctx* c, const EvalParams& p, int ns, const JobSet& js) {
   // (many bins: the rows take the shared memory that one-warp CTAs would need for 18 resident warps: 128-thread CTAs)
-  const int T = pick_block(c, ns, n_jobs, c->bins > 20 ? 128 : NID_HIST_TMAX);
+  const int T = pick_block(c, ns, js.n, c->bins > 20 ? 128 : NID_HIST_TMAX);
   const size_t sm = hist_sell_smem(c, T);
-  for (int s0 = 0; s0 < n_jobs; s0 += NG) {
-    const int n = std::min(NG, n_jobs - s0);
+  for (int s0 = 0; s0 < js.n; s0 += NG) {
+    const int n = std::min(NG, js.n - s0);
     GeoTable<NG> gt;
-    fill_geo(c, gt, job0 + s0, n, true, h_list);
+    fill_geo(c, gt, js, s0, n, true);
     EvalParams q = p;
-    q.job0 = job0 + s0;
+    q.job0 = js.first + s0;
     const dim3 grid = NID_GRID(n, (ns + T / 32 - 1) / (T / 32));
     switch (T) {
-      case 256: k_hist_sell<PTS, NG, 256><<<grid, 256, sm, c->stream>>>(q, gt); c->last_hist_func = (const void*)k_hist_sell<PTS, NG, 256>; break;
-      case 128: k_hist_sell<PTS, NG, 128><<<grid, 128, sm, c->stream>>>(q, gt); c->last_hist_func = (const void*)k_hist_sell<PTS, NG, 128>; break;
-      case 64: k_hist_sell<PTS, NG, 64><<<grid, 64, sm, c->stream>>>(q, gt); c->last_hist_func = (const void*)k_hist_sell<PTS, NG, 64>; break;
-      default: k_hist_sell<PTS, NG, 32><<<grid, 32, sm, c->stream>>>(q, gt); c->last_hist_func = (const void*)k_hist_sell<PTS, NG, 32>; break;
+      case 256: k_hist_sell<PTS, NG, 256><<<grid, 256, sm, js.stream>>>(q, gt); c->last_hist_func = (const void*)k_hist_sell<PTS, NG, 256>; break;
+      case 128: k_hist_sell<PTS, NG, 128><<<grid, 128, sm, js.stream>>>(q, gt); c->last_hist_func = (const void*)k_hist_sell<PTS, NG, 128>; break;
+      case 64: k_hist_sell<PTS, NG, 64><<<grid, 64, sm, js.stream>>>(q, gt); c->last_hist_func = (const void*)k_hist_sell<PTS, NG, 64>; break;
+      default: k_hist_sell<PTS, NG, 32><<<grid, 32, sm, js.stream>>>(q, gt); c->last_hist_func = (const void*)k_hist_sell<PTS, NG, 32>; break;
     }
-    c->launches++;
+    NID_LAUNCH_CHECK(c, "k_hist_sell");
   }
+  return NID_OK;
 }
 template <bool PTS, int NG>
-static void launch_jac_chunks(nid_ctx* c, const EvalParams& p, int ns, int job0, int n_jobs, const int* h_list) {
+static int launch_jac_chunks(nid_ctx* c, const EvalParams& p, int ns, const JobSet& js) {
   // CTA size by geometry (it does not change any result): small cells have short slices, and one-warp CTAs let the SM
   // replace every finished slice at once -- measured at 16x16 cells 5.93 -> 5.47 us per evaluation with 32 threads, at
   // 4x4 cells 3.41 -> 3.66 (there two slices per CTA share the L1 lines of the target gathers)
-  const int T = pick_block(c, ns, n_jobs, (long long)c->rb * c->cb < NID_SMALL_CELL_PX ? 32 : NID_JAC_TMAX);
+  const int T = pick_block(c, ns, js.n, (long long)c->rb * c->cb < NID_SMALL_CELL_PX ? 32 : NID_JAC_TMAX);
   const size_t sm = jac_sell_smem(c, T);
-  for (int s0 = 0; s0 < n_jobs; s0 += NG) {
-    const int n = std::min(NG, n_jobs - s0);
+  for (int s0 = 0; s0 < js.n; s0 += NG) {
+    const int n = std::min(NG, js.n - s0);
     GeoTable<NG> gt;
-    fill_geo(c, gt, job0 + s0, n, false, h_list);
+    fill_geo(c, gt, js, s0, n, false);
     EvalParams q = p;
-    q.job0 = job0 + s0;
+    q.job0 = js.first + s0;
     const dim3 grid = NID_GRID(n, (ns + T / 32 - 1) / (T / 32));
 #define NID_JAC_LAUNCH(TT, BK)                                                 \
   do {                                                                         \
-    k_jac_sell<PTS, NG, TT, BK><<<grid, TT, sm, c->stream>>>(q, gt);           \
+    k_jac_sell<PTS, NG, TT, BK><<<grid, TT, sm, js.stream>>>(q, gt);          \
     c->last_jac_func = (const void*)k_jac_sell<PTS, NG, TT, BK>;               \
   } while (0)
     const bool bulk = q.stage_bulk && NID_FEW_BINS(c->bins);
@@ -1928,28 +1929,21 @@ static void launch_jac_chunks(nid_ctx* c, const EvalParams& p, int ns, int job0,
       default: if (bulk) NID_JAC_LAUNCH(32, true); else NID_JAC_LAUNCH(32, false); break;
     }
 #undef NID_JAC_LAUNCH
-    c->launches++;
+    NID_LAUNCH_CHECK(c, "k_jac_sell");
   }
+  return NID_OK;
 }
 #define NID_GEO_SMALL 8
 #define NID_GEO_LARGE 96
-static void launch_hist_w(nid_ctx* c, const EvalParams& p, int ns, int job0, int n_jobs, const int* h_list) {
-  if (c->sell_points) {
-    if (n_jobs <= NID_GEO_SMALL) launch_hist_chunks<true, NID_GEO_SMALL>(c, p, ns, job0, n_jobs, h_list);
-    else launch_hist_chunks<true, NID_GEO_LARGE>(c, p, ns, job0, n_jobs, h_list);
-  } else {
-    if (n_jobs <= NID_GEO_SMALL) launch_hist_chunks<false, NID_GEO_SMALL>(c, p, ns, job0, n_jobs, h_list);
-    else launch_hist_chunks<false, NID_GEO_LARGE>(c, p, ns, job0, n_jobs, h_list);
-  }
+static int launch_hist_w(nid_ctx* c, const EvalParams& p, int ns, const JobSet& js) {
+  if (c->sell_points)
+    return js.n <= NID_GEO_SMALL ? launch_hist_chunks<true, NID_GEO_SMALL>(c, p, ns, js) : launch_hist_chunks<true, NID_GEO_LARGE>(c, p, ns, js);
+  return js.n <= NID_GEO_SMALL ? launch_hist_chunks<false, NID_GEO_SMALL>(c, p, ns, js) : launch_hist_chunks<false, NID_GEO_LARGE>(c, p, ns, js);
 }
-static void launch_jac_w(nid_ctx* c, const EvalParams& p, int ns, int job0, int n_jobs, const int* h_list) {
-  if (c->sell_points) {
-    if (n_jobs <= NID_GEO_SMALL) launch_jac_chunks<true, NID_GEO_SMALL>(c, p, ns, job0, n_jobs, h_list);
-    else launch_jac_chunks<true, NID_GEO_LARGE>(c, p, ns, job0, n_jobs, h_list);
-  } else {
-    if (n_jobs <= NID_GEO_SMALL) launch_jac_chunks<false, NID_GEO_SMALL>(c, p, ns, job0, n_jobs, h_list);
-    else launch_jac_chunks<false, NID_GEO_LARGE>(c, p, ns, job0, n_jobs, h_list);
-  }
+static int launch_jac_w(nid_ctx* c, const EvalParams& p, int ns, const JobSet& js) {
+  if (c->sell_points)
+    return js.n <= NID_GEO_SMALL ? launch_jac_chunks<true, NID_GEO_SMALL>(c, p, ns, js) : launch_jac_chunks<true, NID_GEO_LARGE>(c, p, ns, js);
+  return js.n <= NID_GEO_SMALL ? launch_jac_chunks<false, NID_GEO_SMALL>(c, p, ns, js) : launch_jac_chunks<false, NID_GEO_LARGE>(c, p, ns, js);
 }
 
 // the natural-order kernels (nid_kernels.cu)
@@ -1961,101 +1955,88 @@ __global__ void k_jac_final(EvalParams p, int n_jobs);
 // Pass 1 of the jobs of js. Sorted: pixel kernel + assembly (histograms, entropies, err; unless p2 == none also the
 // scaled log tables pass 2 needs). Natural: strip histograms, then the cost tail k_entropy unless k_jac will write it.
 int launch_pass1(nid_ctx* c, const JobSet& js, Pass2 p2) {
-  EvalParams p = make_params(c, js.slots);
-  p.job0 = js.first;
-  p.job_list = js.d_list;
+  const EvalParams p = make_params(c, js);
   const int n = js.n;
   if (!use_sorted(c)) {
     const size_t smem = sizeof(double) * p.hist_stride;
-    ktime_mark(c, 0);
-    k_hist<<<dim3(p.S, p.ncell, n), 256, smem, c->stream>>>(p);
+    ktime_mark(c, js.stream, 0);
+    k_hist<<<dim3(p.S, p.ncell, n), 256, smem, js.stream>>>(p);
     NID_LAUNCH_CHECK(c, "k_hist");
-    ktime_mark(c, 1);
+    ktime_mark(c, js.stream, 1);
     if (p2 != Pass2::all) {
-      k_entropy<<<dim3(p.ncell, n), 256, smem, c->stream>>>(p);
+      k_entropy<<<dim3(p.ncell, n), 256, smem, js.stream>>>(p);
       NID_LAUNCH_CHECK(c, "k_entropy");
     }
-    ktime_mark(c, 2);
+    ktime_mark(c, js.stream, 2);
     return NID_OK;
   }
   const int tables = p2 != Pass2::none;
   const int ns = c->max_nslices_prepared;
-  ktime_mark(c, 0);
-  if (ns > 0) {  // (no slices at all: every cell of every prepared pair is inactive; the assembly reports NaN)
-    launch_hist_w(c, p, ns, js.first, n, js.h_list);
-    c->launches--;
-    NID_LAUNCH_CHECK(c, "k_hist_sell");
-  }
-  ktime_mark(c, 1);
+  ktime_mark(c, js.stream, 0);
+  // (no slices at all: every cell of every prepared pair is inactive; the assembly reports NaN)
+  const int r = ns > 0 ? launch_hist_w(c, p, ns, js) : NID_OK;
+  if (r != NID_OK) return r;
+  ktime_mark(c, js.stream, 1);
   if (assemble_warp(c)) {
     const int units = c->ncell * n;
     if (units <= 2 * c->sm_count * NID_ASMW_WARPS)
-      k_assemble_warp<NID_ASMW_BATCH_LAT><<<(units + NID_ASMW_WARPS - 1) / NID_ASMW_WARPS, NID_ASMW_WARPS * 32, assemble_warp_smem(c), c->stream>>>(p, tables, n);
+      k_assemble_warp<NID_ASMW_BATCH_LAT><<<(units + NID_ASMW_WARPS - 1) / NID_ASMW_WARPS, NID_ASMW_WARPS * 32, assemble_warp_smem(c), js.stream>>>(p, tables, n);
     else
-      k_assemble_warp<NID_ASMW_BATCH><<<(units + NID_ASMW_WARPS - 1) / NID_ASMW_WARPS, NID_ASMW_WARPS * 32, assemble_warp_smem(c), c->stream>>>(p, tables, n);
+      k_assemble_warp<NID_ASMW_BATCH><<<(units + NID_ASMW_WARPS - 1) / NID_ASMW_WARPS, NID_ASMW_WARPS * 32, assemble_warp_smem(c), js.stream>>>(p, tables, n);
   } else if (c->opt_asm_wide && (c->ncell * n <= c->sm_count || c->opt_asm_wide == 2 ||
                                  (!assemble_small(c) && assemble_smem(c, NID_ASM_THREADS) > (size_t)100 * 1024))) {
     // the 1024-thread variant (same bits): for a handful of evaluations in flight (fewer units than SMs), and whenever the
     // shared memory of a CTA leaves room for one or two CTAs per SM only (more than ~30 bins) -- 1024 threads then fill the
     // SM where 256 leave it mostly empty (C3, 32 bins: 5.57 -> 4.00 us per evaluation; 40 bins at 640x480: 4.59 -> 2.55;
     // but 28 bins: 1.97 -> 2.09, 24 bins: 1.44 -> 1.88, 16 bins: 0.87 -> 1.51, so not there)
-    k_assemble_wide<<<dim3(c->ncell, n), NID_ASM_WIDE, assemble_smem(c, NID_ASM_WIDE), c->stream>>>(p, tables);
-  } else if (assemble_small(c)) k_assemble_small<<<dim3(c->ncell, n), NID_ASM_SMALL, assemble_smem(c, NID_ASM_THREADS), c->stream>>>(p, tables);
-  else k_assemble<<<dim3(c->ncell, n), NID_ASM_THREADS, assemble_smem(c, NID_ASM_THREADS), c->stream>>>(p, tables);
+    k_assemble_wide<<<dim3(c->ncell, n), NID_ASM_WIDE, assemble_smem(c, NID_ASM_WIDE), js.stream>>>(p, tables);
+  } else if (assemble_small(c)) k_assemble_small<<<dim3(c->ncell, n), NID_ASM_SMALL, assemble_smem(c, NID_ASM_THREADS), js.stream>>>(p, tables);
+  else k_assemble<<<dim3(c->ncell, n), NID_ASM_THREADS, assemble_smem(c, NID_ASM_THREADS), js.stream>>>(p, tables);
   NID_LAUNCH_CHECK(c, "k_assemble");
-  ktime_mark(c, 2);
+  ktime_mark(c, js.stream, 2);
   return NID_OK;
 }
 
 // Pass 2 + Jacobian tail of the jobs of js; their pass 1 must have run at their current poses (sorted: with the tables).
 int launch_pass2(nid_ctx* c, const JobSet& js) {
-  EvalParams p = make_params(c, js.slots);
-  p.job0 = js.first;
-  p.job_list = js.d_list;
+  const EvalParams p = make_params(c, js);
   const int n = js.n;
   if (!use_sorted(c)) {
-    k_jac<<<dim3(p.S, p.ncell, n), 256, sizeof(double) * p.hist_stride, c->stream>>>(p);
+    k_jac<<<dim3(p.S, p.ncell, n), 256, sizeof(double) * p.hist_stride, js.stream>>>(p);
     NID_LAUNCH_CHECK(c, "k_jac");
-    ktime_mark(c, 3);
-    k_jac_final<<<(n * p.ncell * 6 + 255) / 256, 256, 0, c->stream>>>(p, n);
+    ktime_mark(c, js.stream, 3);
+    k_jac_final<<<(n * p.ncell * 6 + 255) / 256, 256, 0, js.stream>>>(p, n);
     NID_LAUNCH_CHECK(c, "k_jac_final");
-    ktime_mark(c, 4);
+    ktime_mark(c, js.stream, 4);
     return NID_OK;
   }
   const int ns = c->max_nslices_prepared;
-  if (ns > 0) {
-    launch_jac_w(c, p, ns, js.first, n, js.h_list);
-    c->launches--;
-    NID_LAUNCH_CHECK(c, "k_jac_sell");
-  }
-  ktime_mark(c, 3);
-  k_jac_final_sorted<<<jac_final_blocks(c, n), 256, 0, c->stream>>>(p, n);
+  const int r = ns > 0 ? launch_jac_w(c, p, ns, js) : NID_OK;
+  if (r != NID_OK) return r;
+  ktime_mark(c, js.stream, 3);
+  k_jac_final_sorted<<<jac_final_blocks(c, n), 256, 0, js.stream>>>(p, n);
   NID_LAUNCH_CHECK(c, "k_jac_final_sorted");
-  ktime_mark(c, 4);
+  ktime_mark(c, js.stream, 4);
   return NID_OK;
 }
 
-int launch_sorted_tail_gn(nid_ctx* c, const int* d_list, const int* h_list, int first, int n, double delta, double* gn_out) {
-  EvalParams p = make_params(c, n);
-  p.job0 = first;
-  p.job_list = d_list;
+int launch_sorted_tail_gn(nid_ctx* c, const JobSet& js, double delta, double* gn_out) {
+  EvalParams p = make_params(c, js);
   p.huber_delta = delta;
   p.huber_dsqr = (double)(float)(delta * delta);  // `float dsqr`, robust_kernel_impl.h:84
+  const int n = js.n;
   const int ns = c->max_nslices_prepared;
-  if (ns > 0) {
-    launch_jac_w(c, p, ns, first, n, h_list);
-    c->launches--;
-    NID_LAUNCH_CHECK(c, "k_jac_sell");
-  }
+  const int r = ns > 0 ? launch_jac_w(c, p, ns, js) : NID_OK;
+  if (r != NID_OK) return r;
   if (c->ncell <= 32) {
-    k_tail_gn<<<n, 256, 0, c->stream>>>(p, gn_out);
+    k_tail_gn<<<n, 256, 0, js.stream>>>(p, gn_out);
     NID_LAUNCH_CHECK(c, "k_tail_gn");
   } else {
     // many cells (the reference's default geometry has 256): one CTA per job would walk them eight at a time (measured
     // ~120 us of a 240 us round); a warp per (job, cell) for the tails, then the block sums
-    k_jac_final_sorted<<<jac_final_blocks(c, n), 256, 0, c->stream>>>(p, n);
+    k_jac_final_sorted<<<jac_final_blocks(c, n), 256, 0, js.stream>>>(p, n);
     NID_LAUNCH_CHECK(c, "k_jac_final_sorted");
-    k_gn_out<<<n, 128, 0, c->stream>>>(p, gn_out);
+    k_gn_out<<<n, 128, 0, js.stream>>>(p, gn_out);
     NID_LAUNCH_CHECK(c, "k_gn_out");
   }
   return NID_OK;
@@ -2078,11 +2059,10 @@ struct LatencyGraph {
   cudaKernelNodeParams hist_np{}, jac_np{};
   EvalParams hist_q, jac_q;  // first argument of the two pixel kernels as captured
   // signature
-  EvalParams sig;
+  EvalParams sig;  // (holds the slot list and the device pose table)
   int nslots = 0, ns = 0, task_px = 0;
   size_t h2d_bytes = 0;
   double delta = 0.0;
-  const int* d_list = nullptr;
   const double* gn_out = nullptr;
   const void* h_src = nullptr;
   cudaStream_t stream = nullptr;
@@ -2090,19 +2070,18 @@ struct LatencyGraph {
 
 void LatencyGraphDelete::operator()(LatencyGraph* g) const { delete g; }
 
-static int capture_latency_graph(nid_ctx* c, LatencyGraph* g, int nslots, const int* d_list, const int* h_list, size_t h2d_bytes,
-                                 double delta, double* gn_out) {
+static int capture_latency_graph(nid_ctx* c, LatencyGraph* g, const JobSet& js, size_t h2d_bytes, double delta, double* gn_out) {
   g->exec.reset();
   g->graph.reset();
-  cudaError_t e = cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal);
+  cudaError_t e = cudaStreamBeginCapture(js.stream, cudaStreamCaptureModeThreadLocal);
   if (e != cudaSuccess) return check_cuda(e, "cudaStreamBeginCapture");
   int r = NID_OK;
-  e = cudaMemcpyAsync(c->poses, c->h_poses, h2d_bytes, cudaMemcpyHostToDevice, c->stream);
+  e = cudaMemcpyAsync(js.d_poses, js.h_poses, h2d_bytes, cudaMemcpyHostToDevice, js.stream);
   if (e != cudaSuccess) r = check_cuda(e, "H2D poses + list (capture)");
-  if (r == NID_OK) r = launch_pass1(c, JobSet{d_list, h_list, 0, nslots, nslots}, Pass2::some);
-  if (r == NID_OK) r = launch_sorted_tail_gn(c, d_list, h_list, 0, nslots, delta, gn_out);
+  if (r == NID_OK) r = launch_pass1(c, js, Pass2::some);
+  if (r == NID_OK) r = launch_sorted_tail_gn(c, js, delta, gn_out);
   cudaGraph_t graph = nullptr;
-  e = cudaStreamEndCapture(c->stream, &graph);
+  e = cudaStreamEndCapture(js.stream, &graph);
   g->graph.reset(graph);
   if (r != NID_OK) return r;
   if (e != cudaSuccess) return check_cuda(e, "cudaStreamEndCapture");
@@ -2134,33 +2113,35 @@ static int capture_latency_graph(nid_ctx* c, LatencyGraph* g, int nslots, const 
   return NID_OK;
 }
 
-// One round of the latency mode over the slots h_list[0 .. nslots) (every slot of the solve, each exactly once).
-int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h_list, size_t h2d_bytes, double delta, double* gn_out) {
+// One round of the latency mode over the slots js.h_list[0 .. js.n) (every slot of the solve, each exactly once): the
+// staging block of h2d_bytes at js.h_poses (poses, then the slot list js.d_list points into) is copied to js.d_poses first.
+int launch_latency_round(nid_ctx* c, const JobSet& js, size_t h2d_bytes, double delta, double* gn_out) {
+  const int nslots = js.n;
   const int ns = c->max_nslices_prepared;
   const bool graph_ok = c->opt_lm_graph && !c->opt_time_kernels && ns > 0 && nslots <= NID_GEO_SMALL;
   if (!graph_ok) {
-    cudaError_t e = cudaMemcpyAsync(c->poses, c->h_poses, h2d_bytes, cudaMemcpyHostToDevice, c->stream);
+    cudaError_t e = cudaMemcpyAsync(js.d_poses, js.h_poses, h2d_bytes, cudaMemcpyHostToDevice, js.stream);
     if (e != cudaSuccess) return check_cuda(e, "H2D poses + list");
-    int r = launch_pass1(c, JobSet{d_list, h_list, 0, nslots, nslots}, Pass2::some);
+    int r = launch_pass1(c, js, Pass2::some);
     if (r != NID_OK) return r;
-    return launch_sorted_tail_gn(c, d_list, h_list, 0, nslots, delta, gn_out);
+    return launch_sorted_tail_gn(c, js, delta, gn_out);
   }
   if (!c->lm_graph) c->lm_graph.reset(new LatencyGraph());
   LatencyGraph* g = c->lm_graph.get();
-  const EvalParams sig = make_params(c, nslots);
+  const EvalParams sig = make_params(c, js);
   const bool same = g->exec && memcmp(&sig, &g->sig, sizeof(sig)) == 0 && g->nslots == nslots && g->ns == ns && g->task_px == c->task_px &&
-                    g->h2d_bytes == h2d_bytes && g->delta == delta && g->d_list == d_list && g->gn_out == gn_out &&
-                    g->h_src == (const void*)c->h_poses && g->stream == c->stream;
+                    g->h2d_bytes == h2d_bytes && g->delta == delta && g->gn_out == gn_out && g->h_src == (const void*)js.h_poses &&
+                    g->stream == js.stream;
   if (!same) {
-    const int r = capture_latency_graph(c, g, nslots, d_list, h_list, h2d_bytes, delta, gn_out);
+    const int r = capture_latency_graph(c, g, js, h2d_bytes, delta, gn_out);
     if (r != NID_OK) { c->lm_graph.reset(); return r; }
     g->sig = sig; g->nslots = nslots; g->ns = ns; g->task_px = c->task_px; g->h2d_bytes = h2d_bytes; g->delta = delta;
-    g->d_list = d_list; g->gn_out = gn_out; g->h_src = c->h_poses; g->stream = c->stream;
+    g->gn_out = gn_out; g->h_src = js.h_poses; g->stream = js.stream;
     // (the graph just captured holds this round's geometry already)
   } else {
     GeoTable<NID_GEO_SMALL> gt;
     for (int pass = 0; pass < 2; pass++) {
-      fill_geo(c, gt, 0, nslots, pass == 0, h_list);
+      fill_geo(c, gt, js, 0, nslots, pass == 0);
       cudaKernelNodeParams np = pass == 0 ? g->hist_np : g->jac_np;
       void* args[2] = {pass == 0 ? (void*)&g->hist_q : (void*)&g->jac_q, (void*)&gt};
       np.kernelParams = args;
@@ -2169,7 +2150,7 @@ int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h
       if (e != cudaSuccess) return check_cuda(e, "cudaGraphExecKernelNodeSetParams");
     }
   }
-  const cudaError_t e = cudaGraphLaunch(g->exec, c->stream);
+  const cudaError_t e = cudaGraphLaunch(g->exec, js.stream);
   if (e != cudaSuccess) return check_cuda(e, "cudaGraphLaunch");
   c->launches += 4;
   return NID_OK;
@@ -2177,8 +2158,8 @@ int launch_latency_round(nid_ctx* c, int nslots, const int* d_list, const int* h
 
 // Geometry table of kernel 1 (see k_warp_sample_jobs): the ray of pixel (col, row) is affine in (col, row)
 template <int NG>
-static void fill_geo_k1(const nid_ctx* c, GeoTable<NG>& gt, int first, int n) {
-  fill_geo(c, gt, first, n, true);  // [0..11] M with rows 0/1 scaled by fx, fy; [12] 1/fx [13] -cx/fx [14] 1/fy [15] -cy/fy
+static void fill_geo_k1(const nid_ctx* c, GeoTable<NG>& gt, const JobSet& js, int s0, int n) {
+  fill_geo(c, gt, js, s0, n, true);  // [0..11] M with rows 0/1 scaled by fx, fy; [12] 1/fx [13] -cx/fx [14] 1/fy [15] -cy/fy
   for (int i = 0; i < n; i++) {
     double* g = gt.g[i];
     const double ifx = g[12], cxo = g[13], ify = g[14], cyo = g[15], cx = g[18], cy = g[19];
@@ -2207,18 +2188,18 @@ int launch_pack_k1(nid_ctx* c, int pair, unsigned short* d_out) {
 }
 
 // all jobs of a launch must take their depth from the same kind of plane (raw 16-bit or fp64): u16 says which
-int launch_warp_sample_jobs(nid_ctx* c, int n_jobs, float4* d_out, bool u16) {
-  EvalParams p = make_params(c, n_jobs);
+int launch_warp_sample_jobs(nid_ctx* c, const JobSet& js, float4* d_out, bool u16) {
+  const EvalParams p = make_params(c, js);
   const int chunks = (c->N + 128 * NID_WS_W - 1) / (128 * NID_WS_W);
-  for (int s0 = 0; s0 < n_jobs; s0 += NID_GEO_LARGE) {
-    const int n = std::min(NID_GEO_LARGE, n_jobs - s0);
+  for (int s0 = 0; s0 < js.n; s0 += NID_GEO_LARGE) {
+    const int n = std::min(NID_GEO_LARGE, js.n - s0);
     GeoTable<NID_GEO_LARGE> gt;
-    fill_geo_k1(c, gt, s0, n);
+    fill_geo_k1(c, gt, js, s0, n);
     EvalParams q = p;
-    q.job0 = s0;
+    q.job0 = js.first + s0;
     const dim3 grid(n, chunks);
-    if (u16) k_warp_sample_jobs<NID_GEO_LARGE, true><<<grid, 128, 0, c->stream>>>(q, gt, nullptr, c->depth16, c->depth_factor, d_out);
-    else k_warp_sample_jobs<NID_GEO_LARGE, false><<<grid, 128, 0, c->stream>>>(q, gt, c->depth, nullptr, nullptr, d_out);
+    if (u16) k_warp_sample_jobs<NID_GEO_LARGE, true><<<grid, 128, 0, js.stream>>>(q, gt, nullptr, c->depth16, c->depth_factor, d_out);
+    else k_warp_sample_jobs<NID_GEO_LARGE, false><<<grid, 128, 0, js.stream>>>(q, gt, c->depth, nullptr, nullptr, d_out);
     NID_LAUNCH_CHECK(c, "k_warp_sample_jobs");
   }
   return NID_OK;

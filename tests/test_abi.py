@@ -83,3 +83,39 @@ def test_cuda_resources_are_acquired_and_released_only_by_their_owner_types():
             found[os.path.basename(path)] = names
     assert set(found) == {"nid_handles.h"}, found
     assert release <= found["nid_handles.h"]
+
+
+def test_evaluation_launches_take_their_stream_and_job_table_from_their_arguments():
+    """The evaluation launchers read the stream they issue on, the pose table and its host mirrors from their JobSet
+    argument: the context holds no view that a caller repoints while a call runs, and every launch is counted once,
+    where it is issued."""
+    import glob
+    import re
+    ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    csrc = os.path.join(ROOT, "nid-pose-estimation_b200", "csrc")
+
+    def code(path):
+        src = re.sub(r'"(?:\\.|[^"\\])*"', '""', open(path).read())
+        return re.sub(r"//[^\n]*|/\*.*?\*/", "", src, flags=re.S)
+
+    sources = {os.path.basename(p): code(p) for p in sorted(glob.glob(os.path.join(csrc, "*.cu*")) + glob.glob(os.path.join(csrc, "*.h")))}
+    hdr = sources["nid_ctx.h"]
+    ctx = re.search(r"struct nid_ctx \{(.*?)\n\};", hdr, re.S).group(1)
+    views = re.findall(r"\b(poses|h_poses|h_job_pair)\s*[=;\[]", ctx)
+    assert not views, views
+    # a context's stream is created once and never assigned: find every name a nid_ctx pointer goes by
+    names = set()
+    for src in sources.values():
+        names |= set(re.findall(r"\bnid_ctx\s*\*\s*(?:const\s*\*?\s*)?(\w+)", src))
+    assert {"c", "dst", "src"} <= names
+    assigned = [(f, m) for f, src in sources.items()
+                for m in re.findall(r"\b(?:%s)->stream\s*=(?!=)" % "|".join(sorted(names)), src)]
+    assert not assigned, assigned
+    decrements = [f for f, src in sources.items() if re.search(r"launches\s*(--|-=)", src)]
+    assert not decrements, decrements
+    launchers = {"launch_pass1", "launch_pass2", "launch_gn", "launch_sorted_tail_gn", "launch_latency_round", "launch_hard",
+                 "launch_warp_sample_jobs"}
+    decl = dict(re.findall(r"\bint (launch_\w+)\(([^)]*)\);", hdr))
+    assert launchers <= set(decl), launchers - set(decl)
+    wrong = [n for n in sorted(launchers) if "const JobSet&" not in decl[n]]
+    assert not wrong, wrong
