@@ -239,6 +239,9 @@ namespace nid {
 __host__ __device__ inline int wv_row(int B) { return NID_FEW_BINS(B) ? B + 1 : B; }
 __host__ __device__ inline int wv_stride(int B) { return (B * wv_row(B) + B + 1) & ~1; }
 __host__ __device__ inline int job_at(const EvalParams& p, int i) { return p.job_list ? p.job_list[p.job0 + i] : p.job0 + i; }
+// The Huber threshold delta^2 as the reference keeps it: `float dsqr` (robust_kernel_impl.h:84). Every launcher that fills
+// EvalParams::huber_dsqr takes it from here, so that all Gauss-Newton kernels classify a cell by the same rounded value.
+inline double huber_dsqr(double delta) { return (double)(float)(delta * delta); }
 #ifdef __CUDACC__
 // a11: the Huber-weighted Gauss-Newton block of a job, summed over its active cells in cell order
 // (base_unary_edge.hpp:43-72, robust_kernel_impl.cpp:78-90, sparse_optimizer.cpp:102-116):

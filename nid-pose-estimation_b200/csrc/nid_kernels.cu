@@ -691,7 +691,7 @@ int launch_ref_weights(nid_ctx* c, int pair) {
 int launch_gn(nid_ctx* c, const JobSet& js, double delta, int want_jac) {
   EvalParams p = make_params(c, js);
   p.huber_delta = delta;
-  p.huber_dsqr = (double)(float)(delta * delta);  // `float dsqr`, robust_kernel_impl.h:84
+  p.huber_dsqr = huber_dsqr(delta);
   k_gn<<<js.n, 128, 0, js.stream>>>(p, want_jac);
   NID_LAUNCH_CHECK(c, want_jac ? "k_gn" : "k_gn(chi2)");
   return NID_OK;

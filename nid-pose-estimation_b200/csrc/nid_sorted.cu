@@ -2023,7 +2023,7 @@ int launch_pass2(nid_ctx* c, const JobSet& js) {
 int launch_sorted_tail_gn(nid_ctx* c, const JobSet& js, double delta, double* gn_out) {
   EvalParams p = make_params(c, js);
   p.huber_delta = delta;
-  p.huber_dsqr = (double)(float)(delta * delta);  // `float dsqr`, robust_kernel_impl.h:84
+  p.huber_dsqr = huber_dsqr(delta);
   const int n = js.n;
   const int ns = c->max_nslices_prepared;
   const int r = ns > 0 ? launch_jac_w(c, p, ns, js) : NID_OK;

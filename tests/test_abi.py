@@ -119,3 +119,24 @@ def test_evaluation_launches_take_their_stream_and_job_table_from_their_argument
     assert launchers <= set(decl), launchers - set(decl)
     wrong = [n for n in sorted(launchers) if "const JobSet&" not in decl[n]]
     assert not wrong, wrong
+
+
+def test_the_huber_threshold_is_rounded_in_one_place():
+    """The reference keeps delta^2 as a float (robust_kernel_impl.h:84). The device code rounds it in one helper,
+    huber_dsqr in nid_ctx.h, and every launcher of a Gauss-Newton kernel fills EvalParams::huber_dsqr from it: the
+    blocks of k_gn, k_tail_gn and k_gn_out classify a cell by the same value, the one
+    tests/test_gpu_large_grids_gn.py::test_float_dsqr_on_the_device pins."""
+    import glob
+    import re
+    ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    csrc = os.path.join(ROOT, "nid-pose-estimation_b200", "csrc")
+    sources = {}
+    for path in sorted(glob.glob(os.path.join(csrc, "*.cu*")) + glob.glob(os.path.join(csrc, "*.h"))):
+        src = re.sub(r'"(?:\\.|[^"\\])*"', '""', open(path).read())
+        sources[os.path.basename(path)] = re.sub(r"//[^\n]*|/\*.*?\*/", "", src, flags=re.S)
+    casts = [(f, m) for f, src in sources.items() for m in re.findall(r"\(float\)\s*\(\s*delta\b[^;]*", src)]
+    assert casts == [("nid_ctx.h", "(float)(delta * delta)")], casts
+    assert re.search(r"inline double huber_dsqr\(double delta\) \{ return \(double\)\(float\)\(delta \* delta\); \}",
+                     sources["nid_ctx.h"])
+    fills = [(f, m.strip()) for f, src in sorted(sources.items()) for m in re.findall(r"\.huber_dsqr\s*=([^;]*);", src)]
+    assert fills == [("nid_kernels.cu", "huber_dsqr(delta)"), ("nid_sorted.cu", "huber_dsqr(delta)")], fills
